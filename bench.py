@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PPN output-parsing path (decode + NMS + limb arg-max + tree parse).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = one pass of the whole path over one batch of synthetic head tensors per GPU
 (BASELINE.json configs[1]: MPII 16-part, 384x384, 12x12 grid, 9x9 window, batch 512).  N > 1 is
@@ -468,6 +468,8 @@ def run_ours(args, rank, world, local_rank):
         last = outs[(n_steps - 1) % 2] if last is None else last
     else:
         elapsed_ms, host_issue_ms, last, t0 = timed_region(step, drain)
+    if args.dump_outputs:
+        dump_outputs(last, args.dump_outputs)
 
     # Spread of the measurement (SURVEY §8d asks for median and min): the same region four more times.
     # `value` stays the FIRST region's (exactly K steps after the warm-up); these are reported beside it.
@@ -750,6 +752,33 @@ def job_checksum(torch, dist, args, parser, gatherer, bufs, outs, B, world, rank
     return h.hexdigest()
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out, directory):
+    """Write the PackedHumans of one step as float32 DIR/<name>.npy, so that two builds can be compared output for
+    output.  Slots past count[b] keep whatever the buffer held before (the parse does not write them), so they are
+    reset to -1 / 0 here as PPN_FLAG_CLEAR_UNUSED would.  `count` covers the whole batch; the per-slot arrays cover
+    every image, or a fixed seeded sample of images (listed in images.npy) when the whole batch exceeds DUMP_BYTES."""
+    import numpy as np
+    a = out.numpy()
+    count = a["count"]
+    B, R = a["root_cell"].shape
+    used = np.arange(R)[None, :] < count[:, None]
+    slots = {"root_cell": np.where(used, a["root_cell"], -1),
+             "part_cell": np.where(used[..., None], a["part_cell"], -1),
+             "part_score": np.where(used[..., None], a["part_score"], 0),
+             "part_box": np.where(used[..., None, None], a["part_box"], 0)}
+    per_image = sum(v[0].size for v in slots.values()) * 4
+    n = min(B, (DUMP_BYTES - 8 * B - 4096) // per_image)      # count and images are 4 bytes an image; 4096 for headers
+    images = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "count.npy"), count.astype(np.float32))
+    np.save(os.path.join(directory, "images.npy"), images.astype(np.float32))
+    for name, v in slots.items():
+        np.save(os.path.join(directory, f"{name}.npy"), v[images].astype(np.float32))
+
+
 def cpu_baseline(cfg, args):
     """The reference-shaped numpy port on all host cores, bounded to ~args.cpu_budget_s seconds."""
     from oracle import cpu_bench, ppn_oracle as O
@@ -808,10 +837,16 @@ def main():
     ap.add_argument("--no-step-overlap", action="store_true",
                     help="do not pass PPN_FLAG_INPUT_COMPLETE (each step's kernels wait for the previous step's)")
     ap.add_argument("--tune", action="append", default=[], help="library knob, e.g. argmax.stages=6")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the poses of the last one as DIR/<name>.npy (float32, at most 64 MB; "
+                         "one GPU, --impl ours)")
     args = ap.parse_args()
     if args.config == "cfg5" and "--steps" not in " ".join(sys.argv):
         args.steps = 10                         # passes over the 8 192-image job
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        # with N > 1 the parse leaves the fixed-stride arrays unwritten and the poses exist only as gathered records
+        ap.error("--dump-outputs writes the one-GPU result of --impl ours")
     if args.impl == "reference":
         return run_reference(args, rank, world)
     return run_ours(args, rank, world, local_rank)
