@@ -25,6 +25,8 @@
  *                            the whole parse, without the head tensor ever reaching memory
  *   ppn_encode_targets ..... the inverse of the path: the "# Encode samples" half of
  *                            KeypointsDataset.__getitem__, dataset.py:89-198, for a whole batch
+ *   ppn_loss_forward ....... the consumer of those targets: PPNLoss.forward, main.py:125-216 (five terms)
+ *   ppn_loss_backward ...... its autograd backward with respect to the head tensor
  *
  * Conventions
  *   - plain C: pointers and sizes only; no CUDA or torch types.  `stream` is a cudaStream_t
@@ -349,6 +351,33 @@ typedef struct PPNTargets {
  * PPN_E_UNSUPPORTED otherwise. */
 int ppn_encode_targets(const PPNPeople* people, const PPNShape* shape, const int32_t* edges,
                        const PPNTargets* out, void* stream);
+
+/* ---- the training loss over the head tensor and the encoded targets --------------------------------
+ * Stands in for the reference's criterion PPNLoss (main.py:125-216), called as criterion(output, delta, weight,
+ * weight_ij, tx_half, ty_half, tx, ty, tw, th, te) in its training loop.  The reference tree is not part of this
+ * project: the specification is the float64 restatement documented in DESIGN.md §11 (IoU differentiable in x, y, w,
+ * h; eps = 1e-6 in the IoU denominator; L_resp unweighted), not bit parity with main.py.  For image b:
+ *   L_resp = sum (resp - delta)^2          L_iou = sum delta (conf - iou)^2
+ *   L_coor = sum weight ((x - tx_half)^2 + (y - ty_half)^2)
+ *   L_size = sum weight ((sqrt(w + eps) - sqrt(tw + eps))^2 + (sqrt(h + eps) - sqrt(th + eps))^2)
+ *   L_limb = sum weight_ij (e - te)^2
+ * over every element of the image, then averaged over the batch (sum / B).  The five terms stay separate: the
+ * reference weights them by GradNorm (main.py:704-708), so weighting is the caller's.
+ * head: fp32 [B, C, H, W] (PPN_HEAD_F32 only: PPN_E_UNSUPPORTED otherwise); `targets` as ppn_encode_targets writes
+ * them (read only).  Every pointer needs 4-byte alignment; the limb block is streamed with 128-bit accesses wherever
+ * the tensors of an image share their phase within 16 bytes.  B >= 1.
+ *   ppn_loss_workspace_bytes: scratch of ppn_loss_forward for this shape (per-CTA partial sums; 8-byte aligned).
+ *   ppn_loss_forward:  loss[5] (device fp32) = (L_resp, L_iou, L_coor, L_size, L_limb).  Deterministic: fp64
+ *                      partials reduced in a fixed order, no float atomics.
+ *   ppn_loss_backward: grad_head [B, C, H, W] (device fp32, every element written) = sum_t grad_loss[t] * dL_t/dhead,
+ *                      grad_loss[5] a DEVICE array (never read by the host).  Recomputes from the inputs; torch's
+ *                      conventions at kinks: relu'(0) = 0, a tie in min / max splits the gradient evenly.  The fp32
+ *                      operation order is documented in csrc/ppn_loss.cu. */
+int ppn_loss_workspace_bytes(const PPNShape* shape, size_t* bytes);
+int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets* targets, float* loss,
+                     void* workspace, size_t workspace_bytes, void* stream);
+int ppn_loss_backward(const float* head, const PPNShape* shape, const PPNTargets* targets, const float* grad_loss,
+                      float* grad_head, void* stream);
 
 #ifdef __cplusplus
 }

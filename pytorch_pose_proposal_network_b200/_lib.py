@@ -109,6 +109,11 @@ EXPORTS = {
                                      C.POINTER(PPNHeadOptions), C.POINTER(PPNHumans), C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                      C.c_void_p]),
     "ppn_encode_targets": (C.c_int, [C.POINTER(PPNPeople), C.POINTER(PPNShape), i32p, C.POINTER(PPNTargets), C.c_void_p]),
+    "ppn_loss_workspace_bytes": (C.c_int, [C.POINTER(PPNShape), C.POINTER(C.c_size_t)]),
+    "ppn_loss_forward": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.c_void_p, C.c_void_p,
+                                   C.c_size_t, C.c_void_p]),
+    "ppn_loss_backward": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.c_void_p, C.c_void_p,
+                                    C.c_void_p]),
     "ppn_debug_argmax_items": (C.c_int, [C.POINTER(PPNShape), C.c_int32, i32p, i32p, i32p, C.c_int32]),
     "ppn_timeline": (C.c_int, [C.c_void_p, C.c_int32]),
     "ppn_profile_enable": (C.c_int, [C.c_int32]),

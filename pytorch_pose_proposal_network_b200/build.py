@@ -17,7 +17,7 @@ ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 INCLUDE = os.path.join(ROOT, "include")
 LIB_PATH = os.path.join(PKG_DIR, "libppn_decode.so")
-SOURCES = ["ppn_kernels.cu", "ppn_encode.cu", "ppn_head.cu", "ppn_capi.cu"]
+SOURCES = ["ppn_kernels.cu", "ppn_encode.cu", "ppn_head.cu", "ppn_loss.cu", "ppn_capi.cu"]
 HEADERS = [os.path.join(CSRC, "ppn_device.cuh"), os.path.join(CSRC, "ppn_kernels.h"),
            os.path.join(INCLUDE, "ppn_decode.h"), os.path.join(INCLUDE, "ppn_decode_bench.h")]
 

@@ -990,6 +990,82 @@ int ppn_encode_targets(const PPNPeople* people, const PPNShape* shape, const int
     return cuda_rc(ppn::launch_encode_targets(a, shape->B, sms, (cudaStream_t)stream));
 }
 
+// ---- the training loss (PPNLoss, main.py:125-216) -----------------------------------------------------
+namespace {
+inline bool bad_f32(const void* p) { return !p || (reinterpret_cast<uintptr_t>(p) & 3); }
+
+int loss_args(const float* head, const PPNShape* shape, const PPNTargets* t, ppn::LossArgs* a) {
+    int rc = check_shape(shape);
+    if (rc) return rc;
+    if (shape->head_dtype != PPN_HEAD_F32) return PPN_E_UNSUPPORTED;
+    if (shape->B < 1) return PPN_E_BADARG;                                   // the batch mean needs an image
+    std::memset(a, 0, sizeof(*a));
+    const ppn::Geom g = make_geom(shape);
+    a->B = g.B; a->K = g.K; a->W = g.W; a->HW = g.HW; a->L = g.S * g.E * g.HW;
+    a->img_stride = g.img_stride; a->limb_off = g.limb_off;
+    a->gW = g.gridW; a->gH = g.gridH; a->inW = g.inW; a->inH = g.inH;
+    ppn::loss_plan(a);
+    if (!t) return PPN_E_BADARG;
+    const float* small[] = {t->delta, t->weight, t->tx, t->ty, t->tx_half, t->ty_half, t->tw, t->th};
+    for (const float* p : small)
+        if (bad_f32(p)) return PPN_E_BADARG;
+    if (bad_f32(head) || (a->L > 0 && (bad_f32(t->te) || bad_f32(t->weight_ij)))) return PPN_E_BADARG;
+    a->head = head;
+    a->delta = t->delta; a->weight = t->weight; a->weight_ij = t->weight_ij; a->tx = t->tx; a->ty = t->ty;
+    a->tx_half = t->tx_half; a->ty_half = t->ty_half; a->tw = t->tw; a->th = t->th; a->te = t->te;
+    return PPN_OK;
+}
+
+int sm_count(int* sms) {
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
+    return cuda_rc(e);
+}
+}  // namespace
+
+int ppn_loss_workspace_bytes(const PPNShape* shape, size_t* bytes) {
+    int rc = check_shape(shape);
+    if (rc) return rc;
+    if (!bytes) return PPN_E_BADARG;
+    if (shape->head_dtype != PPN_HEAD_F32) return PPN_E_UNSUPPORTED;
+    if (shape->B < 1) return PPN_E_BADARG;
+    ppn::LossArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.B = shape->B; a.K = shape->K; a.HW = shape->H * shape->W; a.L = shape->sH * shape->sW * shape->E * a.HW;
+    ppn::loss_plan(&a);
+    *bytes = ppn::loss_workspace_bytes(a);
+    return PPN_OK;
+}
+
+// PPNLoss.forward (main.py:125-216): the five batch-mean terms into loss[5]
+int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets* targets, float* loss,
+                     void* workspace, size_t workspace_bytes, void* stream) {
+    ppn::LossArgs a;
+    int rc = loss_args(head, shape, targets, &a);
+    if (rc) return rc;
+    if (bad_f32(loss) || !workspace || (reinterpret_cast<uintptr_t>(workspace) & 7)) return PPN_E_BADARG;
+    if (workspace_bytes < ppn::loss_workspace_bytes(a)) return PPN_E_WORKSPACE;
+    a.partial = static_cast<double*>(workspace);
+    int sms = 0;
+    if ((rc = sm_count(&sms))) return rc;
+    return cuda_rc(ppn::launch_loss_forward(a, loss, sms, (cudaStream_t)stream));
+}
+
+// PPNLoss's backward under autograd (loss.backward() in main.py's training step), with respect to the head only
+int ppn_loss_backward(const float* head, const PPNShape* shape, const PPNTargets* targets, const float* grad_loss,
+                      float* grad_head, void* stream) {
+    ppn::LossArgs a;
+    int rc = loss_args(head, shape, targets, &a);
+    if (rc) return rc;
+    if (bad_f32(grad_loss) || bad_f32(grad_head)) return PPN_E_BADARG;
+    a.grad_loss = grad_loss;
+    a.grad = grad_head;
+    int sms = 0;
+    if ((rc = sm_count(&sms))) return rc;
+    return cuda_rc(ppn::launch_loss_backward(a, sms, (cudaStream_t)stream));
+}
+
 int ppn_debug_argmax_items(const PPNShape* shape, int32_t sms, int32_t* info, int32_t* first, int32_t* size, int32_t max_items) {
     int rc = check_shape(shape);
     if (rc) return rc;

@@ -171,4 +171,23 @@ struct EncodeArgs {
 };
 cudaError_t launch_encode_targets(EncodeArgs a, int B, int sms, cudaStream_t st);
 
+// ---- the training loss (ppn_loss.cu): forward sums and the head gradient of the reference's PPNLoss -------------
+constexpr int kLossMaxCtas = 2048;     // CTAs of the forward grid at most: the workspace holds one partial set each
+struct LossArgs {
+    const float* head;                  // [B, C, H, W]
+    float* grad;                        // [B, C, H, W] (backward)
+    const float *delta, *weight, *weight_ij, *tx, *ty, *tx_half, *ty_half, *tw, *th, *te;
+    const float* grad_loss;             // [5] device (backward)
+    double* partial;                    // [grid][5] workspace (forward)
+    int32_t B, K, W, HW, L;             // L = E * sH * sW * H * W limb elements per image
+    size_t img_stride, limb_off;        // C * HW, 6 * K * HW
+    float gW, gH, inW, inH;
+    long long small_items, limb_chunks, n_items;   // filled by loss_plan
+};
+void loss_plan(LossArgs* a);
+size_t loss_workspace_bytes(const LossArgs& a);
+// two launches: the streaming kernel (CTA partials into a.partial), then the fixed-order sum into loss[5]
+cudaError_t launch_loss_forward(LossArgs a, float* loss, int sms, cudaStream_t st);
+cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st);
+
 }  // namespace ppn

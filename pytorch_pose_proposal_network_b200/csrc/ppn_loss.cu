@@ -1,0 +1,361 @@
+// PPNLoss (the reference's criterion, main.py:125-216) as two fused kernels over the head tensor and the
+// encoded targets, hand-written for sm_100a.
+//
+// The loss of one image, for head channels resp, conf, x, y, w, h (K each) and the limb block e [E, sH, sW, H, W]
+// (specification: the float64 restatement of the test infrastructure, ppn_loss.py; DESIGN.md §11 says which points of it are
+// reconstructed rather than pinned to the reference):
+//   L_resp = sum (resp - delta)^2                 L_iou  = sum delta (conf - iou)^2
+//   L_coor = sum weight ((x - tx_half)^2 + (y - ty_half)^2)
+//   L_size = sum weight ((sqrt(w + eps) - sqrt(tw + eps))^2 + (sqrt(h + eps) - sqrt(th + eps))^2)
+//   L_limb = sum weight_ij (e - te)^2
+// each averaged over the batch (sum / B); eps = 1e-6 (config.EPSILON).
+//
+// Work is split into ITEMS, handed out statically (CTA c takes items c, c + grid, ...):
+//   small items   1024 cells of the [B, K, H, W] planes: a thread takes whole cells, because the IoU needs all four
+//                 box planes of a cell (6 head values and 8 targets in, 4 loss terms or 6 gradients out);
+//   limb items    8192 consecutive elements of one image's limb block, streamed with 128-bit loads (and, backward,
+//                 128-bit streaming stores) where the head, te, weight_ij (and grad) of that image sit at the same
+//                 phase within 16 bytes, element by element where they do not (only grids with an odd H*W or odd K
+//                 produce such images, or tensors whose storage starts mid-vector).
+// The limb block is 98.6 % of the bytes at the native shape: the kernels are HBM streams with a little arithmetic.
+//
+// Forward: every thread accumulates its terms in fp64 (each fp32 term converted exactly); a CTA reduces its threads
+// in a fixed butterfly order and stores 5 doubles into the caller's workspace; a one-CTA kernel sums the CTA
+// partials in a fixed order and writes loss[t] = (float)(sum_t / B).  No float atomics: the same inputs on the same
+// device give the same bits.
+//
+// Backward: recomputes everything from the inputs (nothing is saved by the forward) and writes every element of
+// grad_head once.  fp32, one rounding per operation (__f*_rn, no FMA contraction; the build also has -fmad=false),
+// in exactly this order (grad_model_f32 of the test infrastructure is the same sequence in numpy float32):
+//   with g = grad_loss[5] (device) and Bf = (float)B:
+//     cr = (2 * g0) / Bf   ci = (2 * g1) / Bf   cc = (2 * g2) / Bf   cs = g3 / Bf   cl = (2 * g4) / Bf
+//   limb     grad = cl * (weight_ij * (e - te))
+//   resp     grad = cr * (resp - delta)
+//   IoU of the cell (column X, row Y as floats):
+//     px = (x + X) * gW   py = (y + Y) * gH   pw = inW * w   ph = inH * h      (q.. likewise from tx, ty, tw, th)
+//     px1 = px - pw * 0.5   px2 = px + pw * 0.5   (qx1, qx2, py1, ... likewise)
+//     iwr = min(px2, qx2) - max(px1, qx1)   iw = iwr > 0 ? iwr : 0          (ihr, ih likewise in y)
+//     I = iw * ih   U = ((pw * ph + qw * qh) - I) + eps   iou = I / U
+//   conf     a = ci * (delta * (conf - iou));  grad = a
+//   IoU chain, from diou = -a:
+//     r = diou / U   ri = r * iou   dI = r + ri                                 (d iou/dI = 1/U + I/U^2)
+//     giw = iwr > 0 ? dI * ih : 0   gih = ihr > 0 ? dI * iw : 0                 (relu'(0) = 0)
+//     s2 = px2 < qx2 ? 1 : px2 == qx2 ? 0.5 : 0   s1 = px1 > qx1 ? 1 : px1 == qx1 ? 0.5 : 0   (ties split evenly)
+//     dpx2 = giw * s2   dpx1 = -(giw * s1)   dpx = dpx2 + dpx1   dpw = (dpx2 - dpx1) * 0.5 - ri * ph
+//     (y: the same with gih, py*, qy*; dph = (dpy2 - dpy1) * 0.5 - ri * pw)
+//   x        grad = cc * (weight * (x - tx_half)) + dpx * gW                    (y likewise with ty_half, dpy, gH)
+//   w        sw = sqrt(w + eps)   st = sqrt(tw + eps);  grad = cs * (weight * ((sw - st) / sw)) + dpw * inW
+//                                                                               (h likewise with th, dph, inH)
+// min / max are fminf / fmaxf: the inputs are taken to be finite (a NaN head is not a training state).
+#include <algorithm>
+#include <atomic>
+
+#include "ppn_kernels.h"
+
+namespace ppn {
+
+namespace {
+
+constexpr int kLossThreads = 256;
+constexpr int kSmallCells = 1024;      // cells of the [B, K, H, W] planes per small item
+constexpr int kLimbChunk = 8192;       // limb elements per limb item: 32 KB of each stream
+constexpr int kLimbUnroll = 4;         // float4 iterations whose loads a thread issues before it computes
+constexpr float kEps = 1e-6f;          // config.EPSILON
+
+__device__ __forceinline__ float lds(const float* p) {     // streaming scalar load, no L1 allocation
+    float v;
+    asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
+    return v;
+}
+
+__device__ __forceinline__ unsigned phase_of(const float* p) { return (unsigned)(reinterpret_cast<uintptr_t>(p) >> 2) & 3u; }
+
+struct Cell {
+    float resp, conf, x, y, w, h;                           // head
+    float delta, weight, txh, tyh, tx, ty, tw, th;          // targets
+};
+
+__device__ __forceinline__ Cell load_cell(const LossArgs& a, long long i) {
+    const long long KHW = (long long)a.K * a.HW;
+    const long long b = i / KHW, r = i - b * KHW;
+    const float* img = a.head + (size_t)b * a.img_stride + (size_t)r;
+    const size_t KH = (size_t)KHW;
+    Cell c;
+    c.resp = lds(img);          c.conf = lds(img + KH);     c.x = lds(img + 2 * KH);
+    c.y = lds(img + 3 * KH);    c.w = lds(img + 4 * KH);    c.h = lds(img + 5 * KH);
+    c.delta = lds(a.delta + i); c.weight = lds(a.weight + i);
+    c.txh = lds(a.tx_half + i); c.tyh = lds(a.ty_half + i);
+    c.tx = lds(a.tx + i);       c.ty = lds(a.ty + i);       c.tw = lds(a.tw + i);       c.th = lds(a.th + i);
+    return c;
+}
+
+struct Box {
+    float p1, p2, q1, q2;       // predicted / target interval along one axis
+    float size, qsize, r, i;    // predicted / target extent (pw, qw or ph, qh), raw and relu'd intersection
+};
+
+__device__ __forceinline__ Box axis(float v, float t, float sz, float tsz, float pos, float grid, float in) {
+    Box o;
+    const float p = __fmul_rn(__fadd_rn(v, pos), grid), q = __fmul_rn(__fadd_rn(t, pos), grid);
+    o.size = __fmul_rn(in, sz);
+    o.qsize = __fmul_rn(in, tsz);
+    const float hp = __fmul_rn(o.size, 0.5f), hq = __fmul_rn(o.qsize, 0.5f);
+    o.p1 = __fsub_rn(p, hp); o.p2 = __fadd_rn(p, hp);
+    o.q1 = __fsub_rn(q, hq); o.q2 = __fadd_rn(q, hq);
+    o.r = __fsub_rn(fminf(o.p2, o.q2), fmaxf(o.p1, o.q1));
+    o.i = o.r > 0.0f ? o.r : 0.0f;
+    return o;
+}
+
+struct Iou { Box x, y; float I, U, iou; };
+
+__device__ __forceinline__ Iou iou_of(const LossArgs& a, const Cell& c, long long i) {
+    const int cell = (int)(i % a.HW);
+    const int row = cell / a.W, col = cell - row * a.W;
+    Iou o;
+    o.x = axis(c.x, c.tx, c.w, c.tw, (float)col, a.gW, a.inW);
+    o.y = axis(c.y, c.ty, c.h, c.th, (float)row, a.gH, a.inH);
+    o.I = __fmul_rn(o.x.i, o.y.i);
+    o.U = __fadd_rn(__fsub_rn(__fadd_rn(__fmul_rn(o.x.size, o.y.size), __fmul_rn(o.x.qsize, o.y.qsize)), o.I), kEps);
+    o.iou = __fdiv_rn(o.I, o.U);
+    return o;
+}
+
+// d(loss)/d(p1), d(loss)/d(p2) of one axis and the resulting gradient of its position and extent (before the
+// area term), from the gradient `gi` of the relu'd intersection
+__device__ __forceinline__ void axis_grad(const Box& b, float gi, float* d_pos, float* d_size_half) {
+    const float s2 = b.p2 < b.q2 ? 1.0f : (b.p2 == b.q2 ? 0.5f : 0.0f);
+    const float s1 = b.p1 > b.q1 ? 1.0f : (b.p1 == b.q1 ? 0.5f : 0.0f);
+    const float d2 = __fmul_rn(gi, s2);
+    const float d1 = -__fmul_rn(gi, s1);
+    *d_pos = __fadd_rn(d2, d1);
+    *d_size_half = __fmul_rn(__fsub_rn(d2, d1), 0.5f);
+}
+
+__device__ __forceinline__ float sq(float v) { return __fmul_rn(v, v); }
+
+// ---- the limb block of one item ---------------------------------------------------------------------------------
+struct LimbItem { const float *hp, *tp, *wp; float* gp; int start, end, pro; bool vec; };
+
+__device__ __forceinline__ LimbItem limb_item(const LossArgs& a, long long j, bool backward) {
+    const long long b = j / a.limb_chunks;
+    const int q = (int)(j - b * a.limb_chunks);
+    LimbItem it;
+    it.hp = a.head + (size_t)b * a.img_stride + a.limb_off;
+    it.tp = a.te + (size_t)b * a.L;
+    it.wp = a.weight_ij + (size_t)b * a.L;
+    it.gp = backward ? a.grad + (size_t)b * a.img_stride + a.limb_off : nullptr;
+    const unsigned ph = phase_of(it.hp);
+    it.vec = phase_of(it.tp) == ph && phase_of(it.wp) == ph && (!backward || phase_of(it.gp) == ph);
+    const int a0 = it.vec ? min(a.L, (int)((4u - ph) & 3u)) : 0;       // elements before the first aligned vector
+    it.pro = q == 0 ? a0 : 0;                                            // chunk 0 also takes those
+    it.start = min(a.L, a0 + q * kLimbChunk);
+    it.end = min(a.L, it.start + kLimbChunk);
+    return it;
+}
+
+__device__ __forceinline__ float limb_term(float e, float t, float w) { return __fmul_rn(w, sq(__fsub_rn(e, t))); }
+__device__ __forceinline__ float limb_grad(float cl, float e, float t, float w) {
+    return __fmul_rn(cl, __fmul_rn(w, __fsub_rn(e, t)));
+}
+
+// deterministic CTA sum of 5 doubles; thread 0..4 store the CTA's partials
+__device__ __forceinline__ void cta_store(double acc[5], double* out) {
+    __shared__ double s[kLossThreads / 32][5];
+#pragma unroll
+    for (int t = 0; t < 5; ++t)
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc[t] += __shfl_xor_sync(0xffffffffu, acc[t], o);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (lane == 0)
+#pragma unroll
+        for (int t = 0; t < 5; ++t) s[warp][t] = acc[t];
+    __syncthreads();
+    if (threadIdx.x < 5) {
+        double v = 0.0;
+        for (int w = 0; w < kLossThreads / 32; ++w) v += s[w][threadIdx.x];
+        out[(size_t)blockIdx.x * 5 + threadIdx.x] = v;
+    }
+}
+
+__global__ void __launch_bounds__(kLossThreads)
+loss_forward_kernel(LossArgs a) {
+    double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    const int tid = threadIdx.x;
+    const long long n_cells = (long long)a.B * a.K * a.HW;
+    for (long long j = blockIdx.x; j < a.n_items; j += gridDim.x) {
+        if (j < a.small_items) {
+            const long long c1 = min(n_cells, (j + 1) * kSmallCells);
+            for (long long i = j * kSmallCells + tid; i < c1; i += kLossThreads) {
+                const Cell c = load_cell(a, i);
+                const Iou u = iou_of(a, c, i);
+                acc[0] += (double)sq(__fsub_rn(c.resp, c.delta));
+                acc[1] += (double)__fmul_rn(c.delta, sq(__fsub_rn(c.conf, u.iou)));
+                acc[2] += (double)__fmul_rn(c.weight, __fadd_rn(sq(__fsub_rn(c.x, c.txh)), sq(__fsub_rn(c.y, c.tyh))));
+                const float dw = __fsub_rn(__fsqrt_rn(__fadd_rn(c.w, kEps)), __fsqrt_rn(__fadd_rn(c.tw, kEps)));
+                const float dh = __fsub_rn(__fsqrt_rn(__fadd_rn(c.h, kEps)), __fsqrt_rn(__fadd_rn(c.th, kEps)));
+                acc[3] += (double)__fmul_rn(c.weight, __fadd_rn(sq(dw), sq(dh)));
+            }
+            continue;
+        }
+        const LimbItem it = limb_item(a, j - a.small_items, false);
+        if (tid < it.pro) acc[4] += (double)limb_term(lds(it.hp + tid), lds(it.tp + tid), lds(it.wp + tid));
+        int s0 = it.start;
+        if (it.vec) {
+            const int nv = (it.end - it.start) >> 2;
+            const float4* h4 = reinterpret_cast<const float4*>(it.hp + it.start);
+            const float4* t4 = reinterpret_cast<const float4*>(it.tp + it.start);
+            const float4* w4 = reinterpret_cast<const float4*>(it.wp + it.start);
+            for (int v0 = tid; v0 < nv; v0 += kLimbUnroll * kLossThreads) {
+                float4 hv[kLimbUnroll], tv[kLimbUnroll], wv[kLimbUnroll];
+#pragma unroll
+                for (int u = 0; u < kLimbUnroll; ++u) {
+                    const int v = v0 + u * kLossThreads;
+                    if (v < nv) { hv[u] = ldg_stream(h4 + v); tv[u] = ldg_stream(t4 + v); wv[u] = ldg_stream(w4 + v); }
+                }
+#pragma unroll
+                for (int u = 0; u < kLimbUnroll; ++u) {
+                    if (v0 + u * kLossThreads < nv) {
+                        acc[4] += (double)limb_term(hv[u].x, tv[u].x, wv[u].x);
+                        acc[4] += (double)limb_term(hv[u].y, tv[u].y, wv[u].y);
+                        acc[4] += (double)limb_term(hv[u].z, tv[u].z, wv[u].z);
+                        acc[4] += (double)limb_term(hv[u].w, tv[u].w, wv[u].w);
+                    }
+                }
+            }
+            s0 = it.start + 4 * nv;
+        }
+        for (int e = s0 + tid; e < it.end; e += kLossThreads)             // vector tail, or the whole unaligned item
+            acc[4] += (double)limb_term(lds(it.hp + e), lds(it.tp + e), lds(it.wp + e));
+    }
+    cta_store(acc, a.partial);
+}
+
+// loss[t] = (float)(sum over CTAs of partial[cta][t] / B): warp t sums term t, lanes in a fixed stride, then a
+// fixed butterfly
+__global__ void __launch_bounds__(160)
+loss_finalize_kernel(const double* __restrict__ partial, int n, int B, float* __restrict__ loss) {
+    const int t = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    double v = 0.0;
+    for (int i = lane; i < n; i += 32) v += partial[(size_t)i * 5 + t];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) loss[t] = (float)(v / (double)B);
+}
+
+__global__ void __launch_bounds__(kLossThreads)
+loss_backward_kernel(LossArgs a) {
+    const float Bf = (float)a.B;
+    const float cr = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[0]), Bf);
+    const float ci = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[1]), Bf);
+    const float cc = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[2]), Bf);
+    const float cs = __fdiv_rn(a.grad_loss[3], Bf);
+    const float cl = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[4]), Bf);
+    const int tid = threadIdx.x;
+    const long long n_cells = (long long)a.B * a.K * a.HW;
+    const long long KHW = (long long)a.K * a.HW;
+    for (long long j = blockIdx.x; j < a.n_items; j += gridDim.x) {
+        if (j < a.small_items) {
+            const long long c1 = min(n_cells, (j + 1) * kSmallCells);
+            for (long long i = j * kSmallCells + tid; i < c1; i += kLossThreads) {
+                const Cell c = load_cell(a, i);
+                const Iou u = iou_of(a, c, i);
+                const float g_resp = __fmul_rn(cr, __fsub_rn(c.resp, c.delta));
+                const float g_conf = __fmul_rn(ci, __fmul_rn(c.delta, __fsub_rn(c.conf, u.iou)));
+                const float diou = -g_conf;
+                const float r = __fdiv_rn(diou, u.U);
+                const float ri = __fmul_rn(r, u.iou);
+                const float dI = __fadd_rn(r, ri);
+                const float giw = u.x.r > 0.0f ? __fmul_rn(dI, u.y.i) : 0.0f;
+                const float gih = u.y.r > 0.0f ? __fmul_rn(dI, u.x.i) : 0.0f;
+                float dpx, dpw, dpy, dph;
+                axis_grad(u.x, giw, &dpx, &dpw);
+                axis_grad(u.y, gih, &dpy, &dph);
+                dpw = __fsub_rn(dpw, __fmul_rn(ri, u.y.size));
+                dph = __fsub_rn(dph, __fmul_rn(ri, u.x.size));
+                const float g_x = __fadd_rn(__fmul_rn(cc, __fmul_rn(c.weight, __fsub_rn(c.x, c.txh))), __fmul_rn(dpx, a.gW));
+                const float g_y = __fadd_rn(__fmul_rn(cc, __fmul_rn(c.weight, __fsub_rn(c.y, c.tyh))), __fmul_rn(dpy, a.gH));
+                const float sw = __fsqrt_rn(__fadd_rn(c.w, kEps)), st = __fsqrt_rn(__fadd_rn(c.tw, kEps));
+                const float sh = __fsqrt_rn(__fadd_rn(c.h, kEps)), sth = __fsqrt_rn(__fadd_rn(c.th, kEps));
+                const float g_w = __fadd_rn(__fmul_rn(cs, __fmul_rn(c.weight, __fdiv_rn(__fsub_rn(sw, st), sw))), __fmul_rn(dpw, a.inW));
+                const float g_h = __fadd_rn(__fmul_rn(cs, __fmul_rn(c.weight, __fdiv_rn(__fsub_rn(sh, sth), sh))), __fmul_rn(dph, a.inH));
+                const long long b = i / KHW, rr = i - b * KHW;
+                float* gimg = a.grad + (size_t)b * a.img_stride + (size_t)rr;
+                const size_t KH = (size_t)KHW;
+                __stcs(gimg, g_resp);          __stcs(gimg + KH, g_conf);     __stcs(gimg + 2 * KH, g_x);
+                __stcs(gimg + 3 * KH, g_y);    __stcs(gimg + 4 * KH, g_w);    __stcs(gimg + 5 * KH, g_h);
+            }
+            continue;
+        }
+        const LimbItem it = limb_item(a, j - a.small_items, true);
+        if (tid < it.pro) __stcs(it.gp + tid, limb_grad(cl, lds(it.hp + tid), lds(it.tp + tid), lds(it.wp + tid)));
+        int s0 = it.start;
+        if (it.vec) {
+            const int nv = (it.end - it.start) >> 2;
+            const float4* h4 = reinterpret_cast<const float4*>(it.hp + it.start);
+            const float4* t4 = reinterpret_cast<const float4*>(it.tp + it.start);
+            const float4* w4 = reinterpret_cast<const float4*>(it.wp + it.start);
+            float4* g4 = reinterpret_cast<float4*>(it.gp + it.start);
+            for (int v0 = tid; v0 < nv; v0 += kLimbUnroll * kLossThreads) {
+                float4 hv[kLimbUnroll], tv[kLimbUnroll], wv[kLimbUnroll];
+#pragma unroll
+                for (int u = 0; u < kLimbUnroll; ++u) {
+                    const int v = v0 + u * kLossThreads;
+                    if (v < nv) { hv[u] = ldg_stream(h4 + v); tv[u] = ldg_stream(t4 + v); wv[u] = ldg_stream(w4 + v); }
+                }
+#pragma unroll
+                for (int u = 0; u < kLimbUnroll; ++u) {
+                    const int v = v0 + u * kLossThreads;
+                    if (v < nv)
+                        __stcs(g4 + v, make_float4(limb_grad(cl, hv[u].x, tv[u].x, wv[u].x), limb_grad(cl, hv[u].y, tv[u].y, wv[u].y),
+                                                   limb_grad(cl, hv[u].z, tv[u].z, wv[u].z), limb_grad(cl, hv[u].w, tv[u].w, wv[u].w)));
+                }
+            }
+            s0 = it.start + 4 * nv;
+        }
+        for (int e = s0 + tid; e < it.end; e += kLossThreads)
+            __stcs(it.gp + e, limb_grad(cl, lds(it.hp + e), lds(it.tp + e), lds(it.wp + e)));
+    }
+}
+
+// resident CTAs per SM of each kernel: a property of the compiled kernel, asked once per process
+int grid_for(const void* kernel, std::atomic<int>* per_sm_cache, long long n_items, int sms) {
+    int per_sm = per_sm_cache->load(std::memory_order_relaxed);
+    if (per_sm < 1) {
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kLossThreads, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
+        per_sm_cache->store(per_sm, std::memory_order_relaxed);
+    }
+    return (int)std::min<long long>(n_items, std::min<long long>((long long)sms * per_sm, kLossMaxCtas));
+}
+std::atomic<int> g_forward_per_sm{0}, g_backward_per_sm{0};
+
+}  // namespace
+
+void loss_plan(LossArgs* a) {
+    const long long n_cells = (long long)a->B * a->K * a->HW;
+    a->small_items = (n_cells + kSmallCells - 1) / kSmallCells;
+    a->limb_chunks = a->L > 0 ? (a->L + kLimbChunk - 1) / kLimbChunk : 0;
+    a->n_items = a->small_items + (long long)a->B * a->limb_chunks;
+}
+
+size_t loss_workspace_bytes(const LossArgs& a) {
+    const long long ctas = std::min<long long>(std::max<long long>(a.n_items, 1), kLossMaxCtas);
+    return (size_t)ctas * 5 * sizeof(double);
+}
+
+cudaError_t launch_loss_forward(LossArgs a, float* loss, int sms, cudaStream_t st) {
+    const int grid = grid_for((const void*)loss_forward_kernel, &g_forward_per_sm, a.n_items, sms);
+    loss_forward_kernel<<<grid, kLossThreads, 0, st>>>(a);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    loss_finalize_kernel<<<1, 160, 0, st>>>(a.partial, grid, a.B, loss);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st) {
+    const int grid = grid_for((const void*)loss_backward_kernel, &g_backward_per_sm, a.n_items, sms);
+    loss_backward_kernel<<<grid, kLossThreads, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+}  // namespace ppn
