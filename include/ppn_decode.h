@@ -27,6 +27,7 @@
  *                            KeypointsDataset.__getitem__, dataset.py:89-198, for a whole batch
  *   ppn_loss_forward ....... the consumer of those targets: PPNLoss.forward, main.py:125-216 (five terms)
  *   ppn_loss_backward ...... its autograd backward with respect to the head tensor
+ *   ppn_loss_*_opt ......... the same for fp16 / bf16 heads and limb targets (mixed-precision training)
  *
  * Conventions
  *   - plain C: pointers and sizes only; no CUDA or torch types.  `stream` is a cudaStream_t
@@ -378,6 +379,34 @@ int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets*
                      void* workspace, size_t workspace_bytes, void* stream);
 int ppn_loss_backward(const float* head, const PPNShape* shape, const PPNTargets* targets, const float* grad_loss,
                       float* grad_head, void* stream);
+
+/* ---- mixed precision: 16-bit heads and limb targets (the reference trains under apex AMP, main.py:282-289) -------
+ * The same loss with shape->head_dtype selecting the element type of the head AND of grad_head, and
+ * opt->limb_dtype (a PPN_HEAD_* code) that of targets->te and targets->weight_ij: with a 16-bit limb_dtype those two
+ * pointers point to fp16 / bf16 elements (despite their float* type).  The eight [B, K, H, W] targets stay fp32.
+ * Supported (head, limb targets): (F32, F32), (F16, F32), (F16, F16), (BF16, F32), (BF16, BF16); any other pair
+ * (an fp32 head with 16-bit limb targets, limb targets in the other 16-bit type) is PPN_E_UNSUPPORTED, a limb_dtype
+ * that is no PPN_HEAD_* code PPN_E_BADARG.
+ * Rule: a 16-bit input is widened exactly and the fp32 loss above is applied to it, operation for operation; every
+ * gradient element is rounded once (round to nearest even) to the head's type, overflow giving +-inf.  So the terms
+ * equal ppn_loss_forward on the widened inputs up to the order of the fp64 sums, and grad_head equals
+ * ppn_loss_backward on the widened inputs converted to the head's type, bit for bit.
+ * Pointers need the alignment of their element (2 bytes for 16-bit, 4 for fp32).  The workspace is the same as for
+ * the fp32 loss of the same batch.  The three fp32 exports above keep rejecting 16-bit shapes. */
+typedef struct PPNLossOptions {
+    int32_t limb_dtype;     /* PPN_HEAD_F32, PPN_HEAD_F16 or PPN_HEAD_BF16: element type of te and weight_ij   */
+} PPNLossOptions;
+int ppn_loss_workspace_bytes_opt(const PPNShape* shape, const PPNLossOptions* opt, size_t* bytes);
+int ppn_loss_forward_opt(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                         float* loss, void* workspace, size_t workspace_bytes, void* stream);
+int ppn_loss_backward_opt(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                          const float* grad_loss, void* grad_head, void* stream);
+
+/* ppn_encode_targets writing te and weight_ij as limb_dtype (PPN_HEAD_*; PPN_E_BADARG otherwise): te in {0, 1} is
+ * exact in every type; weight_ij in {1, 0.0005f} stores 0.0005f rounded to nearest even (fp16 0.000500202...,
+ * bf16 0.000499725...).  The eight small grids are fp32 as above; shape->head_dtype is not used. */
+int ppn_encode_targets_opt(const PPNPeople* people, const PPNShape* shape, const int32_t* edges,
+                           const PPNTargets* out, int32_t limb_dtype, void* stream);
 
 #ifdef __cplusplus
 }

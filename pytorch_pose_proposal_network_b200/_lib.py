@@ -58,6 +58,10 @@ class PPNTargets(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in TARGET_NAMES]
 
 
+class PPNLossOptions(C.Structure):
+    _fields_ = [("limb_dtype", C.c_int32)]
+
+
 # name -> (restype, argtypes); must list every function of include/ppn_decode.h
 EXPORTS = {
     "ppn_abi_version": (C.c_int, []),
@@ -114,6 +118,13 @@ EXPORTS = {
                                    C.c_size_t, C.c_void_p]),
     "ppn_loss_backward": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.c_void_p, C.c_void_p,
                                     C.c_void_p]),
+    "ppn_loss_workspace_bytes_opt": (C.c_int, [C.POINTER(PPNShape), C.POINTER(PPNLossOptions), C.POINTER(C.c_size_t)]),
+    "ppn_loss_forward_opt": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.POINTER(PPNLossOptions),
+                                       C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ppn_loss_backward_opt": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.POINTER(PPNLossOptions),
+                                        C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ppn_encode_targets_opt": (C.c_int, [C.POINTER(PPNPeople), C.POINTER(PPNShape), i32p, C.POINTER(PPNTargets), C.c_int32,
+                                         C.c_void_p]),
     "ppn_debug_argmax_items": (C.c_int, [C.POINTER(PPNShape), C.c_int32, i32p, i32p, i32p, C.c_int32]),
     "ppn_timeline": (C.c_int, [C.c_void_p, C.c_int32]),
     "ppn_profile_enable": (C.c_int, [C.c_int32]),

@@ -954,10 +954,16 @@ int ppn_pack_humans(const PPNHumans* humans, int32_t B, int32_t K, int32_t cap_e
 
 int ppn_encode_targets(const PPNPeople* people, const PPNShape* shape, const int32_t* edges,
                        const PPNTargets* out, void* stream) {
+    return ppn_encode_targets_opt(people, shape, edges, out, PPN_HEAD_F32, stream);
+}
+
+int ppn_encode_targets_opt(const PPNPeople* people, const PPNShape* shape, const int32_t* edges,
+                           const PPNTargets* out, int32_t limb_dtype, void* stream) {
     const ppn::Tuning g_tuning = tuning_now();
     int rc = check_shape(shape);
     if (rc) return rc;
     if (!people || !out) return PPN_E_BADARG;
+    if (limb_dtype < PPN_HEAD_F32 || limb_dtype > PPN_HEAD_BF16) return PPN_E_BADARG;
     if (shape->gridW < 1 || shape->gridH < 1) return PPN_E_BADARG;                     // the encoder divides by them
     if (shape->sH != shape->sW || (shape->sH & 1) == 0) return PPN_E_UNSUPPORTED;      // dataset.py:163-167
     if (shape->B == 0) return PPN_OK;
@@ -977,6 +983,7 @@ int ppn_encode_targets(const PPNPeople* people, const PPNShape* shape, const int
     a.visible = people->visible; a.size = people->size;
     a.delta = out->delta; a.weight = out->weight; a.weight_ij = out->weight_ij; a.tx = out->tx; a.ty = out->ty;
     a.tx_half = out->tx_half; a.ty_half = out->ty_half; a.tw = out->tw; a.th = out->th; a.te = out->te;
+    a.limb_dtype = limb_dtype;
     a.K = shape->K; a.E = shape->E; a.H = shape->H; a.W = shape->W; a.sH = shape->sH; a.sW = shape->sW;
     a.sweep = g_tuning.encode_sweep;
     a.sweep_ctas_per_sm = g_tuning.encode_ctas_per_sm;
@@ -992,24 +999,37 @@ int ppn_encode_targets(const PPNPeople* people, const PPNShape* shape, const int
 
 // ---- the training loss (PPNLoss, main.py:125-216) -----------------------------------------------------
 namespace {
-inline bool bad_f32(const void* p) { return !p || (reinterpret_cast<uintptr_t>(p) & 3); }
+inline bool bad_ptr(const void* p, size_t align) { return !p || (reinterpret_cast<uintptr_t>(p) & (align - 1)); }
+inline bool bad_f32(const void* p) { return bad_ptr(p, 4); }
+inline size_t dtype_bytes(int32_t dtype) { return dtype == PPN_HEAD_F32 ? 4 : 2; }
 
-int loss_args(const float* head, const PPNShape* shape, const PPNTargets* t, ppn::LossArgs* a) {
+// the (head, limb target) element types the kernels are built for: limb targets fp32 or the head's type
+int check_loss_types(const PPNShape* shape, const PPNLossOptions* opt) {
+    if (!opt || opt->limb_dtype < PPN_HEAD_F32 || opt->limb_dtype > PPN_HEAD_BF16) return PPN_E_BADARG;
+    if (opt->limb_dtype != PPN_HEAD_F32 && opt->limb_dtype != shape->head_dtype) return PPN_E_UNSUPPORTED;
+    return PPN_OK;
+}
+
+int loss_args(const void* head, const PPNShape* shape, const PPNTargets* t, const PPNLossOptions* opt, ppn::LossArgs* a) {
     int rc = check_shape(shape);
     if (rc) return rc;
-    if (shape->head_dtype != PPN_HEAD_F32) return PPN_E_UNSUPPORTED;
+    if ((rc = check_loss_types(shape, opt))) return rc;
     if (shape->B < 1) return PPN_E_BADARG;                                   // the batch mean needs an image
     std::memset(a, 0, sizeof(*a));
     const ppn::Geom g = make_geom(shape);
     a->B = g.B; a->K = g.K; a->W = g.W; a->HW = g.HW; a->L = g.S * g.E * g.HW;
     a->img_stride = g.img_stride; a->limb_off = g.limb_off;
     a->gW = g.gridW; a->gH = g.gridH; a->inW = g.inW; a->inH = g.inH;
+    a->head_dtype = shape->head_dtype;
+    a->limb_dtype = opt->limb_dtype;
     ppn::loss_plan(a);
     if (!t) return PPN_E_BADARG;
     const float* small[] = {t->delta, t->weight, t->tx, t->ty, t->tx_half, t->ty_half, t->tw, t->th};
     for (const float* p : small)
         if (bad_f32(p)) return PPN_E_BADARG;
-    if (bad_f32(head) || (a->L > 0 && (bad_f32(t->te) || bad_f32(t->weight_ij)))) return PPN_E_BADARG;
+    const size_t limb_align = dtype_bytes(opt->limb_dtype);
+    if (bad_ptr(head, elem_bytes(shape)) || (a->L > 0 && (bad_ptr(t->te, limb_align) || bad_ptr(t->weight_ij, limb_align))))
+        return PPN_E_BADARG;
     a->head = head;
     a->delta = t->delta; a->weight = t->weight; a->weight_ij = t->weight_ij; a->tx = t->tx; a->ty = t->ty;
     a->tx_half = t->tx_half; a->ty_half = t->ty_half; a->tw = t->tw; a->th = t->th; a->te = t->te;
@@ -1022,13 +1042,21 @@ int sm_count(int* sms) {
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
     return cuda_rc(e);
 }
+
+// the fp32 exports: fp32 head and targets only, as before the 16-bit path existed
+const PPNLossOptions kLossF32 = {PPN_HEAD_F32};
+int check_f32_loss(const PPNShape* shape) {
+    int rc = check_shape(shape);
+    if (rc) return rc;
+    return shape->head_dtype != PPN_HEAD_F32 ? PPN_E_UNSUPPORTED : PPN_OK;
+}
 }  // namespace
 
-int ppn_loss_workspace_bytes(const PPNShape* shape, size_t* bytes) {
+int ppn_loss_workspace_bytes_opt(const PPNShape* shape, const PPNLossOptions* opt, size_t* bytes) {
     int rc = check_shape(shape);
     if (rc) return rc;
     if (!bytes) return PPN_E_BADARG;
-    if (shape->head_dtype != PPN_HEAD_F32) return PPN_E_UNSUPPORTED;
+    if ((rc = check_loss_types(shape, opt))) return rc;
     if (shape->B < 1) return PPN_E_BADARG;
     ppn::LossArgs a;
     std::memset(&a, 0, sizeof(a));
@@ -1038,11 +1066,19 @@ int ppn_loss_workspace_bytes(const PPNShape* shape, size_t* bytes) {
     return PPN_OK;
 }
 
+int ppn_loss_workspace_bytes(const PPNShape* shape, size_t* bytes) {
+    int rc = check_shape(shape);
+    if (rc) return rc;
+    if (!bytes) return PPN_E_BADARG;
+    if ((rc = check_f32_loss(shape))) return rc;
+    return ppn_loss_workspace_bytes_opt(shape, &kLossF32, bytes);
+}
+
 // PPNLoss.forward (main.py:125-216): the five batch-mean terms into loss[5]
-int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets* targets, float* loss,
-                     void* workspace, size_t workspace_bytes, void* stream) {
+int ppn_loss_forward_opt(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                         float* loss, void* workspace, size_t workspace_bytes, void* stream) {
     ppn::LossArgs a;
-    int rc = loss_args(head, shape, targets, &a);
+    int rc = loss_args(head, shape, targets, opt, &a);
     if (rc) return rc;
     if (bad_f32(loss) || !workspace || (reinterpret_cast<uintptr_t>(workspace) & 7)) return PPN_E_BADARG;
     if (workspace_bytes < ppn::loss_workspace_bytes(a)) return PPN_E_WORKSPACE;
@@ -1052,18 +1088,30 @@ int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets*
     return cuda_rc(ppn::launch_loss_forward(a, loss, sms, (cudaStream_t)stream));
 }
 
+int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets* targets, float* loss,
+                     void* workspace, size_t workspace_bytes, void* stream) {
+    const int rc = check_f32_loss(shape);
+    return rc ? rc : ppn_loss_forward_opt(head, shape, targets, &kLossF32, loss, workspace, workspace_bytes, stream);
+}
+
 // PPNLoss's backward under autograd (loss.backward() in main.py's training step), with respect to the head only
-int ppn_loss_backward(const float* head, const PPNShape* shape, const PPNTargets* targets, const float* grad_loss,
-                      float* grad_head, void* stream) {
+int ppn_loss_backward_opt(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                          const float* grad_loss, void* grad_head, void* stream) {
     ppn::LossArgs a;
-    int rc = loss_args(head, shape, targets, &a);
+    int rc = loss_args(head, shape, targets, opt, &a);
     if (rc) return rc;
-    if (bad_f32(grad_loss) || bad_f32(grad_head)) return PPN_E_BADARG;
+    if (bad_f32(grad_loss) || bad_ptr(grad_head, elem_bytes(shape))) return PPN_E_BADARG;
     a.grad_loss = grad_loss;
     a.grad = grad_head;
     int sms = 0;
     if ((rc = sm_count(&sms))) return rc;
     return cuda_rc(ppn::launch_loss_backward(a, sms, (cudaStream_t)stream));
+}
+
+int ppn_loss_backward(const float* head, const PPNShape* shape, const PPNTargets* targets, const float* grad_loss,
+                      float* grad_head, void* stream) {
+    const int rc = check_f32_loss(shape);
+    return rc ? rc : ppn_loss_backward_opt(head, shape, targets, &kLossF32, grad_loss, grad_head, stream);
 }
 
 int ppn_debug_argmax_items(const PPNShape* shape, int32_t sms, int32_t* info, int32_t* first, int32_t* size, int32_t max_items) {

@@ -79,6 +79,17 @@ __device__ __forceinline__ float widen(__nv_bfloat16 v) { return __bfloat162floa
 template <typename T>
 __device__ __forceinline__ float ldf(const T* p) { return widen(__ldg(p)); }      // read-only path + widen
 
+// fp32 -> the element type, rounded once to nearest even; beyond the type's range +-inf (torch's .to())
+template <typename T> __device__ __forceinline__ T narrow(float v) { return v; }
+template <> __device__ __forceinline__ __half narrow<__half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 narrow<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+__device__ __forceinline__ uint32_t bits16(__half v) { return __half_as_ushort(v); }
+__device__ __forceinline__ uint32_t bits16(__nv_bfloat16 v) { return __bfloat16_as_ushort(v); }
+// two narrowed values as one 32-bit word, `lo` at the lower address
+template <typename T> __device__ __forceinline__ uint32_t pack2(float lo, float hi) {
+    return bits16(narrow<T>(lo)) | (bits16(narrow<T>(hi)) << 16);
+}
+
 // ---- the reference's cell arithmetic --------------------------------------------------
 // delta = resp * conf  (rt_test.py:130)
 template <typename T>

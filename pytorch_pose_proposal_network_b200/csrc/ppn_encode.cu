@@ -9,9 +9,9 @@
 //                                                      (max(delta_s at the cell, delta_t at the displaced cell))
 // te and weight_ij are the same size as the head's limb block, i.e. > 92 % of all bytes: the kernel is
 // WRITE-bound and built around that — every element of the two big tensors is written exactly once with
-// 128-bit streaming stores by the CTA that owns its (limb, dy, dx) rows, weight_ij computed on the fly from a
-// per-image byte map of delta kept in shared memory; the few one-hots of te are set afterwards by the same
-// CTA (ordered by a barrier).  In the reference this is ~70 lines of Python per image inside the DataLoader,
+// 128-bit (64-bit when the two are fp16 / bf16) streaming stores by the CTA that owns its (limb, dy, dx) rows,
+// weight_ij computed on the fly from a per-image byte map of delta kept in shared memory; the few one-hots of te
+// are set afterwards by the same CTA (ordered by a barrier).  In the reference this is ~70 lines of Python per image inside the DataLoader,
 // the O(E*H*W) window loop of dataset.py:155-168 among them.
 //
 // Exactness (the reference's types: key points fp32 tensors, box float64 tensor, part size a Python float):
@@ -48,6 +48,14 @@ __device__ __forceinline__ EncPoint enc_point(const EncodeArgs& a, int p, int k)
     return r;
 }
 
+// four consecutive limb-tensor elements (p: 16-byte aligned for fp32, 8-byte for 16 bits), one streaming store
+__device__ __forceinline__ void st4(float* p, const float (&v)[4]) { __stcs(reinterpret_cast<float4*>(p), make_float4(v[0], v[1], v[2], v[3])); }
+template <typename T> __device__ __forceinline__ void st4(T* p, const float (&v)[4]) {
+    __stcs(reinterpret_cast<uint2*>(p), make_uint2(pack2<T>(v[0], v[1]), pack2<T>(v[2], v[3])));
+}
+
+// TL: the element type of te and weight_ij (float, __half or __nv_bfloat16); the eight small grids are fp32
+template <typename TL>
 __global__ void __launch_bounds__(256)
 encode_targets_kernel(EncodeArgs a) {
     extern __shared__ __align__(16) unsigned char s_delta[];              // [K * HW] 0 / 1
@@ -97,6 +105,9 @@ encode_targets_kernel(EncodeArgs a) {
     }
 
     if (a.small_only) return;                         // the two limb tensors come from encode_sweep_kernel
+    TL* const te = static_cast<TL*>(a.te);
+    TL* const weight_ij = static_cast<TL*>(a.weight_ij);
+    const float zeros[4] = {0.f, 0.f, 0.f, 0.f};
     // ---- this CTA's rows of te (zeros) and weight_ij, each element written once -------------------------
     const int rows = a.E * S;
     const int r0 = z * a.rows_per_cta, r1 = min(rows, r0 + a.rows_per_cta);
@@ -126,8 +137,8 @@ encode_targets_kernel(EncodeArgs a) {
                     const bool on = ((ds4 >> (8 * q)) & 0xffu) || (row_in && ww >= 0 && ww < a.W && dt[hh * a.W + ww]);
                     v[q] = on ? 1.0f : 0.0005f;                          // dataset.py:154-175
                 }
-                __stcs(reinterpret_cast<float4*>(a.weight_ij + big + (size_t)r * HW + c), make_float4(v[0], v[1], v[2], v[3]));
-                __stcs(reinterpret_cast<float4*>(a.te + big + (size_t)r * HW + c), make_float4(0.f, 0.f, 0.f, 0.f));
+                st4(weight_ij + big + (size_t)r * HW + c, v);
+                st4(te + big + (size_t)r * HW + c, zeros);
                 wa += RL;
                 while (wa >= S) { wa -= S; ++ei; }
             }
@@ -139,8 +150,8 @@ encode_targets_kernel(EncodeArgs a) {
             const int h = c / a.W, w = c - h * a.W, hh = h + dy - oh, ww = w + dx - ow;
             const bool on = s_delta[a.edges.src[ei] * HW + c] ||
                             (hh >= 0 && hh < a.H && ww >= 0 && ww < a.W && s_delta[a.edges.dst[ei] * HW + hh * a.W + ww]);
-            a.weight_ij[big + (size_t)r * HW + c] = on ? 1.0f : 0.0005f;
-            a.te[big + (size_t)r * HW + c] = 0.0f;
+            weight_ij[big + (size_t)r * HW + c] = narrow<TL>(on ? 1.0f : 0.0005f);
+            te[big + (size_t)r * HW + c] = narrow<TL>(0.0f);
         }
     }
     __syncthreads();                                  // the zeros of this CTA's rows are ordered before its ones
@@ -156,7 +167,7 @@ encode_targets_kernel(EncodeArgs a) {
         const long long jy = (long long)t.iy - s.iy + oh, jx = (long long)t.ix - s.ix + ow;
         if (jy < 0 || jx < 0 || jy >= a.sH || jx >= a.sW) continue;
         const int r = (ei * a.sH + (int)jy) * a.sW + (int)jx;
-        if (r >= r0 && r < r1) a.te[big + (size_t)r * HW + s.iy * a.W + s.ix] = 1.0f;
+        if (r >= r0 && r < r1) te[big + (size_t)r * HW + s.iy * a.W + s.ix] = narrow<TL>(1.0f);
     }
 }
 
@@ -166,6 +177,7 @@ encode_targets_kernel(EncodeArgs a) {
 // plain fill, which is what DRAM write-back wants (with one CTA per (image, half of the rows) there were
 // ~1 800 slow write streams spread over the whole tensors: 4.4 TB/s; a fill reaches 6.9).  Per tile the CTA
 // rebuilds just the two delta planes it needs (the limb's source and target part) from the image's people.
+template <typename TL>
 __global__ void __launch_bounds__(256)
 encode_sweep_kernel(EncodeArgs a, int B, int chunks, int rows_per_tile) {
     extern __shared__ __align__(16) unsigned char s_planes[];              // [2][HW]: delta of the source / target part
@@ -176,6 +188,9 @@ encode_sweep_kernel(EncodeArgs a, int B, int chunks, int rows_per_tile) {
     const int oh = a.sH / 2, ow = a.sW / 2;
     unsigned char* ds = s_planes;
     unsigned char* dt = s_planes + HW;
+    TL* const te = static_cast<TL*>(a.te);
+    TL* const weight_ij = static_cast<TL*>(a.weight_ij);
+    const float zeros[4] = {0.f, 0.f, 0.f, 0.f};
     const long long n_tiles = (long long)B * a.E * chunks;
     for (long long t = blockIdx.x; t < n_tiles; t += gridDim.x) {
         const int ch = (int)(t % chunks);
@@ -207,8 +222,8 @@ encode_sweep_kernel(EncodeArgs a, int B, int chunks, int rows_per_tile) {
                     const bool on = ((ds4 >> (8 * q)) & 0xffu) || (row_in && ww >= 0 && ww < a.W && dt[hh * a.W + ww]);
                     v[q] = on ? 1.0f : 0.0005f;                              // dataset.py:154-175
                 }
-                __stcs(reinterpret_cast<float4*>(a.weight_ij + base + (size_t)wa * HW + c), make_float4(v[0], v[1], v[2], v[3]));
-                __stcs(reinterpret_cast<float4*>(a.te + base + (size_t)wa * HW + c), make_float4(0.f, 0.f, 0.f, 0.f));
+                st4(weight_ij + base + (size_t)wa * HW + c, v);
+                st4(te + base + (size_t)wa * HW + c, zeros);
             }
         }
         __syncthreads();                              // the zeros of this tile are ordered before its ones
@@ -221,13 +236,13 @@ encode_sweep_kernel(EncodeArgs a, int B, int chunks, int rows_per_tile) {
             const long long jy = (long long)q.iy - s.iy + oh, jx = (long long)q.ix - s.ix + ow;
             if (jy < 0 || jx < 0 || jy >= a.sH || jx >= a.sW) continue;
             const int wa = (int)jy * a.sW + (int)jx;
-            if (wa >= wa0 && wa < wa1) a.te[base + (size_t)wa * HW + s.iy * a.W + s.ix] = 1.0f;
+            if (wa >= wa0 && wa < wa1) te[base + (size_t)wa * HW + s.iy * a.W + s.ix] = narrow<TL>(1.0f);
         }
     }
 }
 
-cudaError_t launch_encode_targets(EncodeArgs a, int B, int sms, cudaStream_t st) {
-    if (B == 0) return cudaSuccess;
+template <typename TL>
+cudaError_t encode_as(EncodeArgs a, int B, int sms, cudaStream_t st) {
     const int rows = a.E * a.sH * a.sW;
     const int HW = a.H * a.W, S = a.sH * a.sW;
     const size_t smem_small = ((size_t)a.K * HW + 15) & ~(size_t)15;
@@ -236,21 +251,21 @@ cudaError_t launch_encode_targets(EncodeArgs a, int B, int sms, cudaStream_t st)
         EncodeArgs small = a;
         small.small_only = 1;
         if (smem_small > 48 * 1024) {
-            cudaError_t e = cudaFuncSetAttribute(encode_targets_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_small);
+            cudaError_t e = cudaFuncSetAttribute(encode_targets_kernel<TL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_small);
             if (e != cudaSuccess) return e;
         }
-        encode_targets_kernel<<<dim3(B, 1), 256, smem_small, st>>>(small);
+        encode_targets_kernel<TL><<<dim3(B, 1), 256, smem_small, st>>>(small);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
         // tiles of about 48 KB per tensor, whole rows
-        int rows_per_tile = (48 * 1024) / (HW * 4);
+        int rows_per_tile = (48 * 1024) / (HW * (int)sizeof(TL));
         if (rows_per_tile < 1) rows_per_tile = 1;
         if (rows_per_tile > S) rows_per_tile = S;
         const int chunks = (S + rows_per_tile - 1) / rows_per_tile;
         rows_per_tile = (S + chunks - 1) / chunks;
         const long long n_tiles = (long long)B * a.E * chunks;
         const int grid = (int)std::min<long long>(n_tiles, (long long)sms * a.sweep_ctas_per_sm);
-        encode_sweep_kernel<<<grid, 256, (size_t)2 * HW, st>>>(a, B, chunks, rows_per_tile);
+        encode_sweep_kernel<TL><<<grid, 256, (size_t)2 * HW, st>>>(a, B, chunks, rows_per_tile);
         return cudaGetLastError();
     }
     // enough CTAs to fill the machine a few times over; every CTA rebuilds the image's byte map (cheap)
@@ -261,11 +276,21 @@ cudaError_t launch_encode_targets(EncodeArgs a, int B, int sms, cudaStream_t st)
     Z = rows > 0 ? (rows + a.rows_per_cta - 1) / a.rows_per_cta : 1;
     const size_t smem = ((size_t)a.K * a.H * a.W + 15) & ~(size_t)15;
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(encode_targets_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(encode_targets_kernel<TL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    encode_targets_kernel<<<dim3(B, Z), 256, smem, st>>>(a);
+    encode_targets_kernel<TL><<<dim3(B, Z), 256, smem, st>>>(a);
     return cudaGetLastError();
+}
+
+cudaError_t launch_encode_targets(EncodeArgs a, int B, int sms, cudaStream_t st) {
+    if (B == 0) return cudaSuccess;
+    switch (a.limb_dtype) {
+        case HEAD_F32: return encode_as<float>(a, B, sms, st);
+        case HEAD_F16: return encode_as<__half>(a, B, sms, st);
+        case HEAD_BF16: return encode_as<__nv_bfloat16>(a, B, sms, st);
+        default: return cudaErrorInvalidValue;
+    }
 }
 
 }  // namespace ppn

@@ -718,13 +718,8 @@ head_gemm16_argmax_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid
 // ------------------------------ operand packing for the 16-bit path ------------------------------
 // feat [B][Cin][HW] fp32 (NCHW) -> xt [B * HW][Cin] T (round to nearest even), weight [C][Cin] fp32 -> wt [C][Cin] T.
 // Blocks [0, n_feat_blocks): one 64-channel x 32-cell tile each, transposed through shared memory (128-byte reads along
-// the cells, 128-byte writes along the channels); the blocks after them convert the weights.
-template <typename T> __device__ __forceinline__ T narrow(float v);
-template <> __device__ __forceinline__ __half narrow<__half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 narrow<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-__device__ __forceinline__ uint32_t bits16(__half v) { return __half_as_ushort(v); }
-__device__ __forceinline__ uint32_t bits16(__nv_bfloat16 v) { return __bfloat16_as_ushort(v); }
-
+// the cells, 128-byte writes along the channels); the blocks after them convert the weights.  (narrow / bits16:
+// ppn_device.cuh)
 template <typename T>
 __global__ void __launch_bounds__(256)
 head_pack_kernel(const float* __restrict__ feat, const float* __restrict__ weight, T* __restrict__ xt, T* __restrict__ wt,

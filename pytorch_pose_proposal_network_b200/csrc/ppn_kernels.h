@@ -161,7 +161,9 @@ struct EncodeArgs {
     const float* keypoints;         // [n, K - 1, 2]
     const uint8_t* visible;         // [n, K - 1]
     const double* size;             // [n]
-    float *delta, *weight, *weight_ij, *tx, *ty, *tx_half, *ty_half, *tw, *th, *te;
+    float *delta, *weight, *tx, *ty, *tx_half, *ty_half, *tw, *th;
+    void *weight_ij, *te;           // elements of limb_dtype
+    int32_t limb_dtype;             // HEAD_F32, HEAD_F16 or HEAD_BF16
     int32_t K, E, H, W, sH, sW, rows_per_cta;
     int32_t small_only, sweep, sweep_ctas_per_sm;   // launcher state / tuning (encode.sweep, encode.ctas_per_sm)
     uint32_t magic_sW;              // ceil(2^32 / sW) for exact x / sW, 0 <= x < 65536 (0 when sW == 1)
@@ -174,9 +176,11 @@ cudaError_t launch_encode_targets(EncodeArgs a, int B, int sms, cudaStream_t st)
 // ---- the training loss (ppn_loss.cu): forward sums and the head gradient of the reference's PPNLoss -------------
 constexpr int kLossMaxCtas = 2048;     // CTAs of the forward grid at most: the workspace holds one partial set each
 struct LossArgs {
-    const float* head;                  // [B, C, H, W]
-    float* grad;                        // [B, C, H, W] (backward)
-    const float *delta, *weight, *weight_ij, *tx, *ty, *tx_half, *ty_half, *tw, *th, *te;
+    const void* head;                   // [B, C, H, W] of head_dtype
+    void* grad;                         // [B, C, H, W] of head_dtype (backward)
+    const float *delta, *weight, *tx, *ty, *tx_half, *ty_half, *tw, *th;
+    const void *weight_ij, *te;         // [B, E, sH, sW, H, W] of limb_dtype
+    int32_t head_dtype, limb_dtype;     // HEAD_*: (F32, F32), (F16, F32 or F16), (BF16, F32 or BF16)
     const float* grad_loss;             // [5] device (backward)
     double* partial;                    // [grid][5] workspace (forward)
     int32_t B, K, W, HW, L;             // L = E * sH * sW * H * W limb elements per image

@@ -14,10 +14,18 @@
 //   small items   1024 cells of the [B, K, H, W] planes: a thread takes whole cells, because the IoU needs all four
 //                 box planes of a cell (6 head values and 8 targets in, 4 loss terms or 6 gradients out);
 //   limb items    8192 consecutive elements of one image's limb block, streamed with 128-bit loads (and, backward,
-//                 128-bit streaming stores) where the head, te, weight_ij (and grad) of that image sit at the same
-//                 phase within 16 bytes, element by element where they do not (only grids with an odd H*W or odd K
-//                 produce such images, or tensors whose storage starts mid-vector).
+//                 128-bit streaming stores) from the first element at which the head, te, weight_ij (and grad) of
+//                 that image all sit on a 16-byte boundary, element by element where no such element exists (only
+//                 grids with an odd H*W or odd K produce such images, or tensors whose storage starts mid-vector).
 // The limb block is 98.6 % of the bytes at the native shape: the kernels are HBM streams with a little arithmetic.
+//
+// Element types (the AMP setup of the reference, main.py:282-289): the head, and with it the gradient, may be fp16 or
+// bf16; te and weight_ij then may be fp32 or the head's type; the eight small targets are always fp32.  A 16-bit
+// element is widened to fp32 exactly when it is loaded, everything below is the fp32 arithmetic as written, and a
+// gradient element is rounded once, to nearest even, to the head's type when it is stored (overflow gives +-inf, as
+// torch's .to() does; a GradScaler looks for it).  So a 16-bit run equals the fp32 run on the widened inputs followed
+// by .to(head.dtype).  With a 16-bit stream a vector step covers 8 elements: one 16-byte access per 16-bit stream,
+// two per fp32 stream.
 //
 // Forward: every thread accumulates its terms in fp64 (each fp32 term converted exactly); a CTA reduces its threads
 // in a fixed butterfly order and stores 5 doubles into the caller's workspace; a one-CTA kernel sums the CTA
@@ -58,31 +66,85 @@ namespace {
 
 constexpr int kLossThreads = 256;
 constexpr int kSmallCells = 1024;      // cells of the [B, K, H, W] planes per small item
-constexpr int kLimbChunk = 8192;       // limb elements per limb item: 32 KB of each stream
-constexpr int kLimbUnroll = 4;         // float4 iterations whose loads a thread issues before it computes
+constexpr int kLimbChunk = 8192;       // limb elements per limb item: 32 KB of each fp32 stream
+constexpr int kLimbUnroll = 4;         // vector steps whose loads a thread issues before it computes
 constexpr float kEps = 1e-6f;          // config.EPSILON
 
-__device__ __forceinline__ float lds(const float* p) {     // streaming scalar load, no L1 allocation
+// ---- streaming element access (no L1 allocation), widened to / narrowed from fp32 ------------------------------
+__device__ __forceinline__ float lds(const float* p) {
     float v;
     asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
     return v;
 }
+__device__ __forceinline__ unsigned short lds16(const void* p) {
+    unsigned short v;
+    asm volatile("ld.global.nc.L1::no_allocate.b16 %0, [%1];" : "=h"(v) : "l"(p));
+    return v;
+}
+__device__ __forceinline__ float ldw(const float* p) { return lds(p); }
+__device__ __forceinline__ float ldw(const __half* p) { return widen(__ushort_as_half(lds16(p))); }
+__device__ __forceinline__ float ldw(const __nv_bfloat16* p) { return widen(__ushort_as_bfloat16(lds16(p))); }
 
-__device__ __forceinline__ unsigned phase_of(const float* p) { return (unsigned)(reinterpret_cast<uintptr_t>(p) >> 2) & 3u; }
+__device__ __forceinline__ void st16(void* p, unsigned short v) { asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"(v) : "memory"); }
+__device__ __forceinline__ void stw(float* p, float v) { __stcs(p, v); }
+__device__ __forceinline__ void stw(__half* p, float v) { st16(p, __half_as_ushort(narrow<__half>(v))); }
+__device__ __forceinline__ void stw(__nv_bfloat16* p, float v) { st16(p, __bfloat16_as_ushort(narrow<__nv_bfloat16>(v))); }
+
+// ---- 16-byte vectors: VE consecutive elements of one stream kept as raw words, widened when used -----------------
+__device__ __forceinline__ uint4 ldg_stream_u4(const void* p) {
+    uint4 v;
+    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];"
+                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
+    return v;
+}
+__device__ __forceinline__ uint32_t word(const uint4& q, int k) { return k == 0 ? q.x : k == 1 ? q.y : k == 2 ? q.z : q.w; }
+__device__ __forceinline__ unsigned short half_word(const uint4* q, int i) {
+    const uint32_t w = word(q[i >> 3], (i >> 1) & 3);
+    return (unsigned short)((i & 1) ? (w >> 16) : (w & 0xffffu));
+}
+
+template <typename T, int VE> struct Vec {
+    uint4 q[VE * (int)sizeof(T) / 16];
+    __device__ __forceinline__ void load(const T* p) {                // p: 16-byte aligned
+#pragma unroll
+        for (int i = 0; i < VE * (int)sizeof(T) / 16; ++i) q[i] = ldg_stream_u4(reinterpret_cast<const uint4*>(p) + i);
+    }
+};
+template <int VE> __device__ __forceinline__ float at(const Vec<float, VE>& v, int i) { return __uint_as_float(word(v.q[i >> 2], i & 3)); }
+template <int VE> __device__ __forceinline__ float at(const Vec<__half, VE>& v, int i) { return widen(__ushort_as_half(half_word(v.q, i))); }
+template <int VE> __device__ __forceinline__ float at(const Vec<__nv_bfloat16, VE>& v, int i) {
+    return widen(__ushort_as_bfloat16(half_word(v.q, i)));
+}
+
+// VE gradients (p: 16-byte aligned) with 128-bit streaming stores
+template <int VE> __device__ __forceinline__ void st_vec(float* p, const float (&g)[VE]) {
+#pragma unroll
+    for (int j = 0; j < VE / 4; ++j) __stcs(reinterpret_cast<float4*>(p) + j, make_float4(g[4 * j], g[4 * j + 1], g[4 * j + 2], g[4 * j + 3]));
+}
+template <typename T, int VE> __device__ __forceinline__ void st_vec(T* p, const float (&g)[VE]) {    // 16-bit types
+#pragma unroll
+    for (int j = 0; j < VE / 8; ++j)
+        __stcs(reinterpret_cast<uint4*>(p) + j, make_uint4(pack2<T>(g[8 * j], g[8 * j + 1]), pack2<T>(g[8 * j + 2], g[8 * j + 3]),
+                                                           pack2<T>(g[8 * j + 4], g[8 * j + 5]), pack2<T>(g[8 * j + 6], g[8 * j + 7])));
+}
+
+// elements of a vector step: 4 when every stream is fp32, else 8
+template <typename TH, typename TL> __host__ __device__ constexpr int vec_elems() { return sizeof(TH) == 4 && sizeof(TL) == 4 ? 4 : 8; }
 
 struct Cell {
     float resp, conf, x, y, w, h;                           // head
     float delta, weight, txh, tyh, tx, ty, tw, th;          // targets
 };
 
+template <typename TH>
 __device__ __forceinline__ Cell load_cell(const LossArgs& a, long long i) {
     const long long KHW = (long long)a.K * a.HW;
     const long long b = i / KHW, r = i - b * KHW;
-    const float* img = a.head + (size_t)b * a.img_stride + (size_t)r;
+    const TH* img = static_cast<const TH*>(a.head) + (size_t)b * a.img_stride + (size_t)r;
     const size_t KH = (size_t)KHW;
     Cell c;
-    c.resp = lds(img);          c.conf = lds(img + KH);     c.x = lds(img + 2 * KH);
-    c.y = lds(img + 3 * KH);    c.w = lds(img + 4 * KH);    c.h = lds(img + 5 * KH);
+    c.resp = ldw(img);          c.conf = ldw(img + KH);     c.x = ldw(img + 2 * KH);
+    c.y = ldw(img + 3 * KH);    c.w = ldw(img + 4 * KH);    c.h = ldw(img + 5 * KH);
     c.delta = lds(a.delta + i); c.weight = lds(a.weight + i);
     c.txh = lds(a.tx_half + i); c.tyh = lds(a.ty_half + i);
     c.tx = lds(a.tx + i);       c.ty = lds(a.ty + i);       c.tw = lds(a.tw + i);       c.th = lds(a.th + i);
@@ -135,19 +197,24 @@ __device__ __forceinline__ void axis_grad(const Box& b, float gi, float* d_pos, 
 __device__ __forceinline__ float sq(float v) { return __fmul_rn(v, v); }
 
 // ---- the limb block of one item ---------------------------------------------------------------------------------
-struct LimbItem { const float *hp, *tp, *wp; float* gp; int start, end, pro; bool vec; };
+template <typename TH, typename TL> struct LimbItem { const TH* hp; const TL *tp, *wp; TH* gp; int start, end, pro; bool vec; };
 
-__device__ __forceinline__ LimbItem limb_item(const LossArgs& a, long long j, bool backward) {
+__device__ __forceinline__ bool on_16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+template <typename TH, typename TL>
+__device__ __forceinline__ LimbItem<TH, TL> limb_item(const LossArgs& a, long long j, bool backward) {
     const long long b = j / a.limb_chunks;
     const int q = (int)(j - b * a.limb_chunks);
-    LimbItem it;
-    it.hp = a.head + (size_t)b * a.img_stride + a.limb_off;
-    it.tp = a.te + (size_t)b * a.L;
-    it.wp = a.weight_ij + (size_t)b * a.L;
-    it.gp = backward ? a.grad + (size_t)b * a.img_stride + a.limb_off : nullptr;
-    const unsigned ph = phase_of(it.hp);
-    it.vec = phase_of(it.tp) == ph && phase_of(it.wp) == ph && (!backward || phase_of(it.gp) == ph);
-    const int a0 = it.vec ? min(a.L, (int)((4u - ph) & 3u)) : 0;       // elements before the first aligned vector
+    LimbItem<TH, TL> it;
+    it.hp = static_cast<const TH*>(a.head) + (size_t)b * a.img_stride + a.limb_off;
+    it.tp = static_cast<const TL*>(a.te) + (size_t)b * a.L;
+    it.wp = static_cast<const TL*>(a.weight_ij) + (size_t)b * a.L;
+    it.gp = backward ? static_cast<TH*>(a.grad) + (size_t)b * a.img_stride + a.limb_off : nullptr;
+    // The head has the most elements per 16 bytes of any stream (8 if 16-bit, else 4 like all the others), so the
+    // first element at which every stream is 16-byte aligned, if there is one, is the head's first aligned element.
+    const int h0 = (int)(((16u - (reinterpret_cast<uintptr_t>(it.hp) & 15u)) & 15u) / sizeof(TH));
+    it.vec = on_16(it.tp + h0) && on_16(it.wp + h0) && (!backward || on_16(it.gp + h0));
+    const int a0 = it.vec ? min(a.L, h0) : 0;                           // elements before the first aligned vector
     it.pro = q == 0 ? a0 : 0;                                            // chunk 0 also takes those
     it.start = min(a.L, a0 + q * kLimbChunk);
     it.end = min(a.L, it.start + kLimbChunk);
@@ -178,8 +245,10 @@ __device__ __forceinline__ void cta_store(double acc[5], double* out) {
     }
 }
 
+template <typename TH, typename TL>
 __global__ void __launch_bounds__(kLossThreads)
 loss_forward_kernel(LossArgs a) {
+    constexpr int VE = vec_elems<TH, TL>();
     double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
     const int tid = threadIdx.x;
     const long long n_cells = (long long)a.B * a.K * a.HW;
@@ -187,7 +256,7 @@ loss_forward_kernel(LossArgs a) {
         if (j < a.small_items) {
             const long long c1 = min(n_cells, (j + 1) * kSmallCells);
             for (long long i = j * kSmallCells + tid; i < c1; i += kLossThreads) {
-                const Cell c = load_cell(a, i);
+                const Cell c = load_cell<TH>(a, i);
                 const Iou u = iou_of(a, c, i);
                 acc[0] += (double)sq(__fsub_rn(c.resp, c.delta));
                 acc[1] += (double)__fmul_rn(c.delta, sq(__fsub_rn(c.conf, u.iou)));
@@ -198,35 +267,31 @@ loss_forward_kernel(LossArgs a) {
             }
             continue;
         }
-        const LimbItem it = limb_item(a, j - a.small_items, false);
-        if (tid < it.pro) acc[4] += (double)limb_term(lds(it.hp + tid), lds(it.tp + tid), lds(it.wp + tid));
+        const LimbItem<TH, TL> it = limb_item<TH, TL>(a, j - a.small_items, false);
+        if (tid < it.pro) acc[4] += (double)limb_term(ldw(it.hp + tid), ldw(it.tp + tid), ldw(it.wp + tid));
         int s0 = it.start;
         if (it.vec) {
-            const int nv = (it.end - it.start) >> 2;
-            const float4* h4 = reinterpret_cast<const float4*>(it.hp + it.start);
-            const float4* t4 = reinterpret_cast<const float4*>(it.tp + it.start);
-            const float4* w4 = reinterpret_cast<const float4*>(it.wp + it.start);
+            const int nv = (it.end - it.start) / VE;
             for (int v0 = tid; v0 < nv; v0 += kLimbUnroll * kLossThreads) {
-                float4 hv[kLimbUnroll], tv[kLimbUnroll], wv[kLimbUnroll];
+                Vec<TH, VE> hv[kLimbUnroll];
+                Vec<TL, VE> tv[kLimbUnroll], wv[kLimbUnroll];
 #pragma unroll
                 for (int u = 0; u < kLimbUnroll; ++u) {
-                    const int v = v0 + u * kLossThreads;
-                    if (v < nv) { hv[u] = ldg_stream(h4 + v); tv[u] = ldg_stream(t4 + v); wv[u] = ldg_stream(w4 + v); }
+                    const size_t e = (size_t)it.start + (size_t)(v0 + u * kLossThreads) * VE;
+                    if (v0 + u * kLossThreads < nv) { hv[u].load(it.hp + e); tv[u].load(it.tp + e); wv[u].load(it.wp + e); }
                 }
 #pragma unroll
                 for (int u = 0; u < kLimbUnroll; ++u) {
                     if (v0 + u * kLossThreads < nv) {
-                        acc[4] += (double)limb_term(hv[u].x, tv[u].x, wv[u].x);
-                        acc[4] += (double)limb_term(hv[u].y, tv[u].y, wv[u].y);
-                        acc[4] += (double)limb_term(hv[u].z, tv[u].z, wv[u].z);
-                        acc[4] += (double)limb_term(hv[u].w, tv[u].w, wv[u].w);
+#pragma unroll
+                        for (int k = 0; k < VE; ++k) acc[4] += (double)limb_term(at(hv[u], k), at(tv[u], k), at(wv[u], k));
                     }
                 }
             }
-            s0 = it.start + 4 * nv;
+            s0 = it.start + VE * nv;
         }
         for (int e = s0 + tid; e < it.end; e += kLossThreads)             // vector tail, or the whole unaligned item
-            acc[4] += (double)limb_term(lds(it.hp + e), lds(it.tp + e), lds(it.wp + e));
+            acc[4] += (double)limb_term(ldw(it.hp + e), ldw(it.tp + e), ldw(it.wp + e));
     }
     cta_store(acc, a.partial);
 }
@@ -243,8 +308,10 @@ loss_finalize_kernel(const double* __restrict__ partial, int n, int B, float* __
     if (lane == 0) loss[t] = (float)(v / (double)B);
 }
 
+template <typename TH, typename TL>
 __global__ void __launch_bounds__(kLossThreads)
 loss_backward_kernel(LossArgs a) {
+    constexpr int VE = vec_elems<TH, TL>();
     const float Bf = (float)a.B;
     const float cr = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[0]), Bf);
     const float ci = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[1]), Bf);
@@ -258,7 +325,7 @@ loss_backward_kernel(LossArgs a) {
         if (j < a.small_items) {
             const long long c1 = min(n_cells, (j + 1) * kSmallCells);
             for (long long i = j * kSmallCells + tid; i < c1; i += kLossThreads) {
-                const Cell c = load_cell(a, i);
+                const Cell c = load_cell<TH>(a, i);
                 const Iou u = iou_of(a, c, i);
                 const float g_resp = __fmul_rn(cr, __fsub_rn(c.resp, c.delta));
                 const float g_conf = __fmul_rn(ci, __fmul_rn(c.delta, __fsub_rn(c.conf, u.iou)));
@@ -280,41 +347,40 @@ loss_backward_kernel(LossArgs a) {
                 const float g_w = __fadd_rn(__fmul_rn(cs, __fmul_rn(c.weight, __fdiv_rn(__fsub_rn(sw, st), sw))), __fmul_rn(dpw, a.inW));
                 const float g_h = __fadd_rn(__fmul_rn(cs, __fmul_rn(c.weight, __fdiv_rn(__fsub_rn(sh, sth), sh))), __fmul_rn(dph, a.inH));
                 const long long b = i / KHW, rr = i - b * KHW;
-                float* gimg = a.grad + (size_t)b * a.img_stride + (size_t)rr;
+                TH* gimg = static_cast<TH*>(a.grad) + (size_t)b * a.img_stride + (size_t)rr;
                 const size_t KH = (size_t)KHW;
-                __stcs(gimg, g_resp);          __stcs(gimg + KH, g_conf);     __stcs(gimg + 2 * KH, g_x);
-                __stcs(gimg + 3 * KH, g_y);    __stcs(gimg + 4 * KH, g_w);    __stcs(gimg + 5 * KH, g_h);
+                stw(gimg, g_resp);          stw(gimg + KH, g_conf);     stw(gimg + 2 * KH, g_x);
+                stw(gimg + 3 * KH, g_y);    stw(gimg + 4 * KH, g_w);    stw(gimg + 5 * KH, g_h);
             }
             continue;
         }
-        const LimbItem it = limb_item(a, j - a.small_items, true);
-        if (tid < it.pro) __stcs(it.gp + tid, limb_grad(cl, lds(it.hp + tid), lds(it.tp + tid), lds(it.wp + tid)));
+        const LimbItem<TH, TL> it = limb_item<TH, TL>(a, j - a.small_items, true);
+        if (tid < it.pro) stw(it.gp + tid, limb_grad(cl, ldw(it.hp + tid), ldw(it.tp + tid), ldw(it.wp + tid)));
         int s0 = it.start;
         if (it.vec) {
-            const int nv = (it.end - it.start) >> 2;
-            const float4* h4 = reinterpret_cast<const float4*>(it.hp + it.start);
-            const float4* t4 = reinterpret_cast<const float4*>(it.tp + it.start);
-            const float4* w4 = reinterpret_cast<const float4*>(it.wp + it.start);
-            float4* g4 = reinterpret_cast<float4*>(it.gp + it.start);
+            const int nv = (it.end - it.start) / VE;
             for (int v0 = tid; v0 < nv; v0 += kLimbUnroll * kLossThreads) {
-                float4 hv[kLimbUnroll], tv[kLimbUnroll], wv[kLimbUnroll];
+                Vec<TH, VE> hv[kLimbUnroll];
+                Vec<TL, VE> tv[kLimbUnroll], wv[kLimbUnroll];
 #pragma unroll
                 for (int u = 0; u < kLimbUnroll; ++u) {
-                    const int v = v0 + u * kLossThreads;
-                    if (v < nv) { hv[u] = ldg_stream(h4 + v); tv[u] = ldg_stream(t4 + v); wv[u] = ldg_stream(w4 + v); }
+                    const size_t e = (size_t)it.start + (size_t)(v0 + u * kLossThreads) * VE;
+                    if (v0 + u * kLossThreads < nv) { hv[u].load(it.hp + e); tv[u].load(it.tp + e); wv[u].load(it.wp + e); }
                 }
 #pragma unroll
                 for (int u = 0; u < kLimbUnroll; ++u) {
-                    const int v = v0 + u * kLossThreads;
-                    if (v < nv)
-                        __stcs(g4 + v, make_float4(limb_grad(cl, hv[u].x, tv[u].x, wv[u].x), limb_grad(cl, hv[u].y, tv[u].y, wv[u].y),
-                                                   limb_grad(cl, hv[u].z, tv[u].z, wv[u].z), limb_grad(cl, hv[u].w, tv[u].w, wv[u].w)));
+                    if (v0 + u * kLossThreads < nv) {
+                        float g[VE];
+#pragma unroll
+                        for (int k = 0; k < VE; ++k) g[k] = limb_grad(cl, at(hv[u], k), at(tv[u], k), at(wv[u], k));
+                        st_vec(it.gp + (size_t)it.start + (size_t)(v0 + u * kLossThreads) * VE, g);
+                    }
                 }
             }
-            s0 = it.start + 4 * nv;
+            s0 = it.start + VE * nv;
         }
         for (int e = s0 + tid; e < it.end; e += kLossThreads)
-            __stcs(it.gp + e, limb_grad(cl, lds(it.hp + e), lds(it.tp + e), lds(it.wp + e)));
+            stw(it.gp + e, limb_grad(cl, ldw(it.hp + e), ldw(it.tp + e), ldw(it.wp + e)));
     }
 }
 
@@ -327,7 +393,25 @@ int grid_for(const void* kernel, std::atomic<int>* per_sm_cache, long long n_ite
     }
     return (int)std::min<long long>(n_items, std::min<long long>((long long)sms * per_sm, kLossMaxCtas));
 }
-std::atomic<int> g_forward_per_sm{0}, g_backward_per_sm{0};
+
+template <typename TH, typename TL>
+cudaError_t forward_as(const LossArgs& a, float* loss, int sms, cudaStream_t st) {
+    static std::atomic<int> per_sm{0};
+    const int grid = grid_for((const void*)loss_forward_kernel<TH, TL>, &per_sm, a.n_items, sms);
+    loss_forward_kernel<TH, TL><<<grid, kLossThreads, 0, st>>>(a);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    loss_finalize_kernel<<<1, 160, 0, st>>>(a.partial, grid, a.B, loss);
+    return cudaGetLastError();
+}
+
+template <typename TH, typename TL>
+cudaError_t backward_as(const LossArgs& a, int sms, cudaStream_t st) {
+    static std::atomic<int> per_sm{0};
+    const int grid = grid_for((const void*)loss_backward_kernel<TH, TL>, &per_sm, a.n_items, sms);
+    loss_backward_kernel<TH, TL><<<grid, kLossThreads, 0, st>>>(a);
+    return cudaGetLastError();
+}
 
 }  // namespace
 
@@ -343,19 +427,27 @@ size_t loss_workspace_bytes(const LossArgs& a) {
     return (size_t)ctas * 5 * sizeof(double);
 }
 
+// the five (head, limb target) type pairs of LossArgs; the C ABI rejects every other pair before launching
 cudaError_t launch_loss_forward(LossArgs a, float* loss, int sms, cudaStream_t st) {
-    const int grid = grid_for((const void*)loss_forward_kernel, &g_forward_per_sm, a.n_items, sms);
-    loss_forward_kernel<<<grid, kLossThreads, 0, st>>>(a);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-    loss_finalize_kernel<<<1, 160, 0, st>>>(a.partial, grid, a.B, loss);
-    return cudaGetLastError();
+    switch (a.head_dtype * 3 + a.limb_dtype) {
+        case HEAD_F32 * 3 + HEAD_F32: return forward_as<float, float>(a, loss, sms, st);
+        case HEAD_F16 * 3 + HEAD_F32: return forward_as<__half, float>(a, loss, sms, st);
+        case HEAD_F16 * 3 + HEAD_F16: return forward_as<__half, __half>(a, loss, sms, st);
+        case HEAD_BF16 * 3 + HEAD_F32: return forward_as<__nv_bfloat16, float>(a, loss, sms, st);
+        case HEAD_BF16 * 3 + HEAD_BF16: return forward_as<__nv_bfloat16, __nv_bfloat16>(a, loss, sms, st);
+        default: return cudaErrorInvalidValue;
+    }
 }
 
 cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st) {
-    const int grid = grid_for((const void*)loss_backward_kernel, &g_backward_per_sm, a.n_items, sms);
-    loss_backward_kernel<<<grid, kLossThreads, 0, st>>>(a);
-    return cudaGetLastError();
+    switch (a.head_dtype * 3 + a.limb_dtype) {
+        case HEAD_F32 * 3 + HEAD_F32: return backward_as<float, float>(a, sms, st);
+        case HEAD_F16 * 3 + HEAD_F32: return backward_as<__half, float>(a, sms, st);
+        case HEAD_F16 * 3 + HEAD_F16: return backward_as<__half, __half>(a, sms, st);
+        case HEAD_BF16 * 3 + HEAD_F32: return backward_as<__nv_bfloat16, float>(a, sms, st);
+        case HEAD_BF16 * 3 + HEAD_BF16: return backward_as<__nv_bfloat16, __nv_bfloat16>(a, sms, st);
+        default: return cudaErrorInvalidValue;
+    }
 }
 
 }  // namespace ppn

@@ -13,6 +13,10 @@ tensors; checked bit for bit against outputs of the reference's own ``__getitem_
     batch = enc.encode(samples)                    # samples: what the reference's transforms return
     batch.delta, batch.weight, batch.weight_ij, batch.tx, ... batch.te      # like CustomBatch, on the GPU
 
+For mixed-precision training, ``TargetEncoder(cfg, limb_dtype=torch.float16)`` (or bfloat16) writes the two limb
+tensors — most of the bytes — in 16 bits: te in {0, 1} is exact, weight_ij stores 0.0005 rounded to the type
+(fp16 0.000500202..., bf16 0.000499725...).  The eight [B, K, H, W] grids stay fp32.
+
 Image loading and augmentation (aug.py) stay where they are: they are not on this path.
 """
 from __future__ import annotations
@@ -62,13 +66,20 @@ def flatten_samples(samples: Sequence[dict], K: int):
             cat(vis, (0, K - 1), np.uint8), cat(sizes, (0,), np.float64))
 
 
-class TargetEncoder:
-    """Batched GPU replacement of the encode half of ``KeypointsDataset.__getitem__``."""
+LIMB_DTYPES = {torch.float32: _lib.HEAD_F32, torch.float16: _lib.HEAD_F16, torch.bfloat16: _lib.HEAD_BF16}
 
-    def __init__(self, cfg: PPNConfig, edges=None, device=None):
+
+class TargetEncoder:
+    """Batched GPU replacement of the encode half of ``KeypointsDataset.__getitem__``.  ``limb_dtype``: the
+    element type of te and weight_ij (float32, float16 or bfloat16)."""
+
+    def __init__(self, cfg: PPNConfig, edges=None, device=None, limb_dtype=torch.float32):
         if not torch.cuda.is_available():
             raise RuntimeError("TargetEncoder needs a CUDA device: there is no CPU path")
+        if limb_dtype not in LIMB_DTYPES:
+            raise ValueError(f"limb_dtype must be torch.float32, float16 or bfloat16, got {limb_dtype}")
         self.cfg = cfg
+        self.limb_dtype = limb_dtype
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.lib = _lib.lib()
         self.c = _CConfig(cfg)
@@ -85,7 +96,7 @@ class TargetEncoder:
     def alloc(self, B: int) -> TargetBatch:
         cfg = self.cfg
         small = lambda: torch.empty(B, cfg.K, cfg.H, cfg.W, dtype=torch.float32, device=self.device)
-        big = lambda: torch.empty(B, cfg.E, cfg.sH, cfg.sW, cfg.H, cfg.W, dtype=torch.float32, device=self.device)
+        big = lambda: torch.empty(B, cfg.E, cfg.sH, cfg.sW, cfg.H, cfg.W, dtype=self.limb_dtype, device=self.device)
         return TargetBatch(**{n: (big() if n in ("weight_ij", "te") else small()) for n in _lib.TARGET_NAMES})
 
     @staticmethod
@@ -112,13 +123,21 @@ class TargetEncoder:
                 raise ValueError(f"expected a contiguous {dt} tensor of shape {shp} on {self.device}, got {t.dtype} {tuple(t.shape)} on {t.device}")
         if out is None:
             out = self.alloc(B)
+        elif out.te.dtype != self.limb_dtype or out.weight_ij.dtype != self.limb_dtype:
+            raise ValueError(f"out.te and out.weight_ij must be {self.limb_dtype}, got {out.te.dtype} and {out.weight_ij.dtype}")
         people = _lib.PPNPeople(person_off.data_ptr(), bbox.data_ptr(), keypoints.data_ptr(), visible.data_ptr(), size.data_ptr())
         targets = _lib.PPNTargets(*[getattr(out, nme).data_ptr() for nme in _lib.TARGET_NAMES])
         shape = self.c.shape(B)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        edges = self.edges.ctypes.data_as(_lib.i32p)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.ppn_encode_targets(C.byref(people), C.byref(shape), self.edges.ctypes.data_as(_lib.i32p),
-                                                   C.byref(targets), C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)),
-                       "ppn_encode_targets")
+            if self.limb_dtype == torch.float32:
+                _lib.check(self.lib.ppn_encode_targets(C.byref(people), C.byref(shape), edges, C.byref(targets), stream),
+                           "ppn_encode_targets")
+            else:
+                _lib.check(self.lib.ppn_encode_targets_opt(C.byref(people), C.byref(shape), edges, C.byref(targets),
+                                                           LIMB_DTYPES[self.limb_dtype], stream),
+                           "ppn_encode_targets_opt")
         return out
 
     def encode(self, samples: Sequence[dict], out: Optional[TargetBatch] = None) -> TargetBatch:

@@ -13,6 +13,10 @@ Nothing head-sized is kept between the two: the autograd graph holds references 
     loss = sum(l * t for l, t in zip(lambdas, terms))                    # the reference weights by GradNorm
     loss.backward()
 
+Under mixed precision (the reference trains under apex AMP, main.py:282-289) the head may be fp16 or bf16, and te /
+weight_ij may be stored in the head's type (``TargetEncoder(cfg, limb_dtype=...)``): the loss is the fp32 loss on
+the exactly widened inputs and the gradient comes back in the head's type, rounded once — no fp32 copy of the head.
+
 The reference's training loop is not part of this project: the loss is specified by the float64 restatement
 described in DESIGN.md §11 (IoU differentiable in x, y, w, h; eps = 1e-6 in the IoU denominator; L_resp
 unweighted), not by bit parity with main.py.
@@ -31,6 +35,7 @@ from .parser import _CConfig
 # __getitem__ (tx, ty, tx_half, ty_half)
 ARG_ORDER = ("delta", "weight", "weight_ij", "tx_half", "ty_half", "tx", "ty", "tw", "th", "te")
 TERMS = ("loss_resp", "loss_iou", "loss_coor", "loss_size", "loss_limb")
+HEAD_DTYPES = {torch.float32: _lib.HEAD_F32, torch.float16: _lib.HEAD_F16, torch.bfloat16: _lib.HEAD_BF16}
 
 
 class _PPNLossFunction(torch.autograd.Function):
@@ -60,9 +65,11 @@ class PPNLoss(torch.nn.Module):
     the order of :meth:`dataset.TargetBatch.as_list` (``tx, ty, tx_half, ty_half``, as ``__getitem__`` returns
     them): pass the targets by name, as in the module docstring, or through :meth:`from_batch`.
 
-    feature_map: fp32 [B, 6K + E*sH*sW, H, W], contiguous, on a CUDA device — the sigmoid output the reference's
-    model returns; the eight small targets [B, K, H, W], weight_ij and te [B, E, sH, sW, H, W], all fp32,
-    contiguous, on the same device.  Anything else raises ValueError.  The gradient flows into ``feature_map``
+    feature_map: [B, 6K + E*sH*sW, H, W] fp32, fp16 or bf16, contiguous, on a CUDA device — the sigmoid output the
+    reference's model returns; the eight small targets [B, K, H, W] fp32; weight_ij and te [B, E, sH, sW, H, W],
+    both fp32 or both in the dtype of a 16-bit feature_map; all contiguous, on the same device.  Anything else
+    raises ValueError.  A 16-bit feature_map gets its gradient in its own dtype: the fp32 gradient of the widened
+    inputs, rounded once to nearest even (overflow to +-inf, which a GradScaler detects).  The gradient flows into ``feature_map``
     only.  Terms that do not reach the final loss get no upstream gradient and are skipped in the backward; the
     upstream gradients never travel to the host.
     """
@@ -79,7 +86,7 @@ class PPNLoss(torch.nn.Module):
         self.device = torch.device("cuda", torch.cuda.current_device() if dev.index is None else dev.index)
         self.lib = _lib.lib()
         self.c = _CConfig(cfg)
-        self._shapes = {}
+        self._shapes = {}             # (B, head dtype code) -> PPNShape
         self._ws = None
         self._ws_need = {}            # B -> workspace bytes (ppn_loss_workspace_bytes is pure arithmetic)
 
@@ -90,10 +97,10 @@ class PPNLoss(torch.nn.Module):
     def _stream(self) -> C.c_void_p:
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
-    def _shape(self, B: int) -> _lib.PPNShape:
-        s = self._shapes.get(B)
+    def _shape(self, B: int, head_dtype: int = _lib.HEAD_F32) -> _lib.PPNShape:
+        s = self._shapes.get((B, head_dtype))
         if s is None:
-            s = self._shapes[B] = self.c.shape(B)
+            s = self._shapes[(B, head_dtype)] = self.c.shape(B, head_dtype)
         return s
 
     def _workspace(self, B: int) -> torch.Tensor:
@@ -112,6 +119,7 @@ class PPNLoss(torch.nn.Module):
         return _lib.PPNTargets(*[by_name[n].data_ptr() for n in _lib.TARGET_NAMES])
 
     def _check(self, feature_map, targets) -> int:
+        """Raises ValueError unless the call is one the kernels take; returns B."""
         cfg = self.cfg
         if len(targets) != len(ARG_ORDER):
             raise ValueError(f"expected the {len(ARG_ORDER)} targets {ARG_ORDER}, got {len(targets)}")
@@ -124,11 +132,20 @@ class PPNLoss(torch.nn.Module):
             raise ValueError("the batch mean needs at least one image")
         small = (B, cfg.K, cfg.H, cfg.W)
         big = (B, cfg.E, cfg.sH, cfg.sW, cfg.H, cfg.W)
+        if feature_map.dtype not in HEAD_DTYPES:
+            raise ValueError(f"feature_map must be float32, float16 or bfloat16, got {feature_map.dtype}")
+        limb = dict(zip(ARG_ORDER, targets))["te"]
+        limb_dtype = limb.dtype if isinstance(limb, torch.Tensor) else None
+        limb_ok = (torch.float32, feature_map.dtype)          # the limb targets: fp32 or the head's 16-bit type
         for name, t in (("feature_map", feature_map),) + tuple(zip(ARG_ORDER, targets)):
             want = big if name in ("weight_ij", "te") else (feature_map.shape if name == "feature_map" else small)
             if not isinstance(t, torch.Tensor):
                 raise ValueError(f"{name} must be a tensor, got {type(t)}")
-            if t.dtype != torch.float32:
+            if name in ("weight_ij", "te"):
+                if t.dtype not in limb_ok or t.dtype != limb_dtype:
+                    raise ValueError(f"weight_ij and te must both be float32 or both {feature_map.dtype}, got {t.dtype} "
+                                     f"(te {limb_dtype})")
+            elif name != "feature_map" and t.dtype != torch.float32:
                 raise ValueError(f"{name} must be float32, got {t.dtype}")
             if tuple(t.shape) != tuple(want):
                 raise ValueError(f"{name} must have shape {tuple(want)}, got {tuple(t.shape)}")
@@ -157,31 +174,54 @@ class PPNLoss(torch.nn.Module):
 
     def backward_raw(self, feature_map, *targets, grad_loss: torch.Tensor, out=None) -> torch.Tensor:
         """The backward export without autograd: sum_t grad_loss[t] * dL_t/d(feature_map), grad_loss fp32 [5] on
-        the device; written into `out` (like feature_map) when given."""
+        the device; written into `out` (like feature_map, in its dtype) when given."""
         self._check(feature_map, targets)
         if grad_loss.dtype != torch.float32 or tuple(grad_loss.shape) != (5,) or grad_loss.device != self.device:
             raise ValueError("grad_loss must be a float32 [5] tensor on the loss's device")
         if out is None:
             out = torch.empty_like(feature_map)
-        elif out.dtype != torch.float32 or out.shape != feature_map.shape or out.device != self.device or \
+        elif out.dtype != feature_map.dtype or out.shape != feature_map.shape or out.device != self.device or \
                 not out.is_contiguous():
-            raise ValueError("out must be a contiguous float32 tensor like feature_map")
+            raise ValueError(f"out must be a contiguous {feature_map.dtype} tensor like feature_map")
         return self._launch_backward(feature_map, targets, grad_loss.contiguous(), out)
+
+    @staticmethod
+    def _options(feature_map, targets):
+        """None for an fp32 head (the fp32 exports), else the (shape dtype code, PPNLossOptions) of the _opt exports."""
+        if feature_map.dtype == torch.float32:
+            return None
+        te = targets[ARG_ORDER.index("te")]
+        return HEAD_DTYPES[feature_map.dtype], _lib.PPNLossOptions(HEAD_DTYPES[te.dtype])
 
     def _launch_forward(self, feature_map, targets, loss):
         B = feature_map.shape[0]
-        ws = self._workspace(B)
+        ws = self._workspace(B)                 # the same for every dtype (ppn_loss_workspace_bytes_opt)
         tg = self._targets_struct(targets)
+        opt = self._options(feature_map, targets)
         with self._guard():
-            _lib.check(self.lib.ppn_loss_forward(feature_map.data_ptr(), C.byref(self._shape(B)), C.byref(tg),
-                                                 loss.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()),
-                       "ppn_loss_forward")
+            if opt is None:
+                _lib.check(self.lib.ppn_loss_forward(feature_map.data_ptr(), C.byref(self._shape(B)), C.byref(tg),
+                                                     loss.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()),
+                           "ppn_loss_forward")
+            else:
+                _lib.check(self.lib.ppn_loss_forward_opt(feature_map.data_ptr(), C.byref(self._shape(B, opt[0])), C.byref(tg),
+                                                         C.byref(opt[1]), loss.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                         self._stream()),
+                           "ppn_loss_forward_opt")
         return loss
 
     def _launch_backward(self, feature_map, targets, grad_loss, grad_head):
+        B = feature_map.shape[0]
         tg = self._targets_struct(targets)
+        opt = self._options(feature_map, targets)
         with self._guard():
-            _lib.check(self.lib.ppn_loss_backward(feature_map.data_ptr(), C.byref(self._shape(feature_map.shape[0])),
-                                                  C.byref(tg), grad_loss.data_ptr(), grad_head.data_ptr(), self._stream()),
-                       "ppn_loss_backward")
+            if opt is None:
+                _lib.check(self.lib.ppn_loss_backward(feature_map.data_ptr(), C.byref(self._shape(B)), C.byref(tg),
+                                                      grad_loss.data_ptr(), grad_head.data_ptr(), self._stream()),
+                           "ppn_loss_backward")
+            else:
+                _lib.check(self.lib.ppn_loss_backward_opt(feature_map.data_ptr(), C.byref(self._shape(B, opt[0])), C.byref(tg),
+                                                          C.byref(opt[1]), grad_loss.data_ptr(), grad_head.data_ptr(),
+                                                          self._stream()),
+                           "ppn_loss_backward_opt")
         return grad_head

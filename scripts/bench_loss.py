@@ -2,6 +2,13 @@
 the copy bandwidth measured in the same run.
 
     python scripts/bench_loss.py [--iters 30] > profiles/bench_loss.txt
+    python scripts/bench_loss.py --amp [--iters 30] > profiles/bench_loss_amp.txt
+
+--amp adds, per shape, the mixed-precision rows: fp16 and bf16 heads, each with fp32 and with 16-bit te / weight_ij
+(ppn_loss_forward_opt / ppn_loss_backward_opt); the upcast route an AMP user has without them (crit(head.float(), ...)
+under autograd, the fp32 gradient cast back to the head's dtype by autograd); and the torch composite on the 16-bit
+head.  Algorithmic bytes are counted per dtype: a 16-bit element is 2 bytes.  The upcast route also counts its two
+casts (read the 16-bit head, write it in fp32; read the fp32 gradient, write it in 16 bits).
 
 Shapes: cfg2 (mpii16: K16 / E15, 12x12 grid, 9x9 window) at B = 512 and the reference's native shape (K18 / E17,
 24x24, 21x21) at B = 64; targets from TargetEncoder on random annotation sets, heads sigmoid(randn).  Every input
@@ -23,13 +30,14 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import encode_gt  # noqa: E402  (inputs and the composite baseline)
 from oracle import ppn_loss as L  # noqa: E402
-from pytorch_pose_proposal_network_b200 import PPNLoss  # noqa: E402
+from pytorch_pose_proposal_network_b200 import PPNLoss, _lib  # noqa: E402
 from pytorch_pose_proposal_network_b200.config import PRESETS  # noqa: E402
 from pytorch_pose_proposal_network_b200.dataset import TargetEncoder  # noqa: E402
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--iters", type=int, default=30)
 ap.add_argument("--warmup", type=int, default=3)
+ap.add_argument("--amp", action="store_true", help="also the fp16 / bf16 rows")
 a = ap.parse_args()
 assert torch.cuda.is_available(), "bench_loss measures on the GPU; there is nothing to measure without one"
 
@@ -93,8 +101,79 @@ def peak_extra(fn):
     return torch.cuda.max_memory_allocated() - base
 
 
+def amp_rows(tag, cfg, B, crit, head32, targets32, ws, loss, g, lam):
+    """The mixed-precision rows of one shape (see the module docstring)."""
+    i_wij, i_te = L.ARG_ORDER.index("weight_ij"), L.ARG_ORDER.index("te")
+    codes = {torch.float32: _lib.HEAD_F32, torch.float16: _lib.HEAD_F16, torch.bfloat16: _lib.HEAD_BF16}
+    name = {torch.float32: "f32", torch.float16: "f16", torch.bfloat16: "bf16"}
+    L_el, C_el, S_el = cfg.E * cfg.S * cfg.HW, cfg.C * cfg.HW, 8 * cfg.K * cfg.HW
+
+    def per_img(hb, lb):                                              # forward, backward bytes per image
+        fwd = C_el * hb + 2 * L_el * lb + S_el * 4
+        return fwd, fwd + C_el * hb
+
+    for hd in (torch.float16, torch.bfloat16):
+        head = head32.to(hd)
+        res, mem = {}, {}
+        for ld in (torch.float32, hd):
+            targets = list(targets32)
+            targets[i_wij], targets[i_te] = targets32[i_wij].to(ld), targets32[i_te].to(ld)
+            lb = 4 if ld == torch.float32 else 2
+            fb, bb = per_img(2, lb)
+            shape, tg = crit._shape(B, codes[hd]), crit._targets_struct(targets)
+            opt = _lib.PPNLossOptions(codes[ld])
+            grad = torch.empty_like(head)
+            stream = crit._stream()
+            fwd_args = (C.c_void_p(head.data_ptr()), C.byref(shape), C.byref(tg), C.byref(opt), C.c_void_p(loss.data_ptr()),
+                        C.c_void_p(ws.data_ptr()), C.c_size_t(ws.numel()), stream)
+            bwd_args = (C.c_void_p(head.data_ptr()), C.byref(shape), C.byref(tg), C.byref(opt), C.c_void_p(g.data_ptr()),
+                        C.c_void_p(grad.data_ptr()), stream)
+            assert crit.lib.ppn_loss_forward_opt(*fwd_args) == 0 and crit.lib.ppn_loss_backward_opt(*bwd_args) == 0
+            fm = head.clone().requires_grad_(True)
+
+            def fused_fb():
+                fm.grad = None
+                sum(l * t for l, t in zip(lam, crit(fm, *targets))).backward()
+
+            lt = f"{name[hd]} head, {name[ld]} limb"
+            res[f"{lt} forward"] = (timed(lambda: crit.lib.ppn_loss_forward_opt(*fwd_args)), fb)
+            res[f"{lt} backward"] = (timed(lambda: crit.lib.ppn_loss_backward_opt(*bwd_args)), bb)
+            res[f"{lt} fwd+bwd"] = (timed(fused_fb), fb + bb)
+            fm.grad = None
+            mem[lt] = peak_extra(fused_fb)
+            if ld == hd:
+                def composite_fb():
+                    fm.grad = None
+                    sum(l * t for l, t in zip(lam, L.loss_terms(fm, *targets, cfg))).backward()
+                res[f"composite on {name[hd]} fwd+bwd"] = (timed(composite_fb), fb + bb)
+            del grad, fm
+        # the upcast route: an fp32 copy of the head, the fp32 loss on it (fp32 limb targets), the gradient cast back
+        fm = head.clone().requires_grad_(True)
+
+        def upcast_fb():
+            fm.grad = None
+            sum(l * t for l, t in zip(lam, crit(fm.float(), *targets32))).backward()
+
+        fb, bb = per_img(4, 4)
+        res[f"upcast {name[hd]} -> f32 fwd+bwd"] = (timed(upcast_fb), fb + bb + C_el * (2 + 4) + C_el * (4 + 2))
+        fm.grad = None
+        mem["upcast"] = peak_extra(upcast_fb)
+        del fm, head
+        for path, (ms, pi) in res.items():
+            gbs = B * pi / ms / 1e6
+            print(f"{tag:<18}{path:<32}{ms:>9.3f}{gbs:>9.0f}{gbs / copy_gbs:>8.2f}")
+        for k, (fb, bb) in ((f"{name[hd]} head, f32 limb", per_img(2, 4)), (f"{name[hd]} head, {name[hd]} limb", per_img(2, 2))):
+            print(f"{tag:<18}{k}: algorithmic bytes per image: forward {fb / 1e6:.2f} MB, backward {bb / 1e6:.2f} MB, "
+                  f"peak memory fwd+bwd {mem[k] / 1e9:.2f} GB")
+        up = res[f"upcast {name[hd]} -> f32 fwd+bwd"][0]
+        print(f"{tag:<18}upcast route peak memory fwd+bwd {mem['upcast'] / 1e9:.2f} GB; fused fwd+bwd speed-up over it: "
+              f"{name[hd]} limb {up / res[f'{name[hd]} head, {name[hd]} limb fwd+bwd'][0]:.2f}x, "
+              f"f32 limb {up / res[f'{name[hd]} head, f32 limb fwd+bwd'][0]:.2f}x")
+        torch.cuda.empty_cache()
+
+
 print()
-print(f"{'shape':<18}{'path':<28}{'ms':>9}{'GB/s':>9}{'/copy':>8}")
+print(f"{'shape':<18}{'path':<32}{'ms':>9}{'GB/s':>9}{'/copy':>8}")
 for name, B in (("cfg2", 512), ("native", 64)):
     cfg = PRESETS[name]()
     head, targets = inputs(cfg, B)
@@ -147,7 +226,7 @@ for name, B in (("cfg2", 512), ("native", 64)):
     torch.cuda.synchronize()
     for path, (ms, per_img) in res.items():
         gbs = B * per_img / ms / 1e6
-        print(f"{tag:<18}{path:<28}{ms:>9.3f}{gbs:>9.0f}{gbs / copy_gbs:>8.2f}")
+        print(f"{tag:<18}{path:<32}{ms:>9.3f}{gbs:>9.0f}{gbs / copy_gbs:>8.2f}")
     print(f"{tag:<18}host enqueue per fused call: {host_us:.1f} us")
     fm.grad = None                                                    # the gradient counts in each path's peak
     mem_fused = peak_extra(fused_fb)
@@ -156,5 +235,7 @@ for name, B in (("cfg2", 512), ("native", 64)):
     print(f"{tag:<18}algorithmic bytes per image: forward {per_img_fwd / 1e6:.2f} MB, backward {per_img_bwd / 1e6:.2f} MB")
     print(f"{tag:<18}peak memory beyond the inputs (gradient included), fwd+bwd: fused {mem_fused / 1e9:.2f} GB, composite {mem_comp / 1e9:.2f} GB")
     print(f"{tag:<18}fwd+bwd speed-up over the composite: {res['composite fwd+bwd'][0] / res['fused fwd+bwd (autograd)'][0]:.1f}x")
+    if a.amp:
+        amp_rows(tag, cfg, B, crit, head, targets, ws, loss, g, lam)
     del head, targets, crit, grad, fm, ws, loss
     torch.cuda.empty_cache()
