@@ -28,6 +28,8 @@
  *   ppn_loss_forward ....... the consumer of those targets: PPNLoss.forward, main.py:125-216 (five terms)
  *   ppn_loss_backward ...... its autograd backward with respect to the head tensor
  *   ppn_loss_*_opt ......... the same for fp16 / bf16 heads and limb targets (mixed-precision training)
+ *   ppn_loss_*_logits ...... the same on the conv output before model.py's final sigmoid, the sigmoid fused in
+ *   ppn_sigmoid ............ that sigmoid alone, elementwise (model.py:136 with the loss's exact values)
  *
  * Conventions
  *   - plain C: pointers and sizes only; no CUDA or torch types.  `stream` is a cudaStream_t
@@ -411,6 +413,28 @@ int ppn_loss_backward_opt(const void* head, const PPNShape* shape, const PPNTarg
  * bf16 0.000499725...).  The eight small grids are fp32 as above; shape->head_dtype is not used. */
 int ppn_encode_targets_opt(const PPNPeople* people, const PPNShape* shape, const int32_t* edges,
                            const PPNTargets* out, int32_t limb_dtype, void* stream);
+
+/* ---- the loss on logits: the network's final sigmoid fused into the loss (BCEWithLogitsLoss style) ----------
+ * `logits` is the conv output BEFORE model.py's sigmoid (model.py:133-136), laid out like the head tensor, and every
+ * one of its C channels (resp, conf, x, y, w, h and the limb block) is taken through
+ *   s = 1 / (1 + expf(-x))          fp32: libdevice expf, one add, one IEEE division (-inf gives 0, +inf gives 1)
+ * after a 16-bit logit is widened exactly.  The loss above is then applied to s, operation for operation; s stays
+ * fp32 (it is not rounded to the head's type).  With g_s the fp32 gradient ppn_loss_backward_opt forms for s,
+ *   grad_logits = (g_s * (1 - s)) * s                   (each operation rounded once: torch's sigmoid_backward)
+ * rounded once (to nearest even, overflow to +-inf) to the head's type.  So in fp32 grad_logits equals
+ * ppn_loss_backward(s) followed by torch's sigmoid backward, bit for bit, for s = ppn_sigmoid(logits); and a 16-bit
+ * call equals the fp32 call on the widened inputs, the gradient converted to the head's type.
+ * Types, alignment, workspace (ppn_loss_workspace_bytes_opt) and every PPN_E_* answer are those of the _opt exports;
+ * grad_logits [B, C, H, W] has the head's type and every element is written.  The caller reads loss[5] and grad_logits
+ * in place of the same results on sigmoid(logits); nothing else changes.
+ *   ppn_sigmoid: y[i] = s(x[i]) for i < n, x of x_dtype (PPN_HEAD_*; PPN_E_BADARG otherwise, checked first), y fp32:
+ *                the values the two loss exports use, e.g. to build from a logits model the head tensor that the
+ *                parse entry points read.  n = 0 is a no-op; x and y need the alignment of their element. */
+int ppn_loss_forward_logits(const void* logits, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                            float* loss, void* workspace, size_t workspace_bytes, void* stream);
+int ppn_loss_backward_logits(const void* logits, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                             const float* grad_loss, void* grad_logits, void* stream);
+int ppn_sigmoid(const void* x, int32_t x_dtype, float* y, size_t n, void* stream);
 
 #ifdef __cplusplus
 }

@@ -125,6 +125,11 @@ EXPORTS = {
                                         C.c_void_p, C.c_void_p, C.c_void_p]),
     "ppn_encode_targets_opt": (C.c_int, [C.POINTER(PPNPeople), C.POINTER(PPNShape), i32p, C.POINTER(PPNTargets), C.c_int32,
                                          C.c_void_p]),
+    "ppn_loss_forward_logits": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.POINTER(PPNLossOptions),
+                                          C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ppn_loss_backward_logits": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.POINTER(PPNLossOptions),
+                                           C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ppn_sigmoid": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
     "ppn_debug_argmax_items": (C.c_int, [C.POINTER(PPNShape), C.c_int32, i32p, i32p, i32p, C.c_int32]),
     "ppn_timeline": (C.c_int, [C.c_void_p, C.c_int32]),
     "ppn_profile_enable": (C.c_int, [C.c_int32]),

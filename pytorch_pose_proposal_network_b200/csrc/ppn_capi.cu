@@ -1082,9 +1082,10 @@ int ppn_loss_workspace_bytes(const PPNShape* shape, size_t* bytes) {
     return ppn_loss_workspace_bytes_opt(shape, &kLossF32, bytes);
 }
 
-// PPNLoss.forward (main.py:125-216): the five batch-mean terms into loss[5]
-int ppn_loss_forward_opt(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
-                         float* loss, void* workspace, size_t workspace_bytes, void* stream) {
+namespace {
+// the forward and backward exports with the head as the sigmoid's output (from_logits false) or its input (true)
+int loss_forward(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                 float* loss, void* workspace, size_t workspace_bytes, void* stream, bool from_logits) {
     ppn::LossArgs a;
     int rc = loss_args(head, shape, targets, opt, &a);
     if (rc) return rc;
@@ -1093,7 +1094,27 @@ int ppn_loss_forward_opt(const void* head, const PPNShape* shape, const PPNTarge
     a.partial = static_cast<double*>(workspace);
     int sms = 0;
     if ((rc = sm_count(&sms))) return rc;
-    return cuda_rc(ppn::launch_loss_forward(a, loss, sms, (cudaStream_t)stream));
+    return cuda_rc(ppn::launch_loss_forward(a, loss, sms, (cudaStream_t)stream, from_logits));
+}
+
+int loss_backward(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                  const float* grad_loss, void* grad_head, void* stream, bool from_logits) {
+    ppn::LossArgs a;
+    int rc = loss_args(head, shape, targets, opt, &a);
+    if (rc) return rc;
+    if (bad_f32(grad_loss) || bad_ptr(grad_head, elem_bytes(shape))) return PPN_E_BADARG;
+    a.grad_loss = grad_loss;
+    a.grad = grad_head;
+    int sms = 0;
+    if ((rc = sm_count(&sms))) return rc;
+    return cuda_rc(ppn::launch_loss_backward(a, sms, (cudaStream_t)stream, from_logits));
+}
+}  // namespace
+
+// PPNLoss.forward (main.py:125-216): the five batch-mean terms into loss[5]
+int ppn_loss_forward_opt(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                         float* loss, void* workspace, size_t workspace_bytes, void* stream) {
+    return loss_forward(head, shape, targets, opt, loss, workspace, workspace_bytes, stream, false);
 }
 
 int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets* targets, float* loss,
@@ -1105,21 +1126,31 @@ int ppn_loss_forward(const float* head, const PPNShape* shape, const PPNTargets*
 // PPNLoss's backward under autograd (loss.backward() in main.py's training step), with respect to the head only
 int ppn_loss_backward_opt(const void* head, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
                           const float* grad_loss, void* grad_head, void* stream) {
-    ppn::LossArgs a;
-    int rc = loss_args(head, shape, targets, opt, &a);
-    if (rc) return rc;
-    if (bad_f32(grad_loss) || bad_ptr(grad_head, elem_bytes(shape))) return PPN_E_BADARG;
-    a.grad_loss = grad_loss;
-    a.grad = grad_head;
-    int sms = 0;
-    if ((rc = sm_count(&sms))) return rc;
-    return cuda_rc(ppn::launch_loss_backward(a, sms, (cudaStream_t)stream));
+    return loss_backward(head, shape, targets, opt, grad_loss, grad_head, stream, false);
 }
 
 int ppn_loss_backward(const float* head, const PPNShape* shape, const PPNTargets* targets, const float* grad_loss,
                       float* grad_head, void* stream) {
     const int rc = check_f32_loss(shape);
     return rc ? rc : ppn_loss_backward_opt(head, shape, targets, &kLossF32, grad_loss, grad_head, stream);
+}
+
+// the loss on the conv output before model.py's final sigmoid (model.py:133-136), the sigmoid fused in
+int ppn_loss_forward_logits(const void* logits, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                            float* loss, void* workspace, size_t workspace_bytes, void* stream) {
+    return loss_forward(logits, shape, targets, opt, loss, workspace, workspace_bytes, stream, true);
+}
+
+int ppn_loss_backward_logits(const void* logits, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
+                             const float* grad_loss, void* grad_logits, void* stream) {
+    return loss_backward(logits, shape, targets, opt, grad_loss, grad_logits, stream, true);
+}
+
+int ppn_sigmoid(const void* x, int32_t x_dtype, float* y, size_t n, void* stream) {
+    if (x_dtype < PPN_HEAD_F32 || x_dtype > PPN_HEAD_BF16) return PPN_E_BADARG;
+    if (n == 0) return PPN_OK;
+    if (bad_ptr(x, dtype_bytes(x_dtype)) || bad_f32(y)) return PPN_E_BADARG;
+    return cuda_rc(ppn::launch_sigmoid(x, x_dtype, y, n, (cudaStream_t)stream));
 }
 
 int ppn_debug_argmax_items(const PPNShape* shape, int32_t sms, int32_t* info, int32_t* first, int32_t* size, int32_t max_items) {

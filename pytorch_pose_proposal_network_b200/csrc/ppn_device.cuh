@@ -90,6 +90,11 @@ template <typename T> __device__ __forceinline__ uint32_t pack2(float lo, float 
     return bits16(narrow<T>(lo)) | (bits16(narrow<T>(hi)) << 16);
 }
 
+// torch.sigmoid's fp32 expression, 1 / (1 + exp(-x)): libdevice expf, one add, one IEEE division.  Shared by the
+// fused head (model.py:133-136) and the loss on logits, so that a model trained through the one is parsed through
+// the other with the same values; -inf gives 0, +inf gives 1.
+__device__ __forceinline__ float sigmoid_f32(float x) { return __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-x))); }
+
 // ---- the reference's cell arithmetic --------------------------------------------------
 // delta = resp * conf  (rt_test.py:130)
 template <typename T>

@@ -148,8 +148,7 @@ __device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity, 
 // through the exact rescan; with 1e-3 it is ~2 %.)
 constexpr float kSureStep = 1e-3f, kSureRange = 6.0f;
 
-// torch.sigmoid's fp32 expression, 1 / (1 + exp(-x)): libdevice expf, one add, one IEEE division
-__device__ __forceinline__ float sigmoid_f32(float x) { return __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-x))); }
+// sigmoid_f32 (ppn_device.cuh): torch.sigmoid's fp32 expression, libdevice expf, one add, one IEEE division
 
 // Does a logit x that exceeds every logit so far beat the standing arg-max, whose logit is bx <= x?  numpy sees sigmoid
 // values: only if sigmoid(x) > sigmoid(bx) (a tie keeps the earlier index), and never once a NaN stands.  Out of line:

@@ -190,8 +190,12 @@ struct LossArgs {
 };
 void loss_plan(LossArgs* a);
 size_t loss_workspace_bytes(const LossArgs& a);
-// two launches: the streaming kernel (CTA partials into a.partial), then the fixed-order sum into loss[5]
-cudaError_t launch_loss_forward(LossArgs a, float* loss, int sms, cudaStream_t st);
-cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st);
+// two launches: the streaming kernel (CTA partials into a.partial), then the fixed-order sum into loss[5].
+// from_logits: a.head holds the logits; the kernels apply sigmoid_f32 to every head element and the sigmoid's
+// derivative to every gradient element (ppn_loss.cu)
+cudaError_t launch_loss_forward(LossArgs a, float* loss, int sms, cudaStream_t st, bool from_logits = false);
+cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st, bool from_logits = false);
+// y[i] = sigmoid_f32(x[i]) for x of HeadDtype `dtype`, y fp32 (ppn_sigmoid)
+cudaError_t launch_sigmoid(const void* x, int dtype, float* y, size_t n, cudaStream_t st);
 
 }  // namespace ppn

@@ -55,6 +55,15 @@
 //   w        sw = sqrt(w + eps)   st = sqrt(tw + eps);  grad = cs * (weight * ((sw - st) / sw)) + dpw * inW
 //                                                                               (h likewise with th, dph, inH)
 // min / max are fminf / fmaxf: the inputs are taken to be finite (a NaN head is not a training state).
+//
+// From logits (kLogits, the *_logits exports): the head holds the conv output x before the network's sigmoid
+// (model.py:133-136), for every channel.  Each head element is widened as above and replaced at once by
+// s = sigmoid_f32(x) (ppn_device.cuh: libdevice expf, one add, one IEEE division; +-inf gives 0 or 1); everything
+// above runs on s, operation for operation, and s is never narrowed.  A gradient element g_s (fp32, before any
+// narrowing) becomes
+//   grad_x = (g_s * (1 - s)) * s                                                 (torch's sigmoid_backward)
+// and only then is stored, rounded once to the head's type.  The sigmoid-input instantiations (kLogits = false)
+// compile to what they were before this path existed.
 #include <algorithm>
 #include <atomic>
 
@@ -68,6 +77,8 @@ constexpr int kLossThreads = 256;
 constexpr int kSmallCells = 1024;      // cells of the [B, K, H, W] planes per small item
 constexpr int kLimbChunk = 8192;       // limb elements per limb item: 32 KB of each fp32 stream
 constexpr int kLimbUnroll = 4;         // vector steps whose loads a thread issues before it computes
+constexpr int kLogitsUnroll = 1;       // the same on logits: the sigmoid makes them issue-bound, and 1 (48-62 registers,
+                                       // 4+ CTAs per SM) measured 7-19 % faster per kernel than 4 (DESIGN.md §11)
 constexpr float kEps = 1e-6f;          // config.EPSILON
 
 // ---- streaming element access (no L1 allocation), widened to / narrowed from fp32 ------------------------------
@@ -136,15 +147,24 @@ struct Cell {
     float delta, weight, txh, tyh, tx, ty, tw, th;          // targets
 };
 
-template <typename TH>
+// a head element as the loss uses it: the widened value, or its sigmoid when the head holds logits
+template <bool kLogits> __device__ __forceinline__ float act(float v) {
+    if constexpr (kLogits) return sigmoid_f32(v); else return v;
+}
+// the gradient of the stored head element from g, the gradient of the value act() gave (s)
+template <bool kLogits> __device__ __forceinline__ float chain(float g, float s) {
+    if constexpr (kLogits) return __fmul_rn(__fmul_rn(g, __fsub_rn(1.0f, s)), s); else return g;
+}
+
+template <typename TH, bool kLogits>
 __device__ __forceinline__ Cell load_cell(const LossArgs& a, long long i) {
     const long long KHW = (long long)a.K * a.HW;
     const long long b = i / KHW, r = i - b * KHW;
     const TH* img = static_cast<const TH*>(a.head) + (size_t)b * a.img_stride + (size_t)r;
     const size_t KH = (size_t)KHW;
     Cell c;
-    c.resp = ldw(img);          c.conf = ldw(img + KH);     c.x = ldw(img + 2 * KH);
-    c.y = ldw(img + 3 * KH);    c.w = ldw(img + 4 * KH);    c.h = ldw(img + 5 * KH);
+    c.resp = act<kLogits>(ldw(img));          c.conf = act<kLogits>(ldw(img + KH));     c.x = act<kLogits>(ldw(img + 2 * KH));
+    c.y = act<kLogits>(ldw(img + 3 * KH));    c.w = act<kLogits>(ldw(img + 4 * KH));    c.h = act<kLogits>(ldw(img + 5 * KH));
     c.delta = lds(a.delta + i); c.weight = lds(a.weight + i);
     c.txh = lds(a.tx_half + i); c.tyh = lds(a.ty_half + i);
     c.tx = lds(a.tx + i);       c.ty = lds(a.ty + i);       c.tw = lds(a.tw + i);       c.th = lds(a.th + i);
@@ -225,6 +245,14 @@ __device__ __forceinline__ float limb_term(float e, float t, float w) { return _
 __device__ __forceinline__ float limb_grad(float cl, float e, float t, float w) {
     return __fmul_rn(cl, __fmul_rn(w, __fsub_rn(e, t)));
 }
+// the same from the stored head element h
+template <bool kLogits> __device__ __forceinline__ float limb_term_at(float h, float t, float w) {
+    return limb_term(act<kLogits>(h), t, w);
+}
+template <bool kLogits> __device__ __forceinline__ float limb_grad_at(float cl, float h, float t, float w) {
+    const float e = act<kLogits>(h);
+    return chain<kLogits>(limb_grad(cl, e, t, w), e);
+}
 
 // deterministic CTA sum of 5 doubles; thread 0..4 store the CTA's partials
 __device__ __forceinline__ void cta_store(double acc[5], double* out) {
@@ -245,10 +273,11 @@ __device__ __forceinline__ void cta_store(double acc[5], double* out) {
     }
 }
 
-template <typename TH, typename TL>
+template <typename TH, typename TL, bool kLogits>
 __global__ void __launch_bounds__(kLossThreads)
 loss_forward_kernel(LossArgs a) {
     constexpr int VE = vec_elems<TH, TL>();
+    constexpr int UN = kLogits ? kLogitsUnroll : kLimbUnroll;
     double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
     const int tid = threadIdx.x;
     const long long n_cells = (long long)a.B * a.K * a.HW;
@@ -256,7 +285,7 @@ loss_forward_kernel(LossArgs a) {
         if (j < a.small_items) {
             const long long c1 = min(n_cells, (j + 1) * kSmallCells);
             for (long long i = j * kSmallCells + tid; i < c1; i += kLossThreads) {
-                const Cell c = load_cell<TH>(a, i);
+                const Cell c = load_cell<TH, kLogits>(a, i);
                 const Iou u = iou_of(a, c, i);
                 acc[0] += (double)sq(__fsub_rn(c.resp, c.delta));
                 acc[1] += (double)__fmul_rn(c.delta, sq(__fsub_rn(c.conf, u.iou)));
@@ -268,30 +297,30 @@ loss_forward_kernel(LossArgs a) {
             continue;
         }
         const LimbItem<TH, TL> it = limb_item<TH, TL>(a, j - a.small_items, false);
-        if (tid < it.pro) acc[4] += (double)limb_term(ldw(it.hp + tid), ldw(it.tp + tid), ldw(it.wp + tid));
+        if (tid < it.pro) acc[4] += (double)limb_term_at<kLogits>(ldw(it.hp + tid), ldw(it.tp + tid), ldw(it.wp + tid));
         int s0 = it.start;
         if (it.vec) {
             const int nv = (it.end - it.start) / VE;
-            for (int v0 = tid; v0 < nv; v0 += kLimbUnroll * kLossThreads) {
-                Vec<TH, VE> hv[kLimbUnroll];
-                Vec<TL, VE> tv[kLimbUnroll], wv[kLimbUnroll];
+            for (int v0 = tid; v0 < nv; v0 += UN * kLossThreads) {
+                Vec<TH, VE> hv[UN];
+                Vec<TL, VE> tv[UN], wv[UN];
 #pragma unroll
-                for (int u = 0; u < kLimbUnroll; ++u) {
+                for (int u = 0; u < UN; ++u) {
                     const size_t e = (size_t)it.start + (size_t)(v0 + u * kLossThreads) * VE;
                     if (v0 + u * kLossThreads < nv) { hv[u].load(it.hp + e); tv[u].load(it.tp + e); wv[u].load(it.wp + e); }
                 }
 #pragma unroll
-                for (int u = 0; u < kLimbUnroll; ++u) {
+                for (int u = 0; u < UN; ++u) {
                     if (v0 + u * kLossThreads < nv) {
 #pragma unroll
-                        for (int k = 0; k < VE; ++k) acc[4] += (double)limb_term(at(hv[u], k), at(tv[u], k), at(wv[u], k));
+                        for (int k = 0; k < VE; ++k) acc[4] += (double)limb_term_at<kLogits>(at(hv[u], k), at(tv[u], k), at(wv[u], k));
                     }
                 }
             }
             s0 = it.start + VE * nv;
         }
         for (int e = s0 + tid; e < it.end; e += kLossThreads)             // vector tail, or the whole unaligned item
-            acc[4] += (double)limb_term(ldw(it.hp + e), ldw(it.tp + e), ldw(it.wp + e));
+            acc[4] += (double)limb_term_at<kLogits>(ldw(it.hp + e), ldw(it.tp + e), ldw(it.wp + e));
     }
     cta_store(acc, a.partial);
 }
@@ -308,10 +337,11 @@ loss_finalize_kernel(const double* __restrict__ partial, int n, int B, float* __
     if (lane == 0) loss[t] = (float)(v / (double)B);
 }
 
-template <typename TH, typename TL>
+template <typename TH, typename TL, bool kLogits>
 __global__ void __launch_bounds__(kLossThreads)
 loss_backward_kernel(LossArgs a) {
     constexpr int VE = vec_elems<TH, TL>();
+    constexpr int UN = kLogits ? kLogitsUnroll : kLimbUnroll;
     const float Bf = (float)a.B;
     const float cr = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[0]), Bf);
     const float ci = __fdiv_rn(__fmul_rn(2.0f, a.grad_loss[1]), Bf);
@@ -325,7 +355,7 @@ loss_backward_kernel(LossArgs a) {
         if (j < a.small_items) {
             const long long c1 = min(n_cells, (j + 1) * kSmallCells);
             for (long long i = j * kSmallCells + tid; i < c1; i += kLossThreads) {
-                const Cell c = load_cell<TH>(a, i);
+                const Cell c = load_cell<TH, kLogits>(a, i);
                 const Iou u = iou_of(a, c, i);
                 const float g_resp = __fmul_rn(cr, __fsub_rn(c.resp, c.delta));
                 const float g_conf = __fmul_rn(ci, __fmul_rn(c.delta, __fsub_rn(c.conf, u.iou)));
@@ -349,30 +379,31 @@ loss_backward_kernel(LossArgs a) {
                 const long long b = i / KHW, rr = i - b * KHW;
                 TH* gimg = static_cast<TH*>(a.grad) + (size_t)b * a.img_stride + (size_t)rr;
                 const size_t KH = (size_t)KHW;
-                stw(gimg, g_resp);          stw(gimg + KH, g_conf);     stw(gimg + 2 * KH, g_x);
-                stw(gimg + 3 * KH, g_y);    stw(gimg + 4 * KH, g_w);    stw(gimg + 5 * KH, g_h);
+                stw(gimg, chain<kLogits>(g_resp, c.resp));       stw(gimg + KH, chain<kLogits>(g_conf, c.conf));
+                stw(gimg + 2 * KH, chain<kLogits>(g_x, c.x));    stw(gimg + 3 * KH, chain<kLogits>(g_y, c.y));
+                stw(gimg + 4 * KH, chain<kLogits>(g_w, c.w));    stw(gimg + 5 * KH, chain<kLogits>(g_h, c.h));
             }
             continue;
         }
         const LimbItem<TH, TL> it = limb_item<TH, TL>(a, j - a.small_items, true);
-        if (tid < it.pro) stw(it.gp + tid, limb_grad(cl, ldw(it.hp + tid), ldw(it.tp + tid), ldw(it.wp + tid)));
+        if (tid < it.pro) stw(it.gp + tid, limb_grad_at<kLogits>(cl, ldw(it.hp + tid), ldw(it.tp + tid), ldw(it.wp + tid)));
         int s0 = it.start;
         if (it.vec) {
             const int nv = (it.end - it.start) / VE;
-            for (int v0 = tid; v0 < nv; v0 += kLimbUnroll * kLossThreads) {
-                Vec<TH, VE> hv[kLimbUnroll];
-                Vec<TL, VE> tv[kLimbUnroll], wv[kLimbUnroll];
+            for (int v0 = tid; v0 < nv; v0 += UN * kLossThreads) {
+                Vec<TH, VE> hv[UN];
+                Vec<TL, VE> tv[UN], wv[UN];
 #pragma unroll
-                for (int u = 0; u < kLimbUnroll; ++u) {
+                for (int u = 0; u < UN; ++u) {
                     const size_t e = (size_t)it.start + (size_t)(v0 + u * kLossThreads) * VE;
                     if (v0 + u * kLossThreads < nv) { hv[u].load(it.hp + e); tv[u].load(it.tp + e); wv[u].load(it.wp + e); }
                 }
 #pragma unroll
-                for (int u = 0; u < kLimbUnroll; ++u) {
+                for (int u = 0; u < UN; ++u) {
                     if (v0 + u * kLossThreads < nv) {
                         float g[VE];
 #pragma unroll
-                        for (int k = 0; k < VE; ++k) g[k] = limb_grad(cl, at(hv[u], k), at(tv[u], k), at(wv[u], k));
+                        for (int k = 0; k < VE; ++k) g[k] = limb_grad_at<kLogits>(cl, at(hv[u], k), at(tv[u], k), at(wv[u], k));
                         st_vec(it.gp + (size_t)it.start + (size_t)(v0 + u * kLossThreads) * VE, g);
                     }
                 }
@@ -380,7 +411,7 @@ loss_backward_kernel(LossArgs a) {
             s0 = it.start + VE * nv;
         }
         for (int e = s0 + tid; e < it.end; e += kLossThreads)
-            stw(it.gp + e, limb_grad(cl, ldw(it.hp + e), ldw(it.tp + e), ldw(it.wp + e)));
+            stw(it.gp + e, limb_grad_at<kLogits>(cl, ldw(it.hp + e), ldw(it.tp + e), ldw(it.wp + e)));
     }
 }
 
@@ -394,23 +425,55 @@ int grid_for(const void* kernel, std::atomic<int>* per_sm_cache, long long n_ite
     return (int)std::min<long long>(n_items, std::min<long long>((long long)sms * per_sm, kLossMaxCtas));
 }
 
-template <typename TH, typename TL>
+template <typename TH, typename TL, bool kLogits>
 cudaError_t forward_as(const LossArgs& a, float* loss, int sms, cudaStream_t st) {
     static std::atomic<int> per_sm{0};
-    const int grid = grid_for((const void*)loss_forward_kernel<TH, TL>, &per_sm, a.n_items, sms);
-    loss_forward_kernel<TH, TL><<<grid, kLossThreads, 0, st>>>(a);
+    const int grid = grid_for((const void*)loss_forward_kernel<TH, TL, kLogits>, &per_sm, a.n_items, sms);
+    loss_forward_kernel<TH, TL, kLogits><<<grid, kLossThreads, 0, st>>>(a);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     loss_finalize_kernel<<<1, 160, 0, st>>>(a.partial, grid, a.B, loss);
     return cudaGetLastError();
 }
 
-template <typename TH, typename TL>
+template <typename TH, typename TL, bool kLogits>
 cudaError_t backward_as(const LossArgs& a, int sms, cudaStream_t st) {
     static std::atomic<int> per_sm{0};
-    const int grid = grid_for((const void*)loss_backward_kernel<TH, TL>, &per_sm, a.n_items, sms);
-    loss_backward_kernel<TH, TL><<<grid, kLossThreads, 0, st>>>(a);
+    const int grid = grid_for((const void*)loss_backward_kernel<TH, TL, kLogits>, &per_sm, a.n_items, sms);
+    loss_backward_kernel<TH, TL, kLogits><<<grid, kLossThreads, 0, st>>>(a);
     return cudaGetLastError();
+}
+
+// the five (head, limb target) type pairs of LossArgs; the C ABI rejects every other pair before launching
+template <bool kLogits>
+cudaError_t forward_for(const LossArgs& a, float* loss, int sms, cudaStream_t st) {
+    switch (a.head_dtype * 3 + a.limb_dtype) {
+        case HEAD_F32 * 3 + HEAD_F32: return forward_as<float, float, kLogits>(a, loss, sms, st);
+        case HEAD_F16 * 3 + HEAD_F32: return forward_as<__half, float, kLogits>(a, loss, sms, st);
+        case HEAD_F16 * 3 + HEAD_F16: return forward_as<__half, __half, kLogits>(a, loss, sms, st);
+        case HEAD_BF16 * 3 + HEAD_F32: return forward_as<__nv_bfloat16, float, kLogits>(a, loss, sms, st);
+        case HEAD_BF16 * 3 + HEAD_BF16: return forward_as<__nv_bfloat16, __nv_bfloat16, kLogits>(a, loss, sms, st);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+template <bool kLogits>
+cudaError_t backward_for(const LossArgs& a, int sms, cudaStream_t st) {
+    switch (a.head_dtype * 3 + a.limb_dtype) {
+        case HEAD_F32 * 3 + HEAD_F32: return backward_as<float, float, kLogits>(a, sms, st);
+        case HEAD_F16 * 3 + HEAD_F32: return backward_as<__half, float, kLogits>(a, sms, st);
+        case HEAD_F16 * 3 + HEAD_F16: return backward_as<__half, __half, kLogits>(a, sms, st);
+        case HEAD_BF16 * 3 + HEAD_F32: return backward_as<__nv_bfloat16, float, kLogits>(a, sms, st);
+        case HEAD_BF16 * 3 + HEAD_BF16: return backward_as<__nv_bfloat16, __nv_bfloat16, kLogits>(a, sms, st);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+// ppn_sigmoid: the sigmoid the loss applies, elementwise into fp32 (grid-stride; not a hot path)
+template <typename T>
+__global__ void __launch_bounds__(256) sigmoid_kernel(const T* __restrict__ x, float* __restrict__ y, size_t n) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+        y[i] = sigmoid_f32(widen(x[i]));
 }
 
 }  // namespace
@@ -427,27 +490,24 @@ size_t loss_workspace_bytes(const LossArgs& a) {
     return (size_t)ctas * 5 * sizeof(double);
 }
 
-// the five (head, limb target) type pairs of LossArgs; the C ABI rejects every other pair before launching
-cudaError_t launch_loss_forward(LossArgs a, float* loss, int sms, cudaStream_t st) {
-    switch (a.head_dtype * 3 + a.limb_dtype) {
-        case HEAD_F32 * 3 + HEAD_F32: return forward_as<float, float>(a, loss, sms, st);
-        case HEAD_F16 * 3 + HEAD_F32: return forward_as<__half, float>(a, loss, sms, st);
-        case HEAD_F16 * 3 + HEAD_F16: return forward_as<__half, __half>(a, loss, sms, st);
-        case HEAD_BF16 * 3 + HEAD_F32: return forward_as<__nv_bfloat16, float>(a, loss, sms, st);
-        case HEAD_BF16 * 3 + HEAD_BF16: return forward_as<__nv_bfloat16, __nv_bfloat16>(a, loss, sms, st);
-        default: return cudaErrorInvalidValue;
-    }
+cudaError_t launch_loss_forward(LossArgs a, float* loss, int sms, cudaStream_t st, bool from_logits) {
+    return from_logits ? forward_for<true>(a, loss, sms, st) : forward_for<false>(a, loss, sms, st);
 }
 
-cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st) {
-    switch (a.head_dtype * 3 + a.limb_dtype) {
-        case HEAD_F32 * 3 + HEAD_F32: return backward_as<float, float>(a, sms, st);
-        case HEAD_F16 * 3 + HEAD_F32: return backward_as<__half, float>(a, sms, st);
-        case HEAD_F16 * 3 + HEAD_F16: return backward_as<__half, __half>(a, sms, st);
-        case HEAD_BF16 * 3 + HEAD_F32: return backward_as<__nv_bfloat16, float>(a, sms, st);
-        case HEAD_BF16 * 3 + HEAD_BF16: return backward_as<__nv_bfloat16, __nv_bfloat16>(a, sms, st);
+cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st, bool from_logits) {
+    return from_logits ? backward_for<true>(a, sms, st) : backward_for<false>(a, sms, st);
+}
+
+cudaError_t launch_sigmoid(const void* x, int dtype, float* y, size_t n, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    const int grid = (int)std::min<size_t>((n + 255) / 256, 8192);
+    switch (dtype) {
+        case HEAD_F32: sigmoid_kernel<<<grid, 256, 0, st>>>(static_cast<const float*>(x), y, n); break;
+        case HEAD_F16: sigmoid_kernel<<<grid, 256, 0, st>>>(static_cast<const __half*>(x), y, n); break;
+        case HEAD_BF16: sigmoid_kernel<<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), y, n); break;
         default: return cudaErrorInvalidValue;
     }
+    return cudaGetLastError();
 }
 
 }  // namespace ppn

@@ -17,6 +17,11 @@ Under mixed precision (the reference trains under apex AMP, main.py:282-289) the
 weight_ij may be stored in the head's type (``TargetEncoder(cfg, limb_dtype=...)``): the loss is the fp32 loss on
 the exactly widened inputs and the gradient comes back in the head's type, rounded once — no fp32 copy of the head.
 
+``PPNLoss(cfg, from_logits=True)`` takes the conv output before the model's final sigmoid, as ``BCEWithLogitsLoss``
+does: the kernels apply the sigmoid as they load each element and its derivative as they store each gradient, so
+the sigmoid's own pass over the head and autograd's sigmoid backward never run.  :func:`sigmoid` is that sigmoid
+alone (fp32 out), for parsing the output of a model trained that way.
+
 The reference's training loop is not part of this project: the loss is specified by the float64 restatement
 described in DESIGN.md §11 (IoU differentiable in x, y, w, h; eps = 1e-6 in the IoU denominator; L_resp
 unweighted), not by bit parity with main.py.
@@ -57,6 +62,22 @@ class _PPNLossFunction(torch.autograd.Function):
         return (None, grad) + (None,) * len(ARG_ORDER)
 
 
+def sigmoid(x: torch.Tensor) -> torch.Tensor:
+    """1 / (1 + exp(-x)) of a float32 / float16 / bfloat16 CUDA tensor, as a new float32 tensor of the same shape:
+    the exact values ``PPNLoss(cfg, from_logits=True)`` computes from logits (ppn_sigmoid), e.g. the head tensor that
+    :class:`parser.PoseParser` reads from a model trained on logits.  A 16-bit input is widened exactly; the result is
+    not rounded back to it.  Runs on the current stream of x's device."""
+    if not isinstance(x, torch.Tensor) or x.dtype not in HEAD_DTYPES or x.device.type != "cuda":
+        raise ValueError(f"sigmoid takes a float32, float16 or bfloat16 CUDA tensor, got "
+                         f"{(x.dtype, x.device) if isinstance(x, torch.Tensor) else type(x)}")
+    x = x.contiguous()
+    y = torch.empty(x.shape, dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().ppn_sigmoid(x.data_ptr(), HEAD_DTYPES[x.dtype], y.data_ptr(), x.numel(),
+                                          C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)), "ppn_sigmoid")
+    return y
+
+
 class PPNLoss(torch.nn.Module):
     """``criterion(feature_map, delta, weight, weight_ij, tx_half, ty_half, tx, ty, tw, th, te)`` ->
     ``(loss_resp, loss_iou, loss_coor, loss_size, loss_limb)``, five 0-dim fp32 tensors on the head's device.
@@ -72,10 +93,16 @@ class PPNLoss(torch.nn.Module):
     inputs, rounded once to nearest even (overflow to +-inf, which a GradScaler detects).  The gradient flows into ``feature_map``
     only.  Terms that do not reach the final loss get no upstream gradient and are skipped in the backward; the
     upstream gradients never travel to the host.
+
+    from_logits: feature_map (in every method) is the conv output BEFORE the model's sigmoid, and every channel goes
+    through s = :func:`sigmoid` (in fp32, also for a 16-bit feature_map) before the loss above is applied to s.  The
+    gradient is that of the logits: the fp32 gradient of s times (1 - s) times s, rounded once to feature_map's
+    dtype.  Types, shapes and checks are the same.
     """
 
-    def __init__(self, cfg: PPNConfig, device=None):
+    def __init__(self, cfg: PPNConfig, device=None, from_logits: bool = False):
         super().__init__()
+        self.from_logits = bool(from_logits)
         if not torch.cuda.is_available():
             raise RuntimeError("PPNLoss needs a CUDA device: there is no CPU path")
         self.cfg = cfg
@@ -193,10 +220,23 @@ class PPNLoss(torch.nn.Module):
         te = targets[ARG_ORDER.index("te")]
         return HEAD_DTYPES[feature_map.dtype], _lib.PPNLossOptions(HEAD_DTYPES[te.dtype])
 
+    def _logits_options(self, feature_map, targets):
+        """(shape dtype code, PPNLossOptions) of the _logits exports, which take every dtype pair."""
+        te = targets[ARG_ORDER.index("te")]
+        return HEAD_DTYPES[feature_map.dtype], _lib.PPNLossOptions(HEAD_DTYPES[te.dtype])
+
     def _launch_forward(self, feature_map, targets, loss):
         B = feature_map.shape[0]
         ws = self._workspace(B)                 # the same for every dtype (ppn_loss_workspace_bytes_opt)
         tg = self._targets_struct(targets)
+        if self.from_logits:
+            code, opt = self._logits_options(feature_map, targets)
+            with self._guard():
+                _lib.check(self.lib.ppn_loss_forward_logits(feature_map.data_ptr(), C.byref(self._shape(B, code)), C.byref(tg),
+                                                            C.byref(opt), loss.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                            self._stream()),
+                           "ppn_loss_forward_logits")
+            return loss
         opt = self._options(feature_map, targets)
         with self._guard():
             if opt is None:
@@ -213,6 +253,14 @@ class PPNLoss(torch.nn.Module):
     def _launch_backward(self, feature_map, targets, grad_loss, grad_head):
         B = feature_map.shape[0]
         tg = self._targets_struct(targets)
+        if self.from_logits:
+            code, opt = self._logits_options(feature_map, targets)
+            with self._guard():
+                _lib.check(self.lib.ppn_loss_backward_logits(feature_map.data_ptr(), C.byref(self._shape(B, code)), C.byref(tg),
+                                                             C.byref(opt), grad_loss.data_ptr(), grad_head.data_ptr(),
+                                                             self._stream()),
+                           "ppn_loss_backward_logits")
+            return grad_head
         opt = self._options(feature_map, targets)
         with self._guard():
             if opt is None:

@@ -3,12 +3,18 @@ the copy bandwidth measured in the same run.
 
     python scripts/bench_loss.py [--iters 30] > profiles/bench_loss.txt
     python scripts/bench_loss.py --amp [--iters 30] > profiles/bench_loss_amp.txt
+    python scripts/bench_loss.py --logits [--iters 30] > profiles/bench_loss_logits.txt
 
 --amp adds, per shape, the mixed-precision rows: fp16 and bf16 heads, each with fp32 and with 16-bit te / weight_ij
 (ppn_loss_forward_opt / ppn_loss_backward_opt); the upcast route an AMP user has without them (crit(head.float(), ...)
 under autograd, the fp32 gradient cast back to the head's dtype by autograd); and the torch composite on the 16-bit
 head.  Algorithmic bytes are counted per dtype: a 16-bit element is 2 bytes.  The upcast route also counts its two
 casts (read the 16-bit head, write it in fp32; read the fp32 gradient, write it in 16 bits).
+
+--logits adds, per shape, the loss on logits (PPNLoss(cfg, from_logits=True): ppn_loss_forward_logits /
+ppn_loss_backward_logits) with fp32 logits and targets and with fp16 logits and fp16 te / weight_ij, against today's
+route on the same logits: torch.sigmoid, the sigmoid-input loss, autograd's sigmoid backward.  Its bytes add the
+sigmoid's read and write of the head and the sigmoid backward's two reads and one write.  The logits are randn * 3.
 
 Shapes: cfg2 (mpii16: K16 / E15, 12x12 grid, 9x9 window) at B = 512 and the reference's native shape (K18 / E17,
 24x24, 21x21) at B = 64; targets from TargetEncoder on random annotation sets, heads sigmoid(randn).  Every input
@@ -38,6 +44,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--iters", type=int, default=30)
 ap.add_argument("--warmup", type=int, default=3)
 ap.add_argument("--amp", action="store_true", help="also the fp16 / bf16 rows")
+ap.add_argument("--logits", action="store_true", help="also the loss-on-logits rows")
 a = ap.parse_args()
 assert torch.cuda.is_available(), "bench_loss measures on the GPU; there is nothing to measure without one"
 
@@ -172,6 +179,64 @@ def amp_rows(tag, cfg, B, crit, head32, targets32, ws, loss, g, lam):
         torch.cuda.empty_cache()
 
 
+def logits_rows(tag, cfg, B, targets32, ws, loss, g, lam):
+    """The loss-on-logits rows of one shape (see the module docstring)."""
+    i_wij, i_te = L.ARG_ORDER.index("weight_ij"), L.ARG_ORDER.index("te")
+    codes = {torch.float32: _lib.HEAD_F32, torch.float16: _lib.HEAD_F16}
+    name = {torch.float32: "f32", torch.float16: "f16"}
+    L_el, C_el, S_el = cfg.E * cfg.S * cfg.HW, cfg.C * cfg.HW, 8 * cfg.K * cfg.HW
+    crit, crit_l = PPNLoss(cfg), PPNLoss(cfg, from_logits=True)
+    gen = torch.Generator(device="cuda").manual_seed(1)
+    x32 = torch.randn(B, cfg.C, cfg.H, cfg.W, device="cuda", generator=gen) * 3
+    for hd in (torch.float32, torch.float16):
+        x = x32.to(hd)
+        targets = list(targets32)
+        targets[i_wij], targets[i_te] = targets32[i_wij].to(hd), targets32[i_te].to(hd)
+        eb = 4 if hd == torch.float32 else 2
+        fb = C_el * eb + 2 * L_el * eb + S_el * 4                     # forward bytes per image
+        bb = fb + C_el * eb                                           # backward: the same plus the gradient write
+        shape, tg = crit_l._shape(B, codes[hd]), crit_l._targets_struct(targets)
+        opt = _lib.PPNLossOptions(codes[hd])
+        grad = torch.empty_like(x)
+        stream = crit_l._stream()
+        fwd_args = (C.c_void_p(x.data_ptr()), C.byref(shape), C.byref(tg), C.byref(opt), C.c_void_p(loss.data_ptr()),
+                    C.c_void_p(ws.data_ptr()), C.c_size_t(ws.numel()), stream)
+        bwd_args = (C.c_void_p(x.data_ptr()), C.byref(shape), C.byref(tg), C.byref(opt), C.c_void_p(g.data_ptr()),
+                    C.c_void_p(grad.data_ptr()), stream)
+        assert crit_l.lib.ppn_loss_forward_logits(*fwd_args) == 0 and crit_l.lib.ppn_loss_backward_logits(*bwd_args) == 0
+        fm = x.clone().requires_grad_(True)
+
+        def fused_fb():
+            fm.grad = None
+            sum(l * t for l, t in zip(lam, crit_l(fm, *targets))).backward()
+
+        def today_fb():
+            fm.grad = None
+            sum(l * t for l, t in zip(lam, crit(torch.sigmoid(fm), *targets))).backward()
+
+        lt = f"{name[hd]} logits, {name[hd]} limb"
+        res = {
+            f"{lt} forward": (timed(lambda: crit_l.lib.ppn_loss_forward_logits(*fwd_args)), fb),
+            f"{lt} backward": (timed(lambda: crit_l.lib.ppn_loss_backward_logits(*bwd_args)), bb),
+            f"{lt} fwd+bwd": (timed(fused_fb), fb + bb),
+            f"{name[hd]} sigmoid route fwd+bwd": (timed(today_fb), fb + bb + 2 * C_el * eb + 3 * C_el * eb),
+        }
+        fm.grad = None
+        mem_fused = peak_extra(fused_fb)
+        fm.grad = None
+        mem_today = peak_extra(today_fb)
+        for path, (ms, pi) in res.items():
+            gbs = B * pi / ms / 1e6
+            print(f"{tag:<18}{path:<32}{ms:>9.3f}{gbs:>9.0f}{gbs / copy_gbs:>8.2f}")
+        print(f"{tag:<18}{name[hd]}: algorithmic bytes per image: logits forward {fb / 1e6:.2f} MB, backward {bb / 1e6:.2f} MB, "
+              f"fwd+bwd {(fb + bb) / 1e6:.2f} MB; sigmoid route fwd+bwd {(fb + bb + 5 * C_el * eb) / 1e6:.2f} MB")
+        print(f"{tag:<18}{name[hd]}: peak memory beyond the inputs (gradient included), fwd+bwd: logits {mem_fused / 1e9:.2f} GB, "
+              f"sigmoid route {mem_today / 1e9:.2f} GB; speed-up over the sigmoid route: "
+              f"{res[f'{name[hd]} sigmoid route fwd+bwd'][0] / res[f'{lt} fwd+bwd'][0]:.2f}x")
+        del x, fm, grad
+        torch.cuda.empty_cache()
+
+
 print()
 print(f"{'shape':<18}{'path':<32}{'ms':>9}{'GB/s':>9}{'/copy':>8}")
 for name, B in (("cfg2", 512), ("native", 64)):
@@ -237,5 +302,7 @@ for name, B in (("cfg2", 512), ("native", 64)):
     print(f"{tag:<18}fwd+bwd speed-up over the composite: {res['composite fwd+bwd'][0] / res['fused fwd+bwd (autograd)'][0]:.1f}x")
     if a.amp:
         amp_rows(tag, cfg, B, crit, head, targets, ws, loss, g, lam)
+    if a.logits:
+        logits_rows(tag, cfg, B, targets, ws, loss, g, lam)
     del head, targets, crit, grad, fm, ws, loss
     torch.cuda.empty_cache()
