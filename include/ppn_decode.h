@@ -30,6 +30,8 @@
  *   ppn_loss_*_opt ......... the same for fp16 / bf16 heads and limb targets (mixed-precision training)
  *   ppn_loss_*_logits ...... the same on the conv output before model.py's final sigmoid, the sigmoid fused in
  *   ppn_sigmoid ............ that sigmoid alone, elementwise (model.py:136 with the loss's exact values)
+ *   ppn_ap_match ........... the validation pass's scoring, per image: poseval's eval_helpers.assignGTmulti
+ *   ppn_ap_finalize ........ ... and over the pass: evaluateAP.computeMetrics (computeRPC, VOCap)
  *
  * Conventions
  *   - plain C: pointers and sizes only; no CUDA or torch types.  `stream` is a cudaStream_t
@@ -435,6 +437,59 @@ int ppn_loss_forward_logits(const void* logits, const PPNShape* shape, const PPN
 int ppn_loss_backward_logits(const void* logits, const PPNShape* shape, const PPNTargets* targets, const PPNLossOptions* opt,
                              const float* grad_loss, void* grad_logits, void* stream);
 int ppn_sigmoid(const void* x, int32_t x_dtype, float* y, size_t n, void* stream);
+
+/* ---- multi-person pose AP over the packed result (the validation pass's scoring stage) ----------------------------
+ * Stands in for the poseval fork the reference scores its validation with (main.validate / main.test_output):
+ * eval_helpers.assignGTmulti per image, then evaluateAP.computeMetrics (computeRPC, VOCap) over the pass.  The fork is
+ * not part of this project: the specification is the float64 restatement of DESIGN.md §12.  Joints j < J; the
+ * prediction of joint j is part j + 1 of a human, at the centre of its box (ppn_part_centres), with its part score;
+ * an absent part is a score-0 entry at (0, 0), as evaluation.pred_frame writes it.  Joints j >= K - 1 have no
+ * prediction.
+ * Ground truth, DEVICE pointers: people of image b are rows [person_off[b], person_off[b+1]) of the three arrays. */
+typedef struct PPNPoseGT {
+    const int32_t* person_off;  /* [B + 1]                                                          */
+    const double*  head_box;    /* [n, 4] x1, y1, x2, y2 of the head rectangle                      */
+    const double*  joint_xy;    /* [n, J, 2] x, y                                                   */
+    const uint8_t* joint_valid; /* [n, J] 1 = joint annotated                                       */
+    int32_t        n;           /* rows of the three arrays                                         */
+} PPNPoseGT;
+
+typedef struct PPNAPParams {
+    int32_t n_joints;           /* J, 1..32 (PPN_E_UNSUPPORTED above 32)                             */
+    double  dist_thresh;        /* PCKh threshold: a joint matches if dist / headSize <= it (0.5)    */
+    double  head_scale;         /* headSize = head_scale * |(x2 - x1, y2 - y1)| (0.6)               */
+} PPNAPParams;
+
+/* Per-image match result, caller-owned device memory; slot i of image b stands for the i-th human of the result. */
+typedef struct PPNAPMatch {
+    float*   score;             /* [B, R, J] entry score of (slot, joint), for slots < used[b], joints < min(K - 1, J) */
+    uint8_t* label;             /* [B, R, J] 1 = true positive (same entries)                        */
+    int32_t* used;              /* [B] min(count[b], R of the packed result)                         */
+    int32_t* flags;             /* [B] PPN_AP_* bits                                                 */
+    int32_t* n_gt;              /* [B, J] annotated GT joints of the image (nGTall)                  */
+    int32_t  R;                 /* slot stride of score / label, >= the packed result's R            */
+} PPNAPMatch;
+#define PPN_AP_OVERFLOW 1       /* count[b] > R: humans beyond the slots were never seen             */
+#define PPN_AP_BAD_GT   2       /* more than 64 GT people, or person_off outside [0, n]: GT not used */
+
+/* ppn_ap_match: assignGTmulti on B images of a packed result, one CTA per image (distances in fp64, one rounding per
+ *   operation, dist = sqrt(dx*dx + dy*dy) / headSize, NaN never matches).  A prediction is labelled with its match
+ *   mask against the GT person it is assigned to (the first GT person of maximal PCKh that in turn prefers it, as
+ *   the two arg-max passes of assignGTmulti decide), every other prediction with 0.  Reads `humans` only during the
+ *   call: the parser may overwrite it afterwards.  Up to 64 GT people per image (more: PPN_AP_BAD_GT, checked on the
+ *   device); any R.
+ * ppn_ap_workspace_bytes: scratch of ppn_ap_finalize for N images of R slots and J joints (N * R * J < 2^31).
+ * ppn_ap_finalize: computeMetrics over N images laid out as one PPNAPMatch (images in the order the entries are
+ *   appended): entries of every joint ranked by descending score, equal scores the later-appended entry first, NaN
+ *   first (a CUB segmented radix sort on 64-bit keys in the workspace), then computeRPC and VOCap.  ap, precision,
+ *   recall: [J + 1] fp64 in percent, the last entry the plain mean over the joints.  A joint without entries gives
+ *   0, one with entries and no GT joint NaN recall and AP.  status[3] (int32): images flagged PPN_AP_OVERFLOW, images
+ *   flagged PPN_AP_BAD_GT, entries per joint.  Deterministic: the result depends on the ranked entries alone. */
+int ppn_ap_match(const PPNHumans* humans, int32_t B, int32_t K, const PPNPoseGT* gt, const PPNAPParams* params,
+                 const PPNAPMatch* out, void* stream);
+int ppn_ap_workspace_bytes(int32_t N, int32_t R, int32_t J, size_t* bytes);
+int ppn_ap_finalize(const PPNAPMatch* match, int32_t N, int32_t K, int32_t J, double* ap, double* precision,
+                    double* recall, int32_t* status, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -62,6 +62,24 @@ class PPNLossOptions(C.Structure):
     _fields_ = [("limb_dtype", C.c_int32)]
 
 
+class PPNPoseGT(C.Structure):
+    _fields_ = [("person_off", C.c_void_p), ("head_box", C.c_void_p), ("joint_xy", C.c_void_p),
+                ("joint_valid", C.c_void_p), ("n", C.c_int32)]
+
+
+class PPNAPParams(C.Structure):
+    _fields_ = [("n_joints", C.c_int32), ("dist_thresh", C.c_double), ("head_scale", C.c_double)]
+
+
+class PPNAPMatch(C.Structure):
+    _fields_ = [("score", C.c_void_p), ("label", C.c_void_p), ("used", C.c_void_p), ("flags", C.c_void_p),
+                ("n_gt", C.c_void_p), ("R", C.c_int32)]
+
+
+AP_MAX_JOINTS = 32
+AP_MAX_GT = 64
+
+
 # name -> (restype, argtypes); must list every function of include/ppn_decode.h
 EXPORTS = {
     "ppn_abi_version": (C.c_int, []),
@@ -130,6 +148,11 @@ EXPORTS = {
     "ppn_loss_backward_logits": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNTargets), C.POINTER(PPNLossOptions),
                                            C.c_void_p, C.c_void_p, C.c_void_p]),
     "ppn_sigmoid": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ppn_ap_match": (C.c_int, [C.POINTER(PPNHumans), C.c_int32, C.c_int32, C.POINTER(PPNPoseGT), C.POINTER(PPNAPParams),
+                               C.POINTER(PPNAPMatch), C.c_void_p]),
+    "ppn_ap_workspace_bytes": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_size_t)]),
+    "ppn_ap_finalize": (C.c_int, [C.POINTER(PPNAPMatch), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "ppn_debug_argmax_items": (C.c_int, [C.POINTER(PPNShape), C.c_int32, i32p, i32p, i32p, C.c_int32]),
     "ppn_timeline": (C.c_int, [C.c_void_p, C.c_int32]),
     "ppn_profile_enable": (C.c_int, [C.c_int32]),

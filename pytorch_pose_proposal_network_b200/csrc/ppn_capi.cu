@@ -1153,6 +1153,84 @@ int ppn_sigmoid(const void* x, int32_t x_dtype, float* y, size_t n, void* stream
     return cuda_rc(ppn::launch_sigmoid(x, x_dtype, y, n, (cudaStream_t)stream));
 }
 
+namespace {
+int check_ap_joints(int32_t J) {
+    if (J < 1) return PPN_E_BADARG;
+    return J > ppn::kAPMaxJoints ? PPN_E_UNSUPPORTED : PPN_OK;
+}
+
+int check_ap_match(const PPNAPMatch* m) {
+    if (!m || bad_f32(m->score) || !m->label || bad_ptr(m->used, 4) || bad_ptr(m->flags, 4) || bad_ptr(m->n_gt, 4) || m->R < 1)
+        return PPN_E_BADARG;
+    return PPN_OK;
+}
+
+// N * R entries per joint, J joints: the sort's item count is an int and the append ordinal has 31 bits
+bool ap_fits(long long N, long long R, int J) { return N * R * J <= 0x7fffffffLL; }
+}  // namespace
+
+// eval_helpers.assignGTmulti of the poseval fork, per image of a packed result
+int ppn_ap_match(const PPNHumans* humans, int32_t B, int32_t K, const PPNPoseGT* gt, const PPNAPParams* params,
+                 const PPNAPMatch* out, void* stream) {
+    int rc = check_humans(humans);
+    if (rc) return rc;
+    if (!gt || !params || B < 0 || K < 1 || K > 255) return PPN_E_BADARG;
+    if ((rc = check_ap_joints(params->n_joints))) return rc;
+    if (!(params->dist_thresh > 0.0) || !(params->head_scale > 0.0)) return PPN_E_BADARG;     // NaN fails too
+    if ((rc = check_ap_match(out))) return rc;
+    if (out->R < humans->R) return PPN_E_BADARG;
+    if (bad_ptr(gt->person_off, 4) || gt->n < 0) return PPN_E_BADARG;
+    if (gt->n > 0 && (bad_ptr(gt->head_box, 8) || bad_ptr(gt->joint_xy, 8) || !gt->joint_valid)) return PPN_E_BADARG;
+    if (reinterpret_cast<uintptr_t>(humans->part_box) & 15) return PPN_E_BADARG;
+    if (B == 0) return PPN_OK;
+    ppn::APMatchArgs a;
+    a.count = humans->count; a.cell = humans->part_cell; a.box = reinterpret_cast<const float4*>(humans->part_box);
+    a.part_score = humans->part_score; a.R = humans->R; a.K = K;
+    a.person_off = gt->person_off; a.head_box = gt->head_box; a.joint_xy = gt->joint_xy; a.joint_valid = gt->joint_valid;
+    a.n_gt_rows = gt->n;
+    a.J = params->n_joints; a.thresh = params->dist_thresh; a.head_scale = params->head_scale;
+    a.score = out->score; a.label = out->label; a.used = out->used; a.flags = out->flags; a.n_gt = out->n_gt; a.R_out = out->R;
+    return cuda_rc(ppn::launch_ap_match(a, B, (cudaStream_t)stream));
+}
+
+int ppn_ap_workspace_bytes(int32_t N, int32_t R, int32_t J, size_t* bytes) {
+    if (!bytes || N < 1 || R < 1) return PPN_E_BADARG;
+    int rc = check_ap_joints(J);
+    if (rc) return rc;
+    if (!ap_fits(N, R, J)) return PPN_E_UNSUPPORTED;
+    ppn::APWorkspace w;
+    *bytes = ppn::ap_workspace_layout(N, R, J, &w);
+    return PPN_OK;
+}
+
+// evaluateAP.computeMetrics of the poseval fork over N images of match results
+int ppn_ap_finalize(const PPNAPMatch* match, int32_t N, int32_t K, int32_t J, double* ap, double* precision,
+                    double* recall, int32_t* status, void* workspace, size_t workspace_bytes, void* stream) {
+    int rc = check_ap_match(match);
+    if (rc) return rc;
+    if (N < 1 || K < 1 || K > 255) return PPN_E_BADARG;
+    if ((rc = check_ap_joints(J))) return rc;
+    if (!ap_fits(N, match->R, J)) return PPN_E_UNSUPPORTED;
+    if (bad_ptr(ap, 8) || bad_ptr(precision, 8) || bad_ptr(recall, 8) || bad_ptr(status, 4)) return PPN_E_BADARG;
+    if (bad_ptr(workspace, 256)) return PPN_E_BADARG;
+    ppn::APWorkspace w;
+    if (workspace_bytes < ppn::ap_workspace_layout(N, match->R, J, &w)) return PPN_E_WORKSPACE;
+    char* ws = static_cast<char*>(workspace);
+    ppn::APFinalizeArgs a;
+    a.score = match->score; a.label = match->label; a.used = match->used; a.flags = match->flags; a.n_gt = match->n_gt;
+    a.N = N; a.R = match->R; a.J = J; a.Jp = std::min(K - 1, J);
+    a.cap = N * match->R;
+    a.ord_bits = 1;
+    while (a.ord_bits < 31 && ((long long)a.cap - 1) >> a.ord_bits) ++a.ord_bits;
+    a.ap = ap; a.precision = precision; a.recall = recall; a.status = status;
+    a.offsets = reinterpret_cast<int32_t*>(ws + w.offsets);
+    a.seg_begin = reinterpret_cast<int32_t*>(ws + w.seg_begin);
+    a.seg_end = reinterpret_cast<int32_t*>(ws + w.seg_end);
+    a.keys = reinterpret_cast<unsigned long long*>(ws + w.keys_a);
+    return cuda_rc(ppn::launch_ap_finalize(a, reinterpret_cast<unsigned long long*>(ws + w.keys_b), ws + w.sort_temp,
+                                           (cudaStream_t)stream));
+}
+
 int ppn_debug_argmax_items(const PPNShape* shape, int32_t sms, int32_t* info, int32_t* first, int32_t* size, int32_t max_items) {
     int rc = check_shape(shape);
     if (rc) return rc;

@@ -122,6 +122,13 @@ __device__ __forceinline__ float4 box_at(const T* __restrict__ img, const Geom& 
                     ldf(img + (size_t)(4 * g.K + k) * HW + c), ldf(img + (size_t)(5 * g.K + k) * HW + c), h, w, g);
 }
 
+// centre (y, x) of a (ymin, xmin, ymax, xmax) box, y = (ymin + ymax) / 2, x = (xmin + xmax) / 2 in fp32 (an add and
+// an exact halving): the keypoint of a part (datatest.py:200-211, 314-317).  Shared by ppn_part_centres and the AP
+// matcher (ppn_eval.cu), so that the evaluator scores exactly the points the evaluation frames carry.
+__device__ __forceinline__ float2 box_centre(const float4 b) {
+    return make_float2(__fmul_rn(__fadd_rn(b.x, b.z), 0.5f), __fmul_rn(__fadd_rn(b.y, b.w), 0.5f));
+}
+
 // numpy's maximum / minimum: propagate NaN (datatest.py:145-146)
 __device__ __forceinline__ float np_max(float a, float b) { return (a >= b || a != a) ? a : b; }
 __device__ __forceinline__ float np_min(float a, float b) { return (a <= b || a != a) ? a : b; }

@@ -2129,10 +2129,7 @@ part_centres_kernel(const int32_t* __restrict__ count, const int32_t* __restrict
     const size_t human = i / K;
     const int b = (int)(human / R), slot = (int)(human - (size_t)b * R);
     float2 c = make_float2(0.0f, 0.0f);
-    if (slot < count[b] && cell[i] >= 0) {
-        const float4 bx = box[i];
-        c = make_float2(__fmul_rn(__fadd_rn(bx.x, bx.z), 0.5f), __fmul_rn(__fadd_rn(bx.y, bx.w), 0.5f));
-    }
+    if (slot < count[b] && cell[i] >= 0) c = box_centre(box[i]);
     centre[i] = c;
 }
 

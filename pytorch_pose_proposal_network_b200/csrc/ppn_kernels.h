@@ -198,4 +198,34 @@ cudaError_t launch_loss_backward(LossArgs a, int sms, cudaStream_t st, bool from
 // y[i] = sigmoid_f32(x[i]) for x of HeadDtype `dtype`, y fp32 (ppn_sigmoid)
 cudaError_t launch_sigmoid(const void* x, int dtype, float* y, size_t n, cudaStream_t st);
 
+// ---- multi-person pose AP (ppn_eval.cu): poseval's assignGTmulti per image, computeMetrics per pass ---------------
+constexpr int kAPMaxGT = 64;            // GT persons per image the match kernel holds in shared memory
+constexpr int kAPMaxJoints = 32;        // joints: one warp lane each, match masks are 32-bit
+constexpr size_t kAPSortTempBytes = 64 * 1024;   // CUB's scratch for the segmented sort on double buffers (~1 KB)
+enum : int { APFLAG_OVERFLOW = 1, APFLAG_BAD_GT = 2 };
+struct APMatchArgs {
+    const int32_t* count; const int32_t* cell; const float4* box; const float* part_score;   // PPNHumans
+    int32_t R, K;
+    const int32_t* person_off; const double* head_box; const double* joint_xy; const uint8_t* joint_valid;
+    int32_t n_gt_rows;
+    int32_t J;
+    double thresh, head_scale;
+    float* score; uint8_t* label; int32_t* used; int32_t* flags; int32_t* n_gt;      // [B, R_out, J] ... [B, J]
+    int32_t R_out;
+};
+cudaError_t launch_ap_match(const APMatchArgs& a, int B, cudaStream_t st);
+struct APWorkspace { size_t offsets, seg_begin, seg_end, keys_a, keys_b, sort_temp, total; };
+size_t ap_workspace_layout(long long N, long long R, int J, APWorkspace* w);
+struct APFinalizeArgs {
+    const float* score; const uint8_t* label; const int32_t* used; const int32_t* flags; const int32_t* n_gt;
+    int32_t N, R, J, Jp;        // Jp = min(K - 1, J): joints that have prediction entries
+    int32_t cap, ord_bits;      // cap = N * R entries per joint at most; ord_bits hold cap - 1
+    double *ap, *precision, *recall;
+    int32_t* status;            // [3]: images with count > R, images with unusable GT rows, entries per joint
+    int32_t *offsets, *seg_begin, *seg_end;
+    unsigned long long* keys;   // [J][cap]
+};
+// five launches: offsets, keys, the CUB sort (on keys / keys_b), the curve per joint, the means
+cudaError_t launch_ap_finalize(APFinalizeArgs a, unsigned long long* keys_b, void* sort_temp, cudaStream_t st);
+
 }  // namespace ppn
