@@ -171,7 +171,8 @@ struct HeadArgs {
     int32_t n_bstages;          // 16-bit path: stages of the weight ring
     int32_t bf16;               // 16-bit path: operands are bf16 (else fp16)
     int32_t dry;                // benchmarks only (tune key head.dry): the epilogue releases every accumulator unread
-    uint32_t magic_S;           // ceil(2^32 / S): exact p / S for p < 2^22 (S <= 65535 and S * E channels)
+    uint64_t magic_S;           // ceil(2^40 / S): (p * magic_S) >> 40 == p / S for every limb channel p < S * E < 2^24, since
+                                // p * (magic_S * S - 2^40) < 2^24 * S <= 2^40; S = 1 gives 2^40, the identity
     const float* bias;          // [C] or nullptr
     float* dec;                 // [B, n_dec, HW]   sigmoid of the 6K decode channels
     unsigned long long* keys;   // [B, E, HW]  running (sigmoid, ~position) maxima, zero before the kernel
@@ -280,8 +281,8 @@ __device__ __forceinline__ void head_epilogue(const HeadArgs& a, uint32_t tmem_b
                 float m = -INFINITY, bx = -INFINITY;
                 auto begin = [&](int c) {                             // uniform
                     if (c < a.n_dec) { limb = false; seg_end = min(a.n_dec, r_hi); return; }
-                    const int p = c - a.n_dec;                        // exact magic division, p < 2^22
-                    ei = (int)(((unsigned long long)(unsigned)p * a.magic_S) >> 32);
+                    const int p = c - a.n_dec;                        // exact magic division (HeadArgs::magic_S)
+                    ei = (int)__umul64hi((unsigned long long)(unsigned)p << 24, a.magic_S);   // (p * magic_S) >> 40
                     const int aw = p - ei * a.S;
                     limb = true; wbase = c - aw; seg_end = min(wbase + a.S, r_hi);
                     m = -INFINITY; bx = -INFINITY; idx = aw;
@@ -800,7 +801,7 @@ void fill_common(HeadArgs& a, const Geom& g, int Cin, const float* bias, float* 
     a.acc_n = acc_n; a.acc_stages = kTmemCols / acc_n;
     a.n_ntiles = (g.C + acc_n - 1) / acc_n;
     a.n_last = ((g.C - (a.n_ntiles - 1) * acc_n) + 15) & ~15;              // 16 .. acc_n
-    a.magic_S = g.S <= 1 ? 0u : (uint32_t)(((1ull << 32) + g.S - 1) / g.S);
+    a.magic_S = ((1ull << 40) + g.S - 1) / g.S;
     a.bias = bias; a.dec = dec; a.keys = keys; a.emit_logits = emit_logits; a.emit_head = emit_head;
     a.n_rows = g.B * g.HW; a.n_bstages = 0; a.bf16 = 0; a.dry = 0;
     a.groups_per_img = (g.HW + 31) / 32;
