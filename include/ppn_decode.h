@@ -17,6 +17,8 @@
  *                            segments, datatest.py:162-232
  *   ppn_parse .............. get_humans_by_feature end to end on a device batch: what
  *                            rt_test.py:109-133 / main.py:946-972 do per image after model(image)
+ *   ppn_parse_proposals .... not the reference's parse: per-part proposals, limb scores of candidate pairs and a
+ *                            greedy tree parse in which humans compete for parts (the paper's form, DESIGN.md §13)
  *   ppn_parse_host ......... the same from host memory (the reference's numpy arrays), with the
  *                            copies the reference's `.cpu()` calls stand for done here in reverse
  *   ppn_parse_dense ........ ppn_parse that also emits dense (human, part) records (what a multi-GPU job gathers)
@@ -194,6 +196,34 @@ int ppn_tree_parse(const void* head, const PPNShape* shape, const PPNParams* par
  * predecessor.  Results are identical to calling the four stage functions above in sequence. */
 int ppn_parse(const void* head, const PPNShape* shape, const PPNParams* params,
               const PPNHumans* out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- proposal-pair parse: humans compete for parts (DESIGN.md §13) -------------------------------------------
+ * A second parser over the same head tensor and the same PPNHumans layout.  ppn_parse follows the reference: NMS on
+ * part 0 only, then from each root the arg-max of every limb window, so several humans may hold the same part cell.
+ * This one gives every part proposals and matches them greedily down the skeleton tree.  For one image:
+ *   1. proposals: for EVERY part k, the cells with delta[k] > det_thresh (strict), through ppn_nms's greedy IoU
+ *      suppression (IoU >= nms_thresh; equal scores: larger cell first).  The survivors P_k keep NMS order;
+ *   2. human i is the i-th proposal of P_0, rooted at that cell;
+ *   3. the track orders must form a tree rooted at part 0: every target part reached by one limb from one
+ *      predecessor, part 0 never a target (PPN_E_CHAINS otherwise).  Parts are matched in first-reach order;
+ *   4. limb e = (s -> t) pairs the part-s cell a of every human that has part s with every b in P_t whose
+ *      displacement dy = row(b) - row(a) + off_h, dx = col(b) - col(a) + off_w lies in the window (0 <= dy < sH,
+ *      0 <= dx < sW).  Score sc = (delta[s, a] * lv) * delta[t, b], lv = head[6K + (e*sH + dy)*sW + dx, a], each
+ *      product rounded once; the pair is a candidate iff sc > 0 (NaN, zero and negative limb values never connect);
+ *   5. candidates in order of sc descending, then smaller human index, then smaller cell; a pair is accepted when
+ *      its human has no part t yet and b is unused;
+ *   6. humans stay in root NMS order; those with at least min_num_keypoints non-root parts are kept (after the
+ *      matching: a dropped human's parts go to no one).  part_score / part_box of a present part are those ppn_parse
+ *      computes for that cell; count[b] may exceed R, only the first R humans are stored.
+ * No part instance belongs to two humans, and every present part's parent is present.
+ * params->n_nms_parts is not read (every part is NMSed).  Among the flags only PPN_FLAG_CLEAR_UNUSED is honoured;
+ * calls are stream-ordered (no overlap with the previous call).  Needs K <= 64 and H*W <= PPN_MAX_CELLS
+ * (PPN_E_UNSUPPORTED beyond).  Two kernels: decode + NMS of every (image, part), and the pair-scoring + matching
+ * kernel as its programmatic dependent; no host synchronisation, capturable in a CUDA graph.
+ *   ppn_parse_proposals_workspace_bytes: scratch for the per-part survivor lists (256-byte aligned workspace). */
+int ppn_parse_proposals_workspace_bytes(const PPNShape* shape, const PPNParams* params, size_t* bytes);
+int ppn_parse_proposals(const void* head, const PPNShape* shape, const PPNParams* params, const PPNHumans* out,
+                        void* workspace, size_t workspace_bytes, void* stream);
 
 /* The whole path from HOST memory (pinned for full speed): uploads `head` in chunks
  * overlapped with the kernels, runs ppn_parse, downloads the packed result into the HOST

@@ -19,6 +19,7 @@ FLAG_CLEAR_UNUSED = 2
 MAX_CELLS = 1024
 MAX_CHAINS = 32
 MAX_CHAIN_STEPS = 192
+PROPOSAL_MAX_PARTS = 64
 IPC_HANDLE_BYTES = 64
 
 i32p = C.POINTER(C.c_int32)
@@ -99,6 +100,9 @@ EXPORTS = {
                                  C.c_void_p, C.c_void_p, C.POINTER(PPNHumans), C.c_void_p]),
     "ppn_parse": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNParams), C.POINTER(PPNHumans),
                             C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ppn_parse_proposals_workspace_bytes": (C.c_int, [C.POINTER(PPNShape), C.POINTER(PPNParams), C.POINTER(C.c_size_t)]),
+    "ppn_parse_proposals": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNParams), C.POINTER(PPNHumans),
+                                      C.c_void_p, C.c_size_t, C.c_void_p]),
     "ppn_parse_host_scratch_bytes": (C.c_int, [C.POINTER(PPNShape), C.POINTER(PPNParams), C.c_int32,
                                                C.POINTER(C.c_size_t)]),
     "ppn_parse_host": (C.c_int, [C.c_void_p, C.POINTER(PPNShape), C.POINTER(PPNParams), C.POINTER(PPNHumans),

@@ -483,6 +483,88 @@ int ppn_parse_dense(const void* head, const PPNShape* shape, const PPNParams* pa
     return parse_impl(head, shape, params, out, workspace, workspace_bytes, stream, &d);
 }
 
+// ---- proposal-pair parse ----------------------------------------------------------------------
+namespace {
+// Workspace of ppn_parse_proposals: the surviving cells of every (image, part) [B, K, H*W] and their counts [B, K]
+struct ProposalWorkspace { size_t keep_cell, keep_count, total; };
+ProposalWorkspace carve_proposals(const PPNShape* s) {
+    ProposalWorkspace w;
+    const size_t lists = (size_t)s->B * s->K;
+    w.keep_cell = 0;
+    w.keep_count = align_up(lists * s->H * s->W * sizeof(int32_t), 256);
+    w.total = w.keep_count + align_up(lists * sizeof(int32_t), 256);
+    return w;
+}
+
+// The checks every proposal entry shares; fills the limb tree in first-reach order
+int check_proposals(const PPNShape* shape, const PPNParams* params, ppn::LimbTree* tree) {
+    int rc = check_shape(shape);
+    if (rc) return rc;
+    if (!params) return PPN_E_BADARG;
+    ppn::ChainTable ch;
+    if ((rc = make_chains(shape, params, &ch))) return rc;
+    if (!ch.parallel_ok) return PPN_E_CHAINS;                            // not a tree rooted at part 0
+    if (shape->K > ppn::kProposalMaxParts || (long long)shape->H * shape->W > PPN_MAX_CELLS) return PPN_E_UNSUPPORTED;
+    bool seen[256] = {};
+    tree->n = 0;
+    for (int c = 0; c < ch.n_chains; ++c)
+        for (int q = ch.off[c]; q < ch.off[c + 1]; ++q) {
+            const int t = ch.part[q];
+            if (seen[t]) continue;
+            seen[t] = true;
+            tree->limb[tree->n] = ch.limb[q];
+            tree->src[tree->n] = q == ch.off[c] ? 0 : ch.part[q - 1];
+            tree->dst[tree->n] = (uint8_t)t;
+            ++tree->n;
+        }
+    return PPN_OK;
+}
+}  // namespace
+
+int ppn_parse_proposals_workspace_bytes(const PPNShape* shape, const PPNParams* params, size_t* bytes) {
+    ppn::LimbTree tree;
+    const int rc = check_proposals(shape, params, &tree);
+    if (rc) return rc;
+    if (!bytes) return PPN_E_BADARG;
+    *bytes = carve_proposals(shape).total;
+    return PPN_OK;
+}
+
+int ppn_parse_proposals(const void* head, const PPNShape* shape, const PPNParams* params, const PPNHumans* out,
+                        void* workspace, size_t workspace_bytes, void* stream) {
+    ppn::LimbTree tree;
+    int rc = check_proposals(shape, params, &tree);
+    if (rc) return rc;
+    if ((rc = check_humans(out))) return rc;
+    if (shape->B == 0) return PPN_OK;
+    if (!head || !workspace) return PPN_E_BADARG;
+    if (misaligned(head, shape) || (reinterpret_cast<uintptr_t>(workspace) & 255)) return PPN_E_BADARG;
+    if (reinterpret_cast<uintptr_t>(out->part_box) & 15) return PPN_E_BADARG;
+    const ProposalWorkspace w = carve_proposals(shape);
+    if (workspace_bytes < w.total) return PPN_E_WORKSPACE;
+    int32_t* keep_cell = reinterpret_cast<int32_t*>(static_cast<unsigned char*>(workspace) + w.keep_cell);
+    int32_t* keep_count = reinterpret_cast<int32_t*>(static_cast<unsigned char*>(workspace) + w.keep_count);
+    const ppn::Geom g = make_geom(shape);
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e;
+    if (params->flags & PPN_FLAG_CLEAR_UNUSED) {
+        const size_t slots = (size_t)shape->B * out->R, SK = slots * shape->K;
+        if ((e = cudaMemsetAsync(out->root_cell, 0xFF, slots * sizeof(int32_t), st)) != cudaSuccess) return (int)e;
+        if ((e = cudaMemsetAsync(out->part_cell, 0xFF, SK * sizeof(int32_t), st)) != cudaSuccess) return (int)e;
+        if ((e = cudaMemsetAsync(out->part_score, 0, SK * sizeof(float), st)) != cudaSuccess) return (int)e;
+        if ((e = cudaMemsetAsync(out->part_box, 0, SK * 4 * sizeof(float), st)) != cudaSuccess) return (int)e;
+    }
+    // Stage 1: decode + NMS of every part, fully ordered behind what precedes it on the stream; it releases stage 2
+    // at once, whose CTAs become resident beside it and wait for its lists
+    if ((e = ppn::launch_decode_nms(head, g, shape->K, params->det_thresh, params->nms_thresh, keep_cell, keep_count, st,
+                                    false, ppn::PDL_TRIGGER, 2)) != cudaSuccess) return (int)e;
+    if ((e = ppn::launch_proposal_pairs(head, g, tree, params->min_num_keypoints, keep_cell, keep_count, out->count,
+                                        out->root_cell, out->part_cell, out->part_score, out->part_box, out->R, st)) != cudaSuccess)
+        return (int)e;
+    ppn::chain_break(st);                         // an overlapped ppn_parse after this call starts fully ordered
+    return PPN_OK;
+}
+
 int ppn_parse_dense_remote(const void* head, const PPNShape* shape, const PPNParams* params, const PPNHumans* out,
                            void* local_header, size_t local_header_bytes, void* remote_packed, size_t remote_bytes,
                            int32_t cap_entries, int32_t skip_slots, void* workspace, size_t workspace_bytes, void* stream) {

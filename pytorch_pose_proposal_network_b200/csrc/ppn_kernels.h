@@ -133,6 +133,17 @@ unsigned next_call_parity(cudaStream_t st);   // which workspace half the next w
 bool chain_clean(cudaStream_t st);      // the stream's last whole-path launch was a (publishing) fused parse
 void chain_break(cudaStream_t st);      // ... was something else: the next overlapped call starts fully ordered
 
+// ---- proposal-pair parse (ppn_proposals.cu): limb scores of candidate pairs + greedy tree matching --------------
+constexpr int kProposalMaxParts = 64;   // K: the humans' part cells are int16 [H*W][K] in shared memory
+// The non-root parts in first-reach order over the track orders: part dst[q] is reached from src[q] by limb limb[q]
+struct LimbTree { int32_t n; uint8_t limb[kProposalMaxParts], src[kProposalMaxParts], dst[kProposalMaxParts]; };
+size_t proposal_pairs_smem_bytes(const Geom& g);
+// One CTA per image, launched as a programmatic dependent of launch_decode_nms(n_parts = K), whose surviving cells
+// [B, K, H*W] and counts [B, K] it reads; writes the PPNHumans arrays (slots [0, min(count, R)))
+cudaError_t launch_proposal_pairs(const void* head, const Geom& g, const LimbTree& tree, int min_kp,
+                                  const int32_t* keep_cell, const int32_t* keep_count, int32_t* h_count, int32_t* h_root,
+                                  int32_t* h_cell, float* h_score, float* h_box, int R, cudaStream_t st);
+
 // ---- fused network head (ppn_head.cu): 1x1 convolution (tcgen05 GEMM) + sigmoid + limb-window arg-max ---------
 // feat [B, Cin, H, W] fp32, weight [C, Cin] fp32, bias [C] or nullptr  ->  dec [B, 6K, HW] = sigmoid of the decode
 // channels, amax [B, E, HW]; optional emit_logits / emit_head [B, C, HW] for parity tests (model.py:85, 133-136).

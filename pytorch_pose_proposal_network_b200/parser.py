@@ -310,6 +310,35 @@ class PoseParser:
             raise _lib.PPNError(rc, "ppn_parse" if dense is None else ("ppn_parse_dense" if remote is None else "ppn_parse_dense_remote"))
         return out
 
+    def parse_proposals(self, head: torch.Tensor, out: Optional[PackedHumans] = None,
+                        clear_unused: bool = False) -> PackedHumans:
+        """The proposal-pair parse of a device batch (``ppn_parse_proposals``; asynchronous, on torch's current stream).
+
+        Unlike :meth:`parse`, which walks the arg-max of every limb window from each root as the reference does, this
+        parser gives every part NMS-filtered proposals, scores each candidate pair of a limb as
+        ``(delta_s * limb) * delta_t`` and matches them greedily down the skeleton tree, so no part instance belongs
+        to two humans (DESIGN.md §13).  The result has the layout of :meth:`parse`'s and feeds the same consumers
+        (``to_lists``, ``part_centres``, ``skeleton``, ``evaluation.APEvaluator``).  The track orders must form a tree
+        rooted at part 0.  ``out`` and ``clear_unused`` as for :meth:`parse`."""
+        B = self._check_head(head)
+        if head.device != self.device:
+            raise ValueError(f"head is on {head.device}, parser on {self.device}")
+        if out is None:
+            out = self.alloc_output(B)
+        shape = self._shape(B, self._DTYPES[head.dtype])
+        params = self.c.params_for(_CConfig.flags(clear_unused=clear_unused))
+        need = C.c_size_t()
+        _lib.check(self.lib.ppn_parse_proposals_workspace_bytes(C.byref(shape), C.byref(params), C.byref(need)),
+                   "ppn_parse_proposals_workspace_bytes")
+        if getattr(self, "_prop_ws", None) is None or self._prop_ws.numel() < need.value:
+            self._prop_ws = torch.empty(max(need.value, 256), dtype=torch.uint8, device=self.device)
+        hs = self._humans_struct(out)
+        with self._guard():
+            _lib.check(self.lib.ppn_parse_proposals(head.data_ptr(), C.byref(shape), C.byref(params), C.byref(hs),
+                                                    self._prop_ws.data_ptr(), self._prop_ws.numel(),
+                                                    torch.cuda.current_stream(self.device).cuda_stream), "ppn_parse_proposals")
+        return out
+
     def capture(self, head: torch.Tensor, out: Optional[PackedHumans] = None, **parse_kwargs) -> "CapturedParse":
         """Record ``parse(head, out)`` into a CUDA graph for repeated use on the SAME buffers — the single-image
         loop of rt_test.py:87-147, where the network writes its output into one tensor frame after frame: a replay
