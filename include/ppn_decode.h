@@ -521,6 +521,67 @@ int ppn_ap_workspace_bytes(int32_t N, int32_t R, int32_t J, size_t* bytes);
 int ppn_ap_finalize(const PPNAPMatch* match, int32_t N, int32_t K, int32_t J, double* ap, double* precision,
                     double* recall, int32_t* status, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- batch augmentation: warp, flip and normalise a ragged uint8 batch, and move its annotations -----------------
+ * Stands in for the reference's per-image transform (aug.py: affine / crop / resize of the image, keypoints and boxes,
+ * then ToNormalizedTensor).  The rule is DESIGN.md §14; exactness starts at the parameters.  Per image, a forward
+ * affine A (2x3 fp64, source pixel coordinates -> output coordinates, pixel (row i, col j) centred at (j + .5, i + .5)),
+ * M = A^-1 rounded to fp32, and a flip flag (A already mirrors; the flag swaps left_* and right_* part columns).
+ *
+ * ppn_augment_images: output pixel (u, v), channel c, fp32 with one rounding per operation:
+ *   sx = ((m00 (u + .5) + m01 (v + .5)) + m02) - .5, sy likewise; x0 = floor(sx), ax = sx - x0, the same in y;
+ *   val = (p00 (1 - ax) + p01 ax) (1 - ay) + (p10 (1 - ax) + p11 ax) ay,   p01 the tap at (x0 + 1, y0), ...
+ *   out = (val * in_scale - mean[c]) / std[c]   (IEEE division), rounded once to the output dtype.
+ * A tap outside the source reads fill[c]; a pixel whose four taps are all outside, or whose sx or sy is non-finite or
+ * beyond +-2^30, takes val = fill[c].  One launch for the batch, any mix of sizes, no host synchronisation.
+ * `pixels` is read in aligned 16-byte words that hold at least one byte of an image, so it must be readable up to the
+ * next 16-byte boundary after its last image byte.  out: [B, 3, out_h, out_w] (PPN_LAYOUT_NCHW) or [B, out_h, out_w, 3]
+ * (PPN_LAYOUT_NHWC, a channels_last tensor's memory) of out_dtype (PPN_HEAD_*), out_bytes exactly its size, aligned
+ * to its element.  PPN_E_BADARG: a NULL pointer, B < 1, an image with h or w outside [1, 65535] or outside `bytes`,
+ * an output size outside [1, 65535] or not matching out_bytes, an unknown dtype or layout, std[c] <= 0 (or NaN). */
+typedef struct PPNImageBatch {
+    const uint8_t* pixels;      /* DEVICE: every image, HWC RGB uint8, image b at byte offset[b] (any alignment)      */
+    const int64_t* offset;      /* DEVICE [B]                                                                      */
+    const int32_t* hw;          /* DEVICE [B][2] (h, w)                                                             */
+    const int64_t* offset_host; /* HOST copies of offset and hw with the same values: the checks read these, the      */
+    const int32_t* hw_host;     /*   kernel the device arrays                                                       */
+    size_t         bytes;       /* size of `pixels`                                                                 */
+    int32_t        B;
+} PPNImageBatch;
+
+typedef struct PPNImageNorm {
+    float mean[3];              /* per channel, in units of val * in_scale (ImageNet: 0.485, 0.456, 0.406)         */
+    float std[3];               /* > 0 (ImageNet: 0.229, 0.224, 0.225)                                              */
+    float fill[3];              /* pixel value of taps outside the source, in uint8 units (0)                       */
+    float in_scale;             /* fl32(1 / 255); 1 reproduces rt_test.py's 0-1 statistics on 0-255 pixels          */
+} PPNImageNorm;
+
+#define PPN_LAYOUT_NCHW 0
+#define PPN_LAYOUT_NHWC 1
+
+int ppn_augment_images(const PPNImageBatch* in, const float* M /* DEVICE [B][2][3] */, const PPNImageNorm* norm,
+                       int32_t out_h, int32_t out_w, int32_t out_dtype, int32_t out_layout, void* out, size_t out_bytes,
+                       void* stream);
+
+/* ppn_augment_people: the annotations of B images (the PPNPeople layout ppn_encode_targets reads; n people, K - 1
+ * parts each) through each image's A, in fp64 with one rounding per operation, written to `out` (person_off is
+ * unchanged and not written):
+ *   keypoints: (a00 x + a01 y) + a02, (a10 x + a11 y) + a12 rounded once to fp32; on a flipped image column i of
+ *              keypoints and visible takes column perm[i] (perm: HOST [K - 1], a permutation);
+ *   visible:   never changed otherwise (points that leave the output stay visible; the encoder's bounds drop them);
+ *   bbox:      w > 0 and h > 0: the bounds of the four transformed corners (cx -+ w / 2, cy -+ h / 2), as
+ *              ((min + max) / 2, max - min); otherwise the transformed centre with w = h = 0 (part 0 stays unlabelled);
+ *   size:      size * sqrt(|a00 a11 - a01 a10|).
+ * DEVICE pointers except perm.  PPN_E_BADARG: a NULL pointer, B < 1, n < 0, K outside [1, 256], perm not a
+ * permutation of [0, K - 1).  n = 0 is a no-op.  The rows of `in` are only read, so out may not alias them. */
+typedef struct PPNPeopleOut {
+    double*  bbox;              /* [n, 4]                                                           */
+    float*   keypoints;         /* [n, K - 1, 2]                                                    */
+    uint8_t* visible;           /* [n, K - 1]                                                       */
+    double*  size;              /* [n]                                                              */
+} PPNPeopleOut;
+int ppn_augment_people(const PPNPeople* in, int32_t B, int32_t n, int32_t K, const double* A /* DEVICE [B][2][3] */,
+                       const uint8_t* flip /* DEVICE [B] */, const int32_t* perm, const PPNPeopleOut* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -81,6 +81,22 @@ AP_MAX_JOINTS = 32
 AP_MAX_GT = 64
 
 
+class PPNImageBatch(C.Structure):
+    _fields_ = [("pixels", C.c_void_p), ("offset", C.c_void_p), ("hw", C.c_void_p), ("offset_host", C.c_void_p),
+                ("hw_host", C.c_void_p), ("bytes", C.c_size_t), ("B", C.c_int32)]
+
+
+class PPNImageNorm(C.Structure):
+    _fields_ = [("mean", C.c_float * 3), ("std", C.c_float * 3), ("fill", C.c_float * 3), ("in_scale", C.c_float)]
+
+
+class PPNPeopleOut(C.Structure):
+    _fields_ = [("bbox", C.c_void_p), ("keypoints", C.c_void_p), ("visible", C.c_void_p), ("size", C.c_void_p)]
+
+
+LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
+
+
 # name -> (restype, argtypes); must list every function of include/ppn_decode.h
 EXPORTS = {
     "ppn_abi_version": (C.c_int, []),
@@ -157,6 +173,10 @@ EXPORTS = {
     "ppn_ap_workspace_bytes": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_size_t)]),
     "ppn_ap_finalize": (C.c_int, [C.POINTER(PPNAPMatch), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ppn_augment_images": (C.c_int, [C.POINTER(PPNImageBatch), C.c_void_p, C.POINTER(PPNImageNorm), C.c_int32, C.c_int32,
+                                     C.c_int32, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ppn_augment_people": (C.c_int, [C.POINTER(PPNPeople), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, i32p,
+                                     C.POINTER(PPNPeopleOut), C.c_void_p]),
     "ppn_debug_argmax_items": (C.c_int, [C.POINTER(PPNShape), C.c_int32, i32p, i32p, i32p, C.c_int32]),
     "ppn_timeline": (C.c_int, [C.c_void_p, C.c_int32]),
     "ppn_profile_enable": (C.c_int, [C.c_int32]),

@@ -252,6 +252,7 @@ int ppn_tune(const char* key, int32_t value) {
     else if (!std::strcmp(key, "host.chunk_images")) t.host_chunk_images = value < 1 ? 1 : value;
     else if (!std::strcmp(key, "encode.sweep")) t.encode_sweep = value != 0;
     else if (!std::strcmp(key, "encode.ctas_per_sm")) t.encode_ctas_per_sm = value < 1 ? 1 : (value > 8 ? 8 : value);
+    else if (!std::strcmp(key, "augment.stage_bytes")) t.augment_stage_bytes = value < 0 ? 0 : (value > 48 * 1024 ? 48 * 1024 : value);
     else if (!std::strcmp(key, "nms.blockwise")) ppn::set_nms_blockwise(value);   // NMS phase 3 block by block (round 1/2) instead of the warp wavefront
     else if (!std::strcmp(key, "timeline.phase")) g_timeline.phase = value;      // which in-kernel phase boundary ppn_timeline records
     else return PPN_E_BADARG;
@@ -284,6 +285,7 @@ int ppn_tune_get(const char* key, int32_t* value) {
     else if (!std::strcmp(key, "host.chunk_images")) *value = t.host_chunk_images;
     else if (!std::strcmp(key, "encode.sweep")) *value = t.encode_sweep;
     else if (!std::strcmp(key, "encode.ctas_per_sm")) *value = t.encode_ctas_per_sm;
+    else if (!std::strcmp(key, "augment.stage_bytes")) *value = t.augment_stage_bytes;
     else if (!std::strcmp(key, "nms.blockwise")) *value = ppn::get_nms_blockwise();
     else return PPN_E_BADARG;
     return PPN_OK;
@@ -1311,6 +1313,59 @@ int ppn_ap_finalize(const PPNAPMatch* match, int32_t N, int32_t K, int32_t J, do
     a.keys = reinterpret_cast<unsigned long long*>(ws + w.keys_a);
     return cuda_rc(ppn::launch_ap_finalize(a, reinterpret_cast<unsigned long long*>(ws + w.keys_b), ws + w.sort_temp,
                                            (cudaStream_t)stream));
+}
+
+// ---- batch augmentation (the reference's aug.py transform, DESIGN.md §14) ------------------------------------------
+int ppn_augment_images(const PPNImageBatch* in, const float* M, const PPNImageNorm* norm, int32_t out_h, int32_t out_w,
+                       int32_t out_dtype, int32_t out_layout, void* out, size_t out_bytes, void* stream) {
+    const ppn::Tuning g_tuning = tuning_now();
+    if (!in || !norm || !in->pixels || bad_ptr(in->offset, 8) || bad_ptr(in->hw, 4) || !in->offset_host || !in->hw_host)
+        return PPN_E_BADARG;
+    if (bad_f32(M) || in->B < 1) return PPN_E_BADARG;
+    if (out_dtype < PPN_HEAD_F32 || out_dtype > PPN_HEAD_BF16) return PPN_E_BADARG;
+    if (out_layout != PPN_LAYOUT_NCHW && out_layout != PPN_LAYOUT_NHWC) return PPN_E_BADARG;
+    if (out_h < 1 || out_h > 65535 || out_w < 1 || out_w > 65535) return PPN_E_BADARG;
+    for (int c = 0; c < 3; ++c)
+        if (!(norm->std[c] > 0.0f)) return PPN_E_BADARG;                          // NaN fails too
+    for (int32_t b = 0; b < in->B; ++b) {
+        const long long h = in->hw_host[2 * b], w = in->hw_host[2 * b + 1], off = in->offset_host[b];
+        if (h < 1 || h > 65535 || w < 1 || w > 65535) return PPN_E_BADARG;
+        if (off < 0 || (unsigned long long)off + 3ull * h * w > in->bytes) return PPN_E_BADARG;
+    }
+    const size_t elem = dtype_bytes(out_dtype);
+    if (bad_ptr(out, elem) || out_bytes != (size_t)in->B * 3 * out_h * out_w * elem) return PPN_E_BADARG;
+    ppn::AugmentArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.pixels = in->pixels; a.offset = in->offset; a.hw = in->hw; a.M = M;
+    for (int c = 0; c < 3; ++c) { a.mean[c] = norm->mean[c]; a.std[c] = norm->std[c]; a.fill[c] = norm->fill[c]; }
+    a.in_scale = norm->in_scale;
+    a.out = out; a.B = in->B; a.outH = out_h; a.outW = out_w;
+    a.vec = (reinterpret_cast<uintptr_t>(out) & 15) == 0 && ((size_t)out_w * elem) % 16 == 0;
+    a.stage_bytes = g_tuning.augment_stage_bytes;
+    return cuda_rc(ppn::launch_augment_images(a, out_dtype, out_layout == PPN_LAYOUT_NHWC, (cudaStream_t)stream));
+}
+
+int ppn_augment_people(const PPNPeople* in, int32_t B, int32_t n, int32_t K, const double* A, const uint8_t* flip,
+                       const int32_t* perm, const PPNPeopleOut* out, void* stream) {
+    if (!in || !out || !perm || B < 1 || n < 0 || K < 1 || K > 256) return PPN_E_BADARG;
+    if (bad_ptr(in->person_off, 4) || bad_ptr(A, 8) || !flip) return PPN_E_BADARG;
+    ppn::AugmentPeopleArgs a;
+    std::memset(&a, 0, sizeof(a));
+    const int J = K - 1;
+    bool seen[256] = {};
+    for (int i = 0; i < J; ++i) {
+        if (perm[i] < 0 || perm[i] >= J || seen[perm[i]]) return PPN_E_BADARG;
+        seen[perm[i]] = true;
+        a.perm[i] = (uint8_t)perm[i];
+    }
+    if (bad_ptr(in->bbox, 8) || bad_ptr(in->size, 8) || bad_ptr(out->bbox, 8) || bad_ptr(out->size, 8)) return PPN_E_BADARG;
+    if (J > 0 && (bad_f32(in->keypoints) || !in->visible || bad_f32(out->keypoints) || !out->visible)) return PPN_E_BADARG;
+    if (n == 0) return PPN_OK;
+    a.person_off = in->person_off; a.bbox = in->bbox; a.keypoints = in->keypoints; a.visible = in->visible; a.size = in->size;
+    a.A = A; a.flip = flip;
+    a.bbox_out = out->bbox; a.keypoints_out = out->keypoints; a.visible_out = out->visible; a.size_out = out->size;
+    a.B = B; a.n = n; a.J = J;
+    return cuda_rc(ppn::launch_augment_people(a, (cudaStream_t)stream));
 }
 
 int ppn_debug_argmax_items(const PPNShape* shape, int32_t sms, int32_t* info, int32_t* first, int32_t* size, int32_t max_items) {

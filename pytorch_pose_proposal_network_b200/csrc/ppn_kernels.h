@@ -38,6 +38,9 @@ struct Tuning {
     int host_chunk_images = 64;
     int encode_sweep = 1;              // target encoder: limb tensors by the address-ordered persistent sweep (0: one CTA per image part)
     int encode_ctas_per_sm = 6;
+    int augment_stage_bytes = 0;       // augmentation: shared memory per CTA for a tile's staged source footprint, at most 48 KB;
+                                       // 0: every tap gathered through L1.  Staging measured slower on every workload of
+                                       // profiles/bench_augment.txt (the reservation takes L1 from the gathers)
     int argmax_dry = 0;                // ring kernels only move the bytes (no compares, no stores): the read ceiling of this ring
     int head_subs = 0;                 // fused head: epilogue warps per TMEM lane quadrant (1, 2, 4 or 6; 0 = auto: 4 for TF32 operands, 6 for
                                        // 16-bit ones, where the faster MMAs leave the latency-bound epilogue warps more to hide; bits 8-9:
@@ -238,5 +241,28 @@ struct APFinalizeArgs {
 };
 // five launches: offsets, keys, the CUB sort (on keys / keys_b), the curve per joint, the means
 cudaError_t launch_ap_finalize(APFinalizeArgs a, unsigned long long* keys_b, void* sort_temp, cudaStream_t st);
+
+// ---- batch augmentation (ppn_augment.cu): warp + normalise a ragged uint8 batch, move its annotations ------------
+struct AugmentArgs {
+    const uint8_t* pixels;              // every image, HWC RGB uint8; image b at byte offset[b]
+    const int64_t* offset;              // [B]
+    const int32_t* hw;                  // [B][2] (h, w)
+    const float* M;                     // [B][2][3] output pixel centre -> source coordinates
+    float mean[3], std[3], fill[3], in_scale;
+    void* out;                          // [B, 3, outH, outW] (NCHW) or [B, outH, outW, 3] (NHWC) of the output dtype
+    int32_t B, outH, outW;
+    int32_t vec;                        // out is 16-byte aligned and every output row starts on a 16-byte boundary
+    int32_t stage_bytes;                // shared memory per CTA for the staged source footprint (0: always gather)
+};
+cudaError_t launch_augment_images(const AugmentArgs& a, int out_dtype /* HeadDtype */, bool nhwc, cudaStream_t st);
+struct AugmentPeopleArgs {
+    const int32_t* person_off; const double* bbox; const float* keypoints; const uint8_t* visible; const double* size;
+    const double* A;                    // [B][2][3] source -> output coordinates
+    const uint8_t* flip;                // [B]
+    double* bbox_out; float* keypoints_out; uint8_t* visible_out; double* size_out;
+    int32_t B, n, J;                    // images, people, parts per person (K - 1)
+    uint8_t perm[256];                  // flipped image: column i takes column perm[i]
+};
+cudaError_t launch_augment_people(const AugmentPeopleArgs& a, cudaStream_t st);
 
 }  // namespace ppn

@@ -16,8 +16,6 @@ tensors; checked bit for bit against outputs of the reference's own ``__getitem_
 For mixed-precision training, ``TargetEncoder(cfg, limb_dtype=torch.float16)`` (or bfloat16) writes the two limb
 tensors — most of the bytes — in 16 bits: te in {0, 1} is exact, weight_ij stores 0.0005 rounded to the type
 (fp16 0.000500202..., bf16 0.000499725...).  The eight [B, K, H, W] grids stay fp32.
-
-Image loading and augmentation (aug.py) stay where they are: they are not on this path.
 """
 from __future__ import annotations
 
