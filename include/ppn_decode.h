@@ -34,6 +34,7 @@
  *   ppn_sigmoid ............ that sigmoid alone, elementwise (model.py:136 with the loss's exact values)
  *   ppn_ap_match ........... the validation pass's scoring, per image: poseval's eval_helpers.assignGTmulti
  *   ppn_ap_finalize ........ ... and over the pass: evaluateAP.computeMetrics (computeRPC, VOCap)
+ *   ppn_flip_merge ......... the flip test: a head averaged with the mirrored head of its flipped input (§15)
  *
  * Conventions
  *   - plain C: pointers and sizes only; no CUDA or torch types.  `stream` is a cudaStream_t
@@ -581,6 +582,27 @@ typedef struct PPNPeopleOut {
 } PPNPeopleOut;
 int ppn_augment_people(const PPNPeople* in, int32_t B, int32_t n, int32_t K, const double* A /* DEVICE [B][2][3] */,
                        const uint8_t* flip /* DEVICE [B] */, const int32_t* perm, const PPNPeopleOut* out, void* stream);
+
+/* ---- the flip test: merge a head with the mirrored head of its horizontally flipped input -------------------------
+ * The standard test-time step of a bottom-up pose estimator; the reference has none, so the rule is DESIGN.md §15.
+ * head is the network's head on an input x, head_flipped its head on x.flip(-1) (the exact pixel mirror), both
+ * [B, C, H, W] of shape->head_dtype.  For every element, with p = part_mirror, q = limb_mirror:
+ *   source plane   part group g (resp, conf, x, y, w, h), part k: g * K + p[k];
+ *                  limb plane (e, a, b) of the [E, sH, sW] block: (q[e], a, sW - 1 - b)
+ *   source cell    (i, j) reads head_flipped at (i, W - 1 - j)
+ *   value          widened exactly, then fp32 with one rounding per operation, no FMA: b' = 1 - b in the x group
+ *                  (b otherwise), out = (a + b') * 0.5, rounded once (to nearest even) to the head's dtype.
+ * part_mirror (HOST [K]) maps each part to its mirror part (left_* <-> right_*, part 0 to itself); limb_mirror
+ * (HOST [E]) each limb (s, t) to the limb (p[s], p[t]).  Both travel in the kernel parameters: one launch, no
+ * copies, no host synchronisation, capturable in a CUDA graph.  out may be head (in place: the first half of a
+ * [2B] output); it must not overlap head_flipped, nor overlap head without being it.
+ * PPN_E_BADARG: a NULL pointer, B < 1, an unknown head_dtype, a pointer not aligned to the element size, part_mirror
+ * or limb_mirror not a self-inverse permutation or part_mirror[0] != 0, out overlapping head_flipped (or part of head).
+ * PPN_E_UNSUPPORTED: inW != W * gridW (the cell mirror is not exact), 2 * off_w != sW - 1 (nor the window mirror),
+ * K > 64, H * W > PPN_MAX_CELLS. */
+int ppn_flip_merge(const void* head, const void* head_flipped, void* out, const PPNShape* shape,
+                   const int32_t* part_mirror /* host [K] */, const int32_t* limb_mirror /* host [E] */,
+                   void* stream);
 
 #ifdef __cplusplus
 }

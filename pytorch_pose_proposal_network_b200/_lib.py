@@ -177,6 +177,7 @@ EXPORTS = {
                                      C.c_int32, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
     "ppn_augment_people": (C.c_int, [C.POINTER(PPNPeople), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, i32p,
                                      C.POINTER(PPNPeopleOut), C.c_void_p]),
+    "ppn_flip_merge": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(PPNShape), i32p, i32p, C.c_void_p]),
     "ppn_debug_argmax_items": (C.c_int, [C.POINTER(PPNShape), C.c_int32, i32p, i32p, i32p, C.c_int32]),
     "ppn_timeline": (C.c_int, [C.c_void_p, C.c_int32]),
     "ppn_profile_enable": (C.c_int, [C.c_int32]),

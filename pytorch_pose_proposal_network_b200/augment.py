@@ -25,7 +25,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .config import KEYPOINT_NAMES, KEYPOINT_NAMES_16, PPNConfig
+from .config import PPNConfig, default_skeleton
 
 IMAGENET_MEAN = (0.485, 0.456, 0.406)
 IMAGENET_STD = (0.229, 0.224, 0.225)
@@ -175,10 +175,7 @@ class Augmenter:
                  channels_last=False, device=None):
         if dtype not in OUT_DTYPES:
             raise ValueError(f"dtype must be torch.float32, float16 or bfloat16, got {dtype}")
-        if keypoint_names is None:
-            keypoint_names = {len(KEYPOINT_NAMES): KEYPOINT_NAMES, len(KEYPOINT_NAMES_16): KEYPOINT_NAMES_16}.get(cfg.K)
-            if keypoint_names is None:
-                raise ValueError("pass `keypoint_names` (K part names) for a skeleton that is not one of config.py's")
+        keypoint_names, _ = default_skeleton(cfg, keypoint_names, need=("names",))
         if len(keypoint_names) != cfg.K:
             raise ValueError(f"{len(keypoint_names)} keypoint names for a configuration with K = {cfg.K}")
         lo, hi = (float(v) for v in scale)

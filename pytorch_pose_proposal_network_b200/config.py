@@ -105,6 +105,22 @@ TRACK_ORDERS_16 = [
 DIRECTED_GRAPHS_16 = directed_graphs(TRACK_ORDERS_16, EDGES_BY_NAME_16, KEYPOINT_NAMES_16)
 
 
+def default_skeleton(cfg, keypoint_names=None, edges=None, need=("names", "edges")):
+    """(keypoint_names, edges) of `cfg`'s skeleton, each given one passed through and a missing one of those `need`
+    names taken from config.py's two skeletons: the part names by K, the edges by (K, E).  ValueError where K (or
+    (K, E)) matches neither."""
+    if keypoint_names is None and "names" in need:
+        keypoint_names = {len(KEYPOINT_NAMES): KEYPOINT_NAMES, len(KEYPOINT_NAMES_16): KEYPOINT_NAMES_16}.get(cfg.K)
+        if keypoint_names is None:
+            raise ValueError("pass `keypoint_names` (K part names) for a skeleton that is not one of config.py's")
+    if edges is None and "edges" in need:
+        edges = {(len(KEYPOINT_NAMES), len(EDGES)): EDGES, (len(KEYPOINT_NAMES_16), len(EDGES_16)): EDGES_16}.get(
+            (cfg.K, cfg.E))
+        if edges is None:
+            raise ValueError("pass `edges` ([E][2] part ids) for a skeleton that is not one of config.py's")
+    return keypoint_names, edges
+
+
 def _freeze_graphs(graphs) -> Tuple[Tuple[Tuple[int, ...], Tuple[int, ...]], ...]:
     return tuple((tuple(int(v) for v in eis), tuple(int(v) for v in ts)) for eis, ts in graphs)
 

@@ -143,6 +143,7 @@ int make_chains(const PPNShape* s, const PPNParams* p, ppn::ChainTable* ch) {
 
 inline size_t elem_bytes(const PPNShape* s) { return s->head_dtype == PPN_HEAD_F32 ? 4 : 2; }
 inline bool misaligned(const void* p, const PPNShape* s) { return (reinterpret_cast<uintptr_t>(p) & (elem_bytes(s) - 1)) != 0; }
+inline bool misaligned_or_null(const void* p, const PPNShape* s) { return !p || misaligned(p, s); }
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -1366,6 +1367,41 @@ int ppn_augment_people(const PPNPeople* in, int32_t B, int32_t n, int32_t K, con
     a.bbox_out = out->bbox; a.keypoints_out = out->keypoints; a.visible_out = out->visible; a.size_out = out->size;
     a.B = B; a.n = n; a.J = J;
     return cuda_rc(ppn::launch_augment_people(a, (cudaStream_t)stream));
+}
+
+// ---- the flip test's merge (DESIGN.md §15) ----------------------------------------------------------------------
+int ppn_flip_merge(const void* head, const void* head_flipped, void* out, const PPNShape* shape,
+                   const int32_t* part_mirror, const int32_t* limb_mirror, void* stream) {
+    int rc = check_shape(shape);
+    if (rc) return rc;
+    if (shape->B < 1 || !part_mirror || (shape->E > 0 && !limb_mirror)) return PPN_E_BADARG;
+    if (misaligned_or_null(head, shape) || misaligned_or_null(head_flipped, shape) || misaligned_or_null(out, shape))
+        return PPN_E_BADARG;
+    const int K = shape->K, E = shape->E;
+    if (part_mirror[0] != 0) return PPN_E_BADARG;
+    for (int k = 0; k < K; ++k)                                  // self-inverse, hence a permutation
+        if (part_mirror[k] < 0 || part_mirror[k] >= K || part_mirror[part_mirror[k]] != k) return PPN_E_BADARG;
+    for (int e = 0; e < E; ++e)
+        if (limb_mirror[e] < 0 || limb_mirror[e] >= E || limb_mirror[limb_mirror[e]] != e) return PPN_E_BADARG;
+    const size_t bytes = (size_t)shape->B * (6 * (size_t)K + (size_t)shape->sH * shape->sW * E) * shape->H * shape->W *
+                         elem_bytes(shape);
+    const uintptr_t o = reinterpret_cast<uintptr_t>(out), f = reinterpret_cast<uintptr_t>(head_flipped),
+                    h = reinterpret_cast<uintptr_t>(head);
+    if (o < f + bytes && f < o + bytes) return PPN_E_BADARG;    // out overlaps head_flipped
+    if (o != h && o < h + bytes && h < o + bytes) return PPN_E_BADARG;   // out is head or apart from it
+    if (shape->inW != shape->W * shape->gridW || 2 * shape->off_w != shape->sW - 1) return PPN_E_UNSUPPORTED;
+    const long long planes = (long long)shape->B * (6LL * K + (long long)shape->sH * shape->sW * E);
+    if (K > 64 || shape->H * shape->W > PPN_MAX_CELLS || planes > 0x7fffffffLL) return PPN_E_UNSUPPORTED;
+    ppn::FlipMergeArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.head = head; a.flipped = head_flipped; a.out = out;
+    a.planes = (uint32_t)planes;
+    a.K = K; a.C = 6 * K + shape->sH * shape->sW * E; a.sH = shape->sH; a.sW = shape->sW;
+    a.W = shape->W; a.HW = shape->H * shape->W;
+    for (int k = 0; k < K; ++k) a.part_mirror[k] = (uint8_t)part_mirror[k];
+    for (int e = 0; e < E; ++e) a.limb_mirror[e] = (uint8_t)limb_mirror[e];
+    a.vec = ((o | f | h) & 15) == 0 && ((size_t)a.HW * elem_bytes(shape)) % 16 == 0;
+    return cuda_rc(ppn::launch_flip_merge(a, shape->head_dtype, (cudaStream_t)stream));
 }
 
 int ppn_debug_argmax_items(const PPNShape* shape, int32_t sms, int32_t* info, int32_t* first, int32_t* size, int32_t max_items) {

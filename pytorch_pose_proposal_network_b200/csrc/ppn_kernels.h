@@ -265,4 +265,18 @@ struct AugmentPeopleArgs {
 };
 cudaError_t launch_augment_people(const AugmentPeopleArgs& a, cudaStream_t st);
 
+// ---- the flip test's merge (ppn_flip.cu): a head averaged with the mirrored head of its flipped input -----------
+struct FlipMergeArgs {
+    const void* head;                   // [B, C, H, W] of the head dtype
+    const void* flipped;                // the same, of the flipped input; never overlaps out
+    void* out;                          // may be head
+    uint32_t planes;                    // B * C
+    int32_t K, C, sH, sW, W, HW;
+    int32_t vec;                        // 16-byte units: the three pointers 16-byte aligned, HW * element a multiple of 16
+    int32_t chunk_planes;               // set by the launcher: planes per CTA
+    uint8_t part_mirror[64];            // [K]
+    uint8_t limb_mirror[256];           // [E]
+};
+cudaError_t launch_flip_merge(const FlipMergeArgs& a, int dtype /* HeadDtype */, cudaStream_t st);
+
 }  // namespace ppn

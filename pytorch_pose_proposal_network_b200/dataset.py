@@ -26,7 +26,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .config import PPNConfig
+from .config import PPNConfig, default_skeleton
 from .parser import _CConfig
 
 
@@ -81,11 +81,7 @@ class TargetEncoder:
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.lib = _lib.lib()
         self.c = _CConfig(cfg)
-        if edges is None:                                      # the skeletons config.py knows (config.py:65 EDGES)
-            from . import config as pcfg
-            edges = {(18, 17): pcfg.EDGES, (16, 15): pcfg.EDGES_16}.get((cfg.K, cfg.E))
-            if edges is None:
-                raise ValueError("pass `edges` ([E][2] part ids) for a skeleton that is not one of config.py's")
+        _, edges = default_skeleton(cfg, edges=edges, need=("edges",))
         e = np.asarray(edges, np.int32).reshape(-1, 2)
         if e.shape[0] != cfg.E:
             raise ValueError(f"{e.shape[0]} edges for a configuration with E = {cfg.E}")
